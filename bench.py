@@ -8,7 +8,7 @@ statistics, their EMA, the inverse refresh every 10th update, preconditioning, K
 Weak scaling: 32 environments x 20 steps PER GPU (8 GPUs = BASELINE.json's 256 x 20 configuration), one NCCL
 all-reduce of [gradients | factor statistics | loss scalars] per update.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line (rank 0).  `value` = env-steps/s (updates/s x envs x steps, whole job) with the inputs
@@ -17,6 +17,11 @@ the loss scalars read back; `roofline` = the factor-statistics GEMM stage timed 
 `cpu_baseline` = the CPU restatement of the reference's update (oracle/, fp32 torch-CPU, all host threads)
 timed on this box.  `--impl reference` times that CPU restatement alone (TensorFlow-1.x + tensorflow/kfac, the
 reference's real dependencies, are not installable offline - see DESIGN.md).
+
+`--dump-outputs DIR` writes, after the timed steps of `value`, what the last of them computed as DIR/<name>.npy
+(float32): the updated parameters (one file per variable, e.g. conv1_weights), the forward's logits and values of
+that step's rows, and its scalars (policy_loss, ..., learning_rate).  Inputs, initial parameters and Fisher samples
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -54,10 +59,17 @@ UNIT = "env-steps/s"
 FRAMESKIP = 4   # a2c_acktr.py:195 - emulator frames per env-step
 
 
+def positive_int(text):
+    value = int(text)
+    if value < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % value)
+    return value
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=positive_int, default=50, help="timed updates of each timed leg")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=32)
@@ -71,7 +83,28 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the conv3 = 64 and A2C 16 x 5 extra keys")
     ap.add_argument("--cpu-budget-s", type=float, default=15.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed update computed as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
+    return args
+
+
+DUMP_LIMIT_BYTES = 63 * 10 ** 6    # array data: with the .npy headers a dump stays within 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32.  Should the arrays exceed DUMP_LIMIT_BYTES together, each is
+    replaced by a sample of its flattened elements, the same share of every array, at positions drawn from a fixed
+    seed, so that two runs with the same arguments sample the same elements."""
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, a.size * DUMP_LIMIT_BYTES // total)
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -349,6 +382,11 @@ def run_native(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     ms_dev, launches, _ = timed(resident, False, args.steps, max(3, args.warmup), window=bool(os.environ.get("ACX_BENCH_NCU")))
+    if args.dump_outputs and rank == 0:
+        # every rank holds the same parameters after an update; logits and values are those of rank 0's environments
+        outputs = {name.replace("/", "_"): v for name, v in e.get_params().items()}
+        outputs.update(logits=e.logits.cpu().numpy(), values=e.values.cpu().numpy(), **e.fetch_scalars())
+        dump_outputs(args.dump_outputs, outputs)
     e.stage_batch(host[0])        # prologue of the double-buffered feed (the copy of step 0's batch)
     ms_e2e, _, scal = timed(host, True, args.steps, 3)
     clocks = sampler.stop() if rank == 0 else None

@@ -69,6 +69,20 @@ class LearnerConfig(ctypes.Structure):
                 ("cov_init_identity", ctypes.c_int), ("no_zero_debias", ctypes.c_int), ("inv_init_identity", ctypes.c_int)]
 
 
+class MLPConfig(ctypes.Structure):
+    _fields_ = [("num_envs", ctypes.c_int), ("num_steps", ctypes.c_int), ("obs_dim", ctypes.c_int),
+                ("num_hidden", ctypes.c_int), ("hidden", ctypes.c_int * 4), ("num_actions", ctypes.c_int),
+                ("acktr", ctypes.c_int),
+                ("gamma", ctypes.c_float), ("entropy_beta", ctypes.c_float), ("value_loss_weight", ctypes.c_float),
+                ("lr_start", ctypes.c_float), ("lr_end", ctypes.c_float), ("lr_decay_steps", ctypes.c_double),
+                ("cov_ema_decay", ctypes.c_float), ("damping", ctypes.c_float), ("momentum", ctypes.c_float),
+                ("norm_constraint", ctypes.c_float),
+                ("invert_every", ctypes.c_int), ("num_cold_updates", ctypes.c_int),
+                ("cold_lr", ctypes.c_float), ("cold_momentum", ctypes.c_float), ("clip_norm", ctypes.c_float),
+                ("rms_decay", ctypes.c_float), ("rms_epsilon", ctypes.c_float),
+                ("use_graphs", ctypes.c_int), ("seed", ctypes.c_uint64)]
+
+
 # every symbol include/acx.h declares: name -> (restype, argtypes)
 _P = ctypes.c_void_p
 SIGNATURES = {
@@ -136,6 +150,20 @@ SIGNATURES = {
     "acx_sample_actions": (ctypes.c_int, [_P, _P, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                           _P, _P]),
     "acx_learner_act": (ctypes.c_int, [_P, _P, ctypes.c_int, _P, ctypes.c_int, _P, _P, _P, _P]),
+    "acx_mlp_arena_bytes": (ctypes.c_size_t, [ctypes.POINTER(MLPConfig)]),
+    "acx_mlp_create": (_P, [ctypes.POINTER(MLPConfig), _P, ctypes.c_size_t]),
+    "acx_mlp_destroy": (None, [_P]),
+    "acx_mlp_num_params": (ctypes.c_size_t, [_P]),
+    "acx_mlp_set_params": (ctypes.c_int, [_P, _P, _P]),
+    "acx_mlp_get_params": (ctypes.c_int, [_P, _P, _P]),
+    "acx_mlp_refresh_weights": (ctypes.c_int, [_P, _P]),
+    "acx_mlp_buffer": (_P, [_P, ctypes.c_char_p, ctypes.POINTER(ctypes.c_size_t)]),
+    "acx_mlp_update": (ctypes.c_int, [_P, _P, _P, _P]),
+    "acx_mlp_set_state": (ctypes.c_int, [_P, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, _P]),
+    "acx_mlp_get_state": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64),
+                                         ctypes.POINTER(ctypes.c_int)]),
+    "acx_mlp_global_step": (ctypes.c_int64, [_P]),
+    "acx_mlp_act": (ctypes.c_int, [_P, _P, ctypes.c_int, _P, ctypes.c_int, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -1,4 +1,4 @@
-"""Host-side handle of the native learner engine (include/acx.h `acx_learner_*`).
+"""Host-side handles of the native learner engines (include/acx.h `acx_learner_*`, `acx_mlp_*`).
 
 torch is used for device memory (the arena is one uint8 CUDA tensor, every buffer a view into it),
 the current CUDA stream and `torch.distributed`; all arithmetic runs in libacx.so.  There is no CPU
@@ -175,10 +175,18 @@ class PendingScalars:
         return dict(zip(SCALAR_NAMES, self._pinned.tolist()))
 
 
-class Engine:
-    """One learner per process / GPU."""
+class _ArenaEngine:
+    """What the learner handles of libacx share: one device arena (every buffer a view into it), the engine's stream,
+    parameters, schedule state, the train-step inputs, scalar read-back and acting.  A subclass names its C API prefix
+    (`_API`), its observation dtype and its parameter layout."""
 
-    def __init__(self, config, device=None):
+    _API = None
+    _OBS_DTYPE = torch.uint8
+
+    def _fn(self, name):
+        return getattr(self.lib, self._API + name)
+
+    def _open(self, config, device, obs_shape):
         if not torch.cuda.is_available():
             raise _lib.AcxError("actorcritic_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = _lib.load()
@@ -188,22 +196,23 @@ class Engine:
         # the engine launches on its own (non-default) stream: CUDA graphs cannot be captured on the legacy stream
         self.stream = torch.cuda.Stream(self.device)
         with torch.cuda.device(self.device):
-            nbytes = self.lib.acx_learner_arena_bytes(ctypes.byref(self._c))
+            nbytes = self._fn("arena_bytes")(ctypes.byref(self._c))
             if nbytes == 0:
                 raise _lib.AcxError(self.lib.acx_last_error().decode())
             self.arena = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
             self._arena_off = (-self.arena.data_ptr()) % 256
             base = self.arena.data_ptr() + self._arena_off
-            self._h = self.lib.acx_learner_create(ctypes.byref(self._c), ctypes.c_void_p(base), ctypes.c_size_t(nbytes))
+            self._h = self._fn("create")(ctypes.byref(self._c), ctypes.c_void_p(base), ctypes.c_size_t(nbytes))
             if not self._h:
                 raise _lib.AcxError(self.lib.acx_last_error().decode())
-        self.is_learner = True          # AtariModel marks the engine it builds for acting only (no objective yet)
-        self.num_params = int(self.lib.acx_learner_num_params(self._h))
+        self.is_learner = True          # the models mark the engine they build for acting only (no objective yet)
+        self.num_params = int(self._fn("num_params")(self._h))
         self.num_envs, self.num_steps = config.num_envs, config.num_steps
         self.rows = config.num_envs * config.num_steps
         self._views = {}
+        self.obs_shape = tuple(obs_shape)
         n, e, a = self.rows, config.num_envs, config.num_actions
-        self.observations = self.buffer("observations", torch.uint8, (n + e,) + OBS_SHAPE)
+        self.observations = self.buffer("observations", self._OBS_DTYPE, (n + e,) + self.obs_shape)
         self.actions = self.buffer("actions", torch.uint8, (e, config.num_steps))
         self.rewards = self.buffer("rewards", torch.float32, (e, config.num_steps))
         self.terminals = self.buffer("terminals", torch.uint8, (e, config.num_steps))
@@ -216,7 +225,7 @@ class Engine:
     def __del__(self):
         h, self._h = getattr(self, "_h", None), None
         if h:
-            self.lib.acx_learner_destroy(h)
+            self._fn("destroy")(h)
 
     # ------------------------------------------------------------------ buffers
     def buffer(self, name, dtype=torch.float32, shape=None):
@@ -224,7 +233,7 @@ class Engine:
         if key in self._views:
             return self._views[key]
         nbytes = ctypes.c_size_t(0)
-        ptr = self.lib.acx_learner_buffer(self._h, name.encode(), ctypes.byref(nbytes))
+        ptr = self._fn("buffer")(self._h, name.encode(), ctypes.byref(nbytes))
         if not ptr:
             raise KeyError(self.lib.acx_last_error().decode())
         off = ptr - self.arena.data_ptr()
@@ -252,29 +261,25 @@ class Engine:
 
     # ------------------------------------------------------------------ parameters / state
     def set_params(self, params):
-        flat = params if isinstance(params, np.ndarray) and params.ndim == 1 else flatten_params(
-            params, self.config.num_actions, self.config.conv3_filters)
+        flat = params if isinstance(params, np.ndarray) and params.ndim == 1 else self._flatten(params)
         flat = np.ascontiguousarray(flat, np.float32)
         if flat.size != self.num_params:
             raise ValueError("expected %d parameters, got %d" % (self.num_params, flat.size))
         with self.on_stream():
-            _lib.check(self.lib.acx_learner_set_params(self._h, flat.ctypes.data_as(ctypes.c_void_p), self._stream()))
+            _lib.check(self._fn("set_params")(self._h, flat.ctypes.data_as(ctypes.c_void_p), self._stream()))
 
     def get_params_flat(self):
         out = np.empty(self.num_params, np.float32)
         with self.on_stream():
-            _lib.check(self.lib.acx_learner_get_params(self._h, out.ctypes.data_as(ctypes.c_void_p), self._stream()))
+            _lib.check(self._fn("get_params")(self._h, out.ctypes.data_as(ctypes.c_void_p), self._stream()))
         return out
 
     def get_params(self):
-        return unflatten_params(self.get_params_flat(), self.config.num_actions, self.config.conv3_filters)
+        return self._unflatten(self.get_params_flat())
 
     def layer_matrix(self, kind, layer):
         """[K+1, C] device view of "params" / "grads" / "precon" for one layer."""
-        c = self.config
-        cols = {"conv1": 32, "conv2": 64, "conv3": c.conv3_filters, "fc4": 512, "fc_policy": c.num_actions,
-                "fc_baseline": 1}[layer]
-        return self.buffer("%s/%s" % (kind, layer), torch.float32).view(-1, cols)
+        return self.buffer("%s/%s" % (kind, layer), torch.float32).view(-1, self._layer_cols(layer))
 
     def factor(self, kind, which, name):
         """Square device view: kind in {"stats","sums","inv"}, which in {"A","G"}."""
@@ -284,22 +289,22 @@ class Engine:
 
     @property
     def global_step(self):
-        return int(self.lib.acx_learner_global_step(self._h))
+        return int(self._fn("global_step")(self._h))
 
     def get_state(self):
         gs, nc, iv = ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int(0)
-        _lib.check(self.lib.acx_learner_get_state(self._h, ctypes.byref(gs), ctypes.byref(nc), ctypes.byref(iv)))
+        _lib.check(self._fn("get_state")(self._h, ctypes.byref(gs), ctypes.byref(nc), ctypes.byref(iv)))
         return dict(global_step=gs.value, num_cov_updates=nc.value, inverses_valid=bool(iv.value))
 
     def set_state(self, global_step, num_cov_updates=0, inverses_valid=False):
         with self.on_stream():
-            _lib.check(self.lib.acx_learner_set_state(self._h, int(global_step), int(num_cov_updates),
-                                                      int(bool(inverses_valid)), self._stream()))
+            _lib.check(self._fn("set_state")(self._h, int(global_step), int(num_cov_updates), int(bool(inverses_valid)),
+                                             self._stream()))
 
     def refresh_derived(self):
         """Re-derive the bf16 operand planes after writing "params" / "inverses" on the device."""
         with self.on_stream():
-            _lib.check(self.lib.acx_learner_refresh_weights(self._h, self._stream()))
+            _lib.check(self._fn("refresh_weights")(self._h, self._stream()))
 
     def wait_pending_ema(self):
         """A split exchange's EMA (Engine._split_exchange) may still be reading the statistics / writing the running sums on
@@ -329,8 +334,8 @@ class Engine:
     # ------------------------------------------------------------------ one update
     def load_batch(self, observations, bootstrap_observations, actions, rewards, terminals, non_blocking=True):
         """Copy the five train-step inputs (ActorCriticModel placeholders, model.py:97-105) into the arena.
-        Accepts host (numpy / pinned torch) or device tensors; layouts [E,T,84,84,4] u8, [E,84,84,4] u8,
-        [E,T] u8, [E,T] f32, [E,T] bool/u8."""
+        Accepts host (numpy / pinned torch) or device tensors; layouts [E,T,*obs_shape], [E,*obs_shape] (uint8 for
+        AtariModel, float32 for MLPModel), [E,T] u8, [E,T] f32, [E,T] bool/u8."""
         n = self.rows
 
         def as_t(x, dtype):
@@ -342,12 +347,88 @@ class Engine:
             return t
 
         with self.on_stream():
-            self.observations[:n].view(self.num_envs, self.num_steps, *OBS_SHAPE).copy_(as_t(observations, torch.uint8),
-                                                                                      non_blocking=non_blocking)
-            self.observations[n:].copy_(as_t(bootstrap_observations, torch.uint8), non_blocking=non_blocking)
+            self.observations[:n].view(self.num_envs, self.num_steps, *self.obs_shape).copy_(
+                as_t(observations, self._OBS_DTYPE), non_blocking=non_blocking)
+            self.observations[n:].copy_(as_t(bootstrap_observations, self._OBS_DTYPE), non_blocking=non_blocking)
             self.actions.copy_(as_t(actions, torch.uint8), non_blocking=non_blocking)
             self.rewards.copy_(as_t(rewards, torch.float32), non_blocking=non_blocking)
             self.terminals.copy_(as_t(terminals, torch.uint8), non_blocking=non_blocking)
+
+    def _fetched(self, fetch):
+        if not fetch:
+            return None
+        if fetch == "async":
+            return self.fetch_scalars_async()
+        return self.fetch_scalars()
+
+    def fetch_scalars_async(self):
+        """Start the device-to-host copy of this update's scalars (losses, clip coefficient, learning rate ...) and return
+        a handle; `handle.result()` waits for THAT copy only, so the host can enqueue the next update before it reads the
+        numbers of this one (`update(fetch="async")`).  Four pinned slots are cycled: resolve a handle before four more
+        updates have been fetched."""
+        if getattr(self, "_pending_slots", None) is None:
+            self._pending_slots = [torch.empty(16, dtype=torch.float32).pin_memory() for _ in range(4)]
+            self._pending_events = [torch.cuda.Event() for _ in range(4)]
+            self._pending_next = 0
+        k = self._pending_next % 4
+        self._pending_next += 1
+        with self.on_stream():
+            self._pending_slots[k].copy_(self.scalars, non_blocking=True)
+            self._pending_events[k].record(self.stream)
+        return PendingScalars(self._pending_slots[k], self._pending_events[k])
+
+    def fetch_scalars(self):
+        with self.on_stream():
+            self._pinned_scalars.copy_(self.scalars, non_blocking=True)
+        self.stream.synchronize()
+        vals = self._pinned_scalars.tolist()
+        return dict(zip(SCALAR_NAMES, vals))
+
+    # ------------------------------------------------------------------ acting
+    def act(self, observations, uniform=None, greedy=False, want_logits=False, out=None):
+        """Forward + categorical sample / argmax on [rows, *obs_shape] device observations
+        (ActorCriticModel.sample_actions / select_max_actions, model.py:135-169).
+
+        `out` (int32 [rows], optional): where the actions go.  A rollout loop that passes the same observation buffer and
+        the same `out` every step has stable pointers, which lets the library replay the whole acting step as one CUDA
+        graph (acx_learner_act / acx_mlp_act); without `out` every call returns fresh tensors."""
+        if not observations.is_cuda:
+            observations = observations.to(self.device, non_blocking=True)
+        observations = observations.to(self._OBS_DTYPE).contiguous()
+        rows = observations.shape[0]
+        actions = out if out is not None else torch.empty(rows, dtype=torch.int32, device=self.device)
+        logits = torch.empty((rows, self.config.num_actions), dtype=torch.float32, device=self.device) if want_logits else None
+        values = torch.empty(rows, dtype=torch.float32, device=self.device) if want_logits else None
+        with self.on_stream():
+            _lib.check(self._fn("act")(
+                self._h, ctypes.c_void_p(observations.data_ptr()), rows,
+                ctypes.c_void_p(uniform.data_ptr()) if uniform is not None else None, int(bool(greedy)),
+                ctypes.c_void_p(actions.data_ptr()),
+                ctypes.c_void_p(logits.data_ptr()) if want_logits else None,
+                ctypes.c_void_p(values.data_ptr()) if want_logits else None, self._stream()))
+        if want_logits:
+            return actions, logits, values
+        return actions
+
+
+class Engine(_ArenaEngine):
+    """One learner per process / GPU (AtariModel's Nature-CNN, include/acx.h `acx_learner_*`)."""
+
+    _API = "acx_learner_"
+
+    def __init__(self, config, device=None):
+        self._open(config, device, OBS_SHAPE)
+
+    def _flatten(self, params):
+        return flatten_params(params, self.config.num_actions, self.config.conv3_filters)
+
+    def _unflatten(self, flat):
+        return unflatten_params(flat, self.config.num_actions, self.config.conv3_filters)
+
+    def _layer_cols(self, layer):
+        c = self.config
+        return {"conv1": 32, "conv2": 64, "conv3": c.conv3_filters, "fc4": 512, "fc_policy": c.num_actions,
+                "fc_baseline": 1}[layer]
 
     # --- double-buffered host feed: the H2D copy of the next batch overlaps the current update ---------------
     def _ensure_staging(self):
@@ -600,11 +681,7 @@ class Engine:
             self.phase1(fisher_labels, fisher_eps, defer_factors="ACX_DEFER_FACTORS" in os.environ)
             self.allreduce(group)
             self.phase2()
-        if not fetch:
-            return None
-        if fetch == "async":
-            return self.fetch_scalars_async()
-        return self.fetch_scalars()
+        return self._fetched(fetch)
 
     def update_separate(self, batch, policy_spec, baseline_spec, step_increments=(1, 1)):
         """objectives.py:31-54 `optimize_separate`: the gradient of the policy loss and the gradient of the baseline loss,
@@ -645,29 +722,6 @@ class Engine:
                     clip_coeff=float("nan"), fisher_norm=float("nan"), grad_norm=float(norms[0]),
                     learning_rate=float(policy_spec[1].value_at(gs)), baseline_grad_norm=float(norms[1]))
 
-    def fetch_scalars_async(self):
-        """Start the device-to-host copy of this update's scalars (losses, clip coefficient, learning rate ...) and return
-        a handle; `handle.result()` waits for THAT copy only, so the host can enqueue the next update before it reads the
-        numbers of this one (`update(fetch="async")`).  Four pinned slots are cycled: resolve a handle before four more
-        updates have been fetched."""
-        if getattr(self, "_pending_slots", None) is None:
-            self._pending_slots = [torch.empty(16, dtype=torch.float32).pin_memory() for _ in range(4)]
-            self._pending_events = [torch.cuda.Event() for _ in range(4)]
-            self._pending_next = 0
-        k = self._pending_next % 4
-        self._pending_next += 1
-        with self.on_stream():
-            self._pending_slots[k].copy_(self.scalars, non_blocking=True)
-            self._pending_events[k].record(self.stream)
-        return PendingScalars(self._pending_slots[k], self._pending_events[k])
-
-    def fetch_scalars(self):
-        with self.on_stream():
-            self._pinned_scalars.copy_(self.scalars, non_blocking=True)
-        self.stream.synchronize()
-        vals = self._pinned_scalars.tolist()
-        return dict(zip(SCALAR_NAMES, vals))
-
     # ------------------------------------------------------------------ stage timing
     STAGES = ("forward", "loss_heads", "backward", "factors", "ema_or_cold", "inverse", "precondition", "apply")
 
@@ -679,28 +733,131 @@ class Engine:
         _lib.check(self.lib.acx_learner_stage_ms(self._h, arr))
         return dict(zip(self.STAGES, [float(x) for x in arr]))
 
-    # ------------------------------------------------------------------ acting
-    def act(self, observations, uniform=None, greedy=False, want_logits=False, out=None):
-        """Forward + categorical sample / argmax on [rows,84,84,4] uint8 device observations
-        (ActorCriticModel.sample_actions / select_max_actions, model.py:135-169).
 
-        `out` (int32 [rows], optional): where the actions go.  A rollout loop that passes the same observation buffer and
-        the same `out` every step has stable pointers, which lets the library replay the whole acting step as one CUDA
-        graph (acx_learner_act); without `out` every call returns fresh tensors."""
-        if not observations.is_cuda:
-            observations = observations.to(self.device, non_blocking=True)
-        observations = observations.contiguous()
-        rows = observations.shape[0]
-        actions = out if out is not None else torch.empty(rows, dtype=torch.int32, device=self.device)
-        logits = torch.empty((rows, self.config.num_actions), dtype=torch.float32, device=self.device) if want_logits else None
-        values = torch.empty(rows, dtype=torch.float32, device=self.device) if want_logits else None
+# ---------------------------------------------------------------------------------------------------------------------
+# fully connected models (MLPModel, include/acx.h `acx_mlp_*`)
+# ---------------------------------------------------------------------------------------------------------------------
+def mlp_layers(num_hidden):
+    """Block names of a fully connected model with `num_hidden` hidden layers, in the order of the flat parameter vector."""
+    return tuple("fc%d" % (i + 1) for i in range(num_hidden)) + ("fc_policy", "fc_baseline")
+
+
+def mlp_param_shapes(obs_dim, hidden_sizes, num_actions):
+    """nn.fully_connected_params layout: weights [in, out], bias [out]."""
+    ins = [int(obs_dim)] + [int(h) for h in hidden_sizes]
+    outs = [int(h) for h in hidden_sizes] + [int(num_actions), 1]
+    ins.append(ins[-1])                     # both heads read the last hidden layer
+    shapes = {}
+    for name, k, c in zip(mlp_layers(len(hidden_sizes)), ins, outs):
+        shapes[name + "/weights"], shapes[name + "/bias"] = (k, c), (c,)
+    return shapes
+
+
+@dataclasses.dataclass
+class MLPEngineConfig:
+    num_envs: int = 16
+    num_steps: int = 5
+    obs_dim: int = 4
+    hidden_sizes: tuple = (64, 64)
+    num_actions: int = 2
+    acktr: bool = True
+    gamma: float = 0.99
+    entropy_beta: float = 0.01
+    value_loss_weight: float = 0.5
+    lr_start: float = 0.25
+    lr_end: float = 0.025
+    lr_decay_steps: float = None            # None: 1e7 / (num_envs * num_steps), as EngineConfig
+    cov_ema_decay: float = 0.99
+    damping: float = 0.01
+    momentum: float = 0.9
+    norm_constraint: float = 0.0001
+    invert_every: int = 10
+    num_cold_updates: int = 30
+    cold_lr: float = 0.0003
+    cold_momentum: float = 0.9
+    clip_norm: float = 0.5
+    rms_decay: float = 0.9
+    rms_epsilon: float = 1e-10
+    use_graphs: bool = True
+    seed: int = 0
+
+    def to_c(self):
+        c = _lib.MLPConfig()
+        c.num_envs, c.num_steps, c.obs_dim, c.num_actions = self.num_envs, self.num_steps, self.obs_dim, self.num_actions
+        if not 1 <= len(self.hidden_sizes) <= 4:
+            raise ValueError("1 to 4 hidden layers")
+        c.num_hidden = len(self.hidden_sizes)
+        for i, h in enumerate(self.hidden_sizes):
+            c.hidden[i] = int(h)
+        c.acktr = int(self.acktr)
+        c.gamma, c.entropy_beta, c.value_loss_weight = self.gamma, self.entropy_beta, self.value_loss_weight
+        c.lr_start, c.lr_end = self.lr_start, self.lr_end
+        steps = self.lr_decay_steps
+        c.lr_decay_steps = float(steps) if steps is not None else 1e7 / (self.num_envs * self.num_steps)
+        c.cov_ema_decay, c.damping, c.momentum = self.cov_ema_decay, self.damping, self.momentum
+        c.norm_constraint = self.norm_constraint
+        c.invert_every, c.num_cold_updates = self.invert_every, self.num_cold_updates
+        c.cold_lr, c.cold_momentum, c.clip_norm = self.cold_lr, self.cold_momentum, self.clip_norm
+        c.rms_decay, c.rms_epsilon = self.rms_decay, self.rms_epsilon
+        c.use_graphs, c.seed = int(bool(self.use_graphs)), self.seed
+        return c
+
+
+class MLPEngine(_ArenaEngine):
+    """Learner of a fully connected actor-critic model on flat float32 observations [rows, obs_dim]: one update
+    (`update`) is one captured CUDA graph of acx_mlp_update."""
+
+    _API = "acx_mlp_"
+    _OBS_DTYPE = torch.float32
+
+    def __init__(self, config, device=None):
+        self._open(config, device, (config.obs_dim,))
+        self.layers = mlp_layers(len(config.hidden_sizes))
+        self._shapes = mlp_param_shapes(config.obs_dim, config.hidden_sizes, config.num_actions)
+
+    def _flatten(self, params):
+        parts = []
+        for layer in self.layers:
+            w = np.asarray(params[layer + "/weights"], np.float32)
+            b = np.asarray(params[layer + "/bias"], np.float32)
+            if w.shape != self._shapes[layer + "/weights"] or b.shape != self._shapes[layer + "/bias"]:
+                raise ValueError("bad shape for layer %s: %s / %s" % (layer, w.shape, b.shape))
+            parts += [w.ravel(), b.ravel()]
+        return np.concatenate(parts)
+
+    def _unflatten(self, flat):
+        out, off = {}, 0
+        for layer in self.layers:
+            for kind in ("weights", "bias"):
+                shape = self._shapes[layer + "/" + kind]
+                n = int(np.prod(shape))
+                out[layer + "/" + kind] = np.asarray(flat[off:off + n]).reshape(shape).copy()
+                off += n
+        return out
+
+    def _layer_cols(self, layer):
+        return self._shapes[layer + "/bias"][0]
+
+    # Session.run drives a train step as phase1 / allreduce / phase2: here the whole update is one call (one graph), so
+    # phase1 only takes the Fisher samples and phase2 runs it; the loss scalars are read after phase2.
+    def phase1(self, fisher_labels=None, fisher_eps=None):
+        self._fisher = (fisher_labels, fisher_eps)
+
+    def allreduce(self, group=None):
+        pass
+
+    def phase2(self):
+        fl, fe = getattr(self, "_fisher", (None, None))
+        self._fisher = (None, None)
+        self.update(None, fl, fe, fetch=False)
+
+    def update(self, batch=None, fisher_labels=None, fisher_eps=None, fetch=True):
+        """The reference's `session.run([..., optimize_op], feed_dict)` (a2c_acktr.py:117-126) for this model."""
+        if batch is not None:
+            self.load_batch(batch["observations"], batch["bootstrap_observations"], batch["actions"], batch["rewards"],
+                            batch["terminals"])
+        fl = ctypes.c_void_p(fisher_labels.data_ptr()) if fisher_labels is not None else None
+        fe = ctypes.c_void_p(fisher_eps.data_ptr()) if fisher_eps is not None else None
         with self.on_stream():
-            _lib.check(self.lib.acx_learner_act(
-                self._h, ctypes.c_void_p(observations.data_ptr()), rows,
-                ctypes.c_void_p(uniform.data_ptr()) if uniform is not None else None, int(bool(greedy)),
-                ctypes.c_void_p(actions.data_ptr()),
-                ctypes.c_void_p(logits.data_ptr()) if want_logits else None,
-                ctypes.c_void_p(values.data_ptr()) if want_logits else None, self._stream()))
-        if want_logits:
-            return actions, logits, values
-        return actions
+            _lib.check(self.lib.acx_mlp_update(self._h, fl, fe, self._stream()))
+        return self._fetched(fetch)

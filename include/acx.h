@@ -370,6 +370,60 @@ int acx_sample_actions(const float* d_logits, const float* d_uniform, uint64_t s
 int acx_learner_act(acx_learner_t* l, const uint8_t* d_obs, int rows, const float* d_uniform,
                     int greedy, int32_t* d_actions, float* d_logits, float* d_values, void* stream);
 
+/* ---- fully connected learner (one process per GPU) ------------------------------------------- */
+/* The same ACKTR / A2C update as acx_learner_*, for a stack of fully connected ReLU layers on flat fp32 observations:
+ * hidden layers fc1 .. fcL (x @ W + b, ReLU; nn.py:37-52) and the heads fc_policy [H_L, A], fc_baseline [H_L, 1] reading the
+ * last hidden layer, with one K-FAC fully connected block per layer (register_fully_connected, model.py:107-119; the two heads
+ * share one input factor as in envs/atari/model.py:243,246).  The hyper-parameter fields mean what they mean in
+ * acx_learner_config_t; precision is that config's default preset. */
+typedef struct {
+  int num_envs, num_steps;
+  int obs_dim;                 /* D: observation features (the Box flattened row-major), 1..2048 */
+  int num_hidden;              /* L: 1..4 hidden layers */
+  int hidden[4];               /* their widths, multiples of 8 in [8, 1024] */
+  int num_actions;             /* 1..31 */
+  int acktr;
+  float gamma, entropy_beta, value_loss_weight;
+  float lr_start, lr_end; double lr_decay_steps;
+  float cov_ema_decay, damping, momentum, norm_constraint;
+  int invert_every, num_cold_updates;
+  float cold_lr, cold_momentum, clip_norm;
+  float rms_decay, rms_epsilon;
+  int use_graphs;
+  uint64_t seed;
+} acx_mlp_config_t;
+
+typedef struct acx_mlp acx_mlp_t;
+
+size_t acx_mlp_arena_bytes(const acx_mlp_config_t* cfg);
+acx_mlp_t* acx_mlp_create(const acx_mlp_config_t* cfg, void* d_arena, size_t arena_bytes);
+void acx_mlp_destroy(acx_mlp_t* l);
+/* flat fp32 parameter vector, per layer [K_l+1, C_l] (the [in, out] weights of nn.fully_connected_params, nn.py:8-33, then
+ * the bias row), layers in the order fc1 .. fcL, fc_policy, fc_baseline. */
+size_t acx_mlp_num_params(const acx_mlp_t* l);
+int acx_mlp_set_params(acx_mlp_t* l, const float* h_params, void* stream);
+int acx_mlp_get_params(acx_mlp_t* l, float* h_params, void* stream);
+int acx_mlp_refresh_weights(acx_mlp_t* l, void* stream);
+/* named device views, as acx_learner_buffer: "observations" f32 [N+E, D] (train rows batch-major [E,T], then the E bootstrap
+ * rows), "actions" "rewards" "terminals", "params" "velocity" "accum" "grads" "precon" "factor_stats" "factor_sums"
+ * "inverses" "reduce_bucket" "scalars" "sched" "logits" "values" "targets" "advantages" "dheads", per block
+ * "params/<layer>" "grads/<layer>" "precon/<layer>" "velocity/<layer>" "accum/<layer>", "stats/A/<factor>" "sums/A/<factor>"
+ * (fc1 .. fcL, heads), "stats/G/<layer>" "sums/G/<layer>" "inv/A/<layer>" "inv/G/<layer>", and "act_hi/fc<i>": the hi plane
+ * of each hidden activation, whose sign is the ReLU mask of the backward pass. */
+void* acx_mlp_buffer(acx_mlp_t* l, const char* name, size_t* num_bytes);
+/* One update = session.run(optimize_op, feed_dict) (a2c_acktr.py:117-126) for this model: forward, returns, A2C loss and
+ * gradients, Fisher backward and factor statistics, then ColdStartPeriodicInvUpdateKfacOpt.apply_gradients (kfac_utils.py:38-53)
+ * or ClipGlobalNorm(RMSProp) (a2c_acktr.py:250-251); one captured CUDA graph per schedule variant.  Fisher samples as in
+ * acx_learner_phase1 (NULL = Philox). */
+int acx_mlp_update(acx_mlp_t* l, const int32_t* d_fisher_labels, const float* d_fisher_eps, void* stream);
+int acx_mlp_set_state(acx_mlp_t* l, int64_t global_step, int64_t num_cov_updates, int inverses_valid, void* stream);
+int acx_mlp_get_state(const acx_mlp_t* l, int64_t* global_step, int64_t* num_cov_updates, int* inverses_valid);
+int64_t acx_mlp_global_step(const acx_mlp_t* l);
+/* ActorCriticModel.sample_actions / select_max_actions (model.py:135-169): forward on `rows` <= N+E observations
+ * d_obs f32 [rows, D] -> logits, values; then the categorical draw / argmax of acx_sample_actions. */
+int acx_mlp_act(acx_mlp_t* l, const float* d_obs, int rows, const float* d_uniform, int greedy, int32_t* d_actions,
+                float* d_logits, float* d_values, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,7 +5,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(os.path.dirname(HERE), "libacx.so")
-SOURCES = ["lib.cu", "preprocess.cu", "returns.cu", "gemm.cu", "conv.cu", "layers.cu", "kfac.cu", "kfac_inv.cu", "peer.cu", "learner.cu", "mlp.cu"]
+SOURCES = ["lib.cu", "preprocess.cu", "returns.cu", "gemm.cu", "conv.cu", "layers.cu", "kfac.cu", "kfac_inv.cu", "peer.cu", "learner_core.cu", "learner.cu", "mlp.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--expt-relaxed-constexpr",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xcompiler", "-Wno-unused-function",
          "-fmad=true", "-shared", "-lcudart_static", "-lpthread", "-ldl", "-lrt"]

@@ -12,15 +12,15 @@
 //   phase 2  schedule of ColdStartPeriodicInvUpdateKfacOpt.apply_gradients as coded (kfac_utils.py:38-53):
 //            cold momentum-SGD step or factor EMA, scheduled inverse refresh, precondition, KL clip, momentum,
 //            apply; or the A2C RMSProp step (a2c_acktr.py:250-251).
+// The host code it shares with the fully connected learner (mlp.cu) - arena, K-FAC blocks and their state, schedule, inverse
+// refresh, graph cache - lives in learner_core.cuh / learner_core.cu.
 #include <algorithm>
-#include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <map>
 #include <string>
 #include <vector>
 
-#include "layers.cuh"
+#include "learner_core.cuh"
 
 namespace acx {
 
@@ -34,30 +34,9 @@ int peer_allreduce(const PeerState& ps, size_t region_offset_bytes, size_t flags
 size_t peer_flag_bytes();
 size_t peer_epoch_bytes();
 
-struct Layer {
-  const char* name;
-  int K, C;         // V_l = [K+1, C]
+struct Layer {       // geometry of layer l; its K-FAC block (K, C, parameter offset, T~) is acx_learner::blk[l]
   int T;            // output locations (1 for fc)
-  int Tnorm;        // T~_l used for lambda/T~ and the 1/T~ rescale (SURVEY A.7-U1)
-  int conv, k, s, cin, hw_in, hw_out;
-  size_t off;       // offset of V_l in the flat parameter vector
-  int afac;         // index of its input factor (the two heads share one)
-};
-
-struct Buf {
-  void* ptr;
-  size_t bytes;
-};
-
-struct Arena {
-  uint8_t* base = nullptr;
-  size_t used = 0;
-  void* take(size_t bytes) {
-    used = align_up(used, 256);
-    void* p = base ? base + used : nullptr;
-    used += bytes;
-    return p;
-  }
+  int k, s, cin, hw_in, hw_out;
 };
 
 // Per-lane scratch: kernels of different lanes run concurrently (streams forked from the caller's stream, also inside a
@@ -73,61 +52,16 @@ struct Scratch {
 // onto the last one (3 lanes: wgrad + output factors + column sums share lane 2 - round 1's arrangement).
 constexpr int kMaxLanes = 5;
 
-struct GraphKey {
-  int phase, variant;
-  const void* p0;
-  const void* p1;
-  const void* p2 = nullptr;
-  const void* p3 = nullptr;
-  const void* p4 = nullptr;
-  bool operator<(const GraphKey& o) const {
-    if (phase != o.phase) return phase < o.phase;
-    if (variant != o.variant) return variant < o.variant;
-    if (p0 != o.p0) return p0 < o.p0;
-    if (p1 != o.p1) return p1 < o.p1;
-    if (p2 != o.p2) return p2 < o.p2;
-    if (p3 != o.p3) return p3 < o.p3;
-    return p4 < o.p4;
-  }
-};
-struct GraphEntry {
-  int uses = 0;
-  cudaGraphExec_t exec = nullptr;
-  uint64_t launches = 0;
-};
-
 }  // namespace acx
 
 using namespace acx;
 
-struct acx_learner {
+// the K-FAC blocks conv1, conv2, conv3, fc4, fc_policy, fc_baseline and their state (KfacBlocks), plus the Nature-CNN's
+// activations, lanes and data-parallel exchange
+struct acx_learner : KfacBlocks {
   acx_learner_config_t cfg;
   int E, T, N, R, A, c3;
   Layer L[6];
-  size_t num_params, params_pad;
-  int adim[5];
-  size_t aoff[5], goff[6], factor_floats;
-  // fp32 state
-  float *params, *precon, *velocity, *accum;
-  float *bucket, *grads, *stats, *bscalars;
-  size_t bucket_floats;
-  float *sums;            // running factor sums, same layout as stats
-  float *inv;             // fp32 inverses: A^-1 per layer (6) then G^-1 per layer (6)
-  size_t ainv_off[6], ginv_off[6], inv_floats;
-  Planes ainv_pl[6], ginv_pl[6];
-  float *damp, *lambdas, *scalars;
-  Sched* sched;
-  const float** d_a_ptrs;
-  const float** d_g_ptrs;
-  int *d_a_dims, *d_g_dims;
-  InvJob h_jobs[12];
-  InvJob* d_jobs;
-  unsigned int* inv_bar;     // grid-barrier counter of the persistent inverse kernel
-  unsigned long long* act_counter;   // device-resident number of acting calls (Philox step of sample_actions)
-  PreconJob h_pjobs[6];
-  PreconJob* d_pjobs;
-  int num_pjobs, pjobs_max_d;
-  float* precon_w;
   // inputs
   uint8_t *obs, *actions, *terminals;
   float* rewards;
@@ -163,9 +97,7 @@ struct acx_learner {
   cudaEvent_t patches_ready[4] = {nullptr, nullptr, nullptr, nullptr};   // P_l complete on the aux lane (this update)
   cudaEvent_t a_ready = nullptr;     // all input-factor statistics of the current phase 1 are complete (external event)
   bool a_ready_valid = false;        // the last phase 1 recorded it
-  // host mirror of the schedule
-  int64_t gs, ncov;
-  bool inverses_valid;
+  Schedule sch;
   uint64_t act_calls;
   int lvl_fwd, lvl_bwd, lvl_fisher, lvl_factor, lvl_precon, act_planes, grad_planes;
   // optional stage timing (CUDA events on the launching stream)
@@ -177,35 +109,17 @@ struct acx_learner {
   int deferred = 0;                       // what the last phase 1 actually left to phase 2
   cudaEvent_t ev[ACX_NUM_STAGES + 2];
   bool ev_set[ACX_NUM_STAGES + 2];
-  std::map<std::string, Buf> named;
-  std::map<GraphKey, GraphEntry> graphs;
+  GraphCache graphs;
 };
 
 namespace acx {
 
-static const int kColsumChunks = 592;
 static const int kBorderChunks = 160;   // row chunks of the batch-sum pass over a conv input (4 samples per CTA at 32 x 20)
 static const int kGramChunks = 444;   // 3 CTAs per SM
 static const size_t kDgradChunkBytes = 0;   // 0 = whole batch in one piece.  Measured on B200 at 32x20 (ACX_DGRAD_CHUNK_MB sweep):
                                             // whole 1.510 ms/update, 128 MB 1.533, 64 MB 1.551, 32 MB 1.599, 16 MB 1.681 - the
                                             // extra launches and wave tails cost more than the HBM round trip saves
-static const int kDotPartials = 296;   // two chunks per SM: ~11 elements per thread at 865 k parameters
 
-static int pad8(int x) { return (x + 7) / 8 * 8; }
-
-static Planes take_planes(Arena& ar, int nplanes, size_t rows, int ld) {
-  Planes pl;
-  pl.n = nplanes;
-  pl.ld = ld;
-  for (int i = 0; i < nplanes; ++i) pl.p[i] = reinterpret_cast<bf16*>(ar.take(rows * (size_t)ld * sizeof(bf16)));
-  return pl;
-}
-
-static Planes offset_rows(const Planes& p, size_t rows) {
-  Planes q = p;
-  for (int i = 0; i < p.n; ++i) q.p[i] = p.p[i] + rows * (size_t)p.ld;
-  return q;
-}
 static Planes with_ld(const Planes& p, int ld) {
   Planes q = p;
   q.ld = ld;
@@ -225,48 +139,26 @@ static bool fwd_tc_enabled() {   // tuning knob: ACX_CONV_FWD=0 keeps im2col + G
 static void setup_layers(acx_learner* l) {
   const int c3 = l->c3, A = l->A;
   const int mode = l->cfg.num_locations_mode;
-  Layer defs[6] = {
-      {"conv1", 256, 32, 400, mode ? 84 * 84 / 16 : 400, 1, 8, 4, 4, 84, 20, 0, 0},
-      {"conv2", 512, 64, 81, mode ? 20 * 20 / 4 : 81, 1, 4, 2, 32, 20, 9, 0, 1},
-      {"conv3", 576, c3, 49, mode ? 81 : 49, 1, 3, 1, 64, 9, 7, 0, 2},
-      {"fc4", 49 * c3, 512, 1, 1, 0, 0, 0, 0, 0, 0, 0, 3},
-      {"fc_policy", 512, A, 1, 1, 0, 0, 0, 0, 0, 0, 0, 4},
-      {"fc_baseline", 512, 1, 1, 1, 0, 0, 0, 0, 0, 0, 0, 4},
-  };
-  size_t off = 0;
+  static const char* names[6] = {"conv1", "conv2", "conv3", "fc4", "fc_policy", "fc_baseline"};
+  const int K[6] = {256, 512, 576, 49 * c3, 512, 512}, C[6] = {32, 64, c3, 512, A, 1};
+  const int Tnorm[6] = {mode ? 84 * 84 / 16 : 400, mode ? 20 * 20 / 4 : 81, mode ? 81 : 49, 1, 1, 1};
+  const Layer geo[6] = {{400, 8, 4, 4, 84, 20}, {81, 4, 2, 32, 20, 9}, {49, 3, 1, 64, 9, 7}, {1}, {1}, {1}};
   for (int i = 0; i < 6; ++i) {
-    l->L[i] = defs[i];
-    l->L[i].off = off;
-    off += (size_t)(defs[i].K + 1) * defs[i].C;
+    Block& b = l->blk[i];
+    b.name = names[i];
+    b.K = K[i];
+    b.C = C[i];
+    b.afac = i < 5 ? i : 4;
+    b.Tnorm = Tnorm[i];
+    l->L[i] = geo[i];
   }
-  l->num_params = off;
-  l->params_pad = align_up(off, 4);
-  const int adims[5] = {257, 513, 577, 49 * c3 + 1, 513};
-  size_t f = 0;
-  for (int i = 0; i < 5; ++i) {
-    l->adim[i] = adims[i];
-    l->aoff[i] = f;
-    f += align_up((size_t)adims[i] * adims[i], 4);
-  }
-  for (int i = 0; i < 6; ++i) {
-    l->goff[i] = f;
-    f += align_up((size_t)l->L[i].C * l->L[i].C, 4);
-  }
-  l->factor_floats = f;
-  size_t v = 0;
-  for (int i = 0; i < 6; ++i) {
-    const int d = l->L[i].K + 1;
-    l->ainv_off[i] = v;
-    v += align_up((size_t)d * d, 4);
-  }
-  for (int i = 0; i < 6; ++i) {
-    l->ginv_off[i] = v;
-    v += align_up((size_t)l->L[i].C * l->L[i].C, 4);
-  }
-  l->inv_floats = v;
+  l->set_blocks(6);
 }
 
-static void reg(acx_learner* l, const char* name, void* p, size_t bytes) { l->named[name] = Buf{p, bytes}; }
+static ConvGeom geom_of(const acx_learner* l, int i) {
+  const Layer& L = l->L[i];
+  return ConvGeom{L.hw_in, L.cin, L.k, L.s, L.hw_out, l->blk[i].C};
+}
 
 // lay the arena out (base == nullptr: size pass only)
 static size_t layout(acx_learner* l, uint8_t* base) {
@@ -274,95 +166,26 @@ static size_t layout(acx_learner* l, uint8_t* base) {
   ar.base = base;
   const int N = l->N, R = l->R, A = l->A, c3 = l->c3;
   const size_t B2 = 2 * (size_t)N;
-  const size_t P = l->params_pad, F = l->factor_floats;
-  auto f32 = [&](size_t n) { return reinterpret_cast<float*>(ar.take(n * sizeof(float))); };
-  // ---- persistent fp32 state (one contiguous block so that it can be zeroed / checkpointed as a whole)
-  l->params = f32(P);
-  l->velocity = f32(P);
-  l->accum = f32(P);
-  l->precon = f32(P);
-  l->bucket_floats = P + F + 4;
-  l->bucket = f32(l->bucket_floats);
-  l->stats = l->bucket;            // [A | G]: one contiguous block for the EMA, A first (the early all-reduce prefix)
-  l->grads = l->bucket + F;
-  l->bscalars = l->bucket + F + P;
-  l->sums = f32(F);
-  l->inv = f32(l->inv_floats);
-  l->damp = f32(16);
-  l->lambdas = f32(8);
-  l->scalars = f32(16);
-  l->sched = reinterpret_cast<Sched*>(ar.take(sizeof(Sched)));
+  l->take_state(ar);
   l->peer_flags = reinterpret_cast<unsigned int*>(ar.take(peer_flag_bytes()));
   l->peer_epochs = reinterpret_cast<unsigned int*>(ar.take(peer_epoch_bytes()));
-  l->d_a_ptrs = reinterpret_cast<const float**>(ar.take(6 * sizeof(float*)));
-  l->d_g_ptrs = reinterpret_cast<const float**>(ar.take(6 * sizeof(float*)));
-  l->d_a_dims = reinterpret_cast<int*>(ar.take(6 * sizeof(int)));
-  l->d_g_dims = reinterpret_cast<int*>(ar.take(6 * sizeof(int)));
-  l->d_jobs = reinterpret_cast<InvJob*>(ar.take(12 * sizeof(InvJob)));
-  l->d_pjobs = reinterpret_cast<PreconJob*>(ar.take(6 * sizeof(PreconJob)));
-  l->inv_bar = reinterpret_cast<unsigned int*>(ar.take(256));
-  l->act_counter = reinterpret_cast<unsigned long long*>(ar.take(256));
-  l->precon_w = f32(P);
-  for (int i = 0; i < 6; ++i) {
-    const int d = l->L[i].K + 1, c = l->L[i].C;
-    l->ainv_pl[i] = take_planes(ar, 3, d, pad8(d));
-    l->ginv_pl[i] = take_planes(ar, 3, c, pad8(c));
-  }
-  // inverse jobs (sorted by decreasing n later)
-  for (int i = 0; i < 6; ++i) {
-    const int d = l->L[i].K + 1, c = l->L[i].C;
-    InvJob& ja = l->h_jobs[i];
-    ja.s = l->sums + l->aoff[l->L[i].afac];
-    ja.n = d;
-    ja.damp_index = 2 * i;
-    ja.work_m = reinterpret_cast<double*>(ar.take((size_t)d * d * sizeof(double)));
-    ja.work_x = reinterpret_cast<double*>(ar.take(((size_t)3 * 32 * d + 2 * 32 * 32 + 2048) * sizeof(double)));
-    ja.inv = l->inv + l->ainv_off[i];
-    for (int q = 0; q < 3; ++q) ja.planes[q] = l->ainv_pl[i].p[q];
-    ja.ld_planes = l->ainv_pl[i].ld;
-    InvJob& jg = l->h_jobs[6 + i];
-    jg.s = l->sums + l->goff[i];
-    jg.n = c;
-    jg.damp_index = 2 * i + 1;
-    jg.work_m = reinterpret_cast<double*>(ar.take((size_t)c * c * sizeof(double)));
-    jg.work_x = reinterpret_cast<double*>(ar.take(((size_t)3 * 32 * c + 2 * 32 * 32 + 2048) * sizeof(double)));
-    jg.inv = l->inv + l->ginv_off[i];
-    for (int q = 0; q < 3; ++q) jg.planes[q] = l->ginv_pl[i].p[q];
-    jg.ld_planes = l->ginv_pl[i].ld;
-  }
-  // small blocks (C <= 64) are preconditioned by the batched fp32 SIMT kernels
-  l->num_pjobs = 0;
-  l->pjobs_max_d = 0;
-  for (int i = 0; i < 6; ++i) {
-    if (l->L[i].C > 64) continue;
-    PreconJob& pj = l->h_pjobs[l->num_pjobs++];
-    pj.v = l->grads + l->L[i].off;
-    pj.ginv = l->inv + l->ginv_off[i];
-    pj.ainv = l->inv + l->ainv_off[i];
-    pj.w = l->precon_w + l->L[i].off;
-    pj.u = l->precon + l->L[i].off;
-    pj.d = l->L[i].K + 1;
-    pj.c = l->L[i].C;
-    pj.scale = 1.0f / (float)l->L[i].Tnorm;
-    l->pjobs_max_d = std::max(l->pjobs_max_d, pj.d);
-  }
+  l->take_tables(ar);
   // ---- inputs
   l->obs = reinterpret_cast<uint8_t*>(ar.take((size_t)R * 28224));
   l->actions = reinterpret_cast<uint8_t*>(ar.take(N));
   l->terminals = reinterpret_cast<uint8_t*>(ar.take(N));
-  l->rewards = f32(N);
+  l->rewards = ar.f32(N);
   // ---- weights as GEMM operands
   for (int i = 0; i < 4; ++i) {
-    l->wT[i] = take_planes(ar, 3, l->L[i].C, pad8(l->L[i].K));   // W^T [C, K]   (forward: B operand, K-major)
-    l->wN[i] = take_planes(ar, 3, l->L[i].K, pad8(l->L[i].C));   // W   [K, C]   (dgrad:   B operand, K-major)
+    l->wT[i] = take_planes(ar, 3, l->blk[i].C, pad8(l->blk[i].K));   // W^T [C, K]   (forward: B operand, K-major)
+    l->wN[i] = take_planes(ar, 3, l->blk[i].K, pad8(l->blk[i].C));   // W   [K, C]   (dgrad:   B operand, K-major)
   }
   for (int i = 1; i <= 2; ++i) {
     const Layer& L = l->L[i];
-    const ConvGeom g = {L.hw_in, L.cin, L.k, L.s, L.hw_out, L.C};
-    l->conv_tc[i] = l->cfg.conv_impl == 0 && l->cfg.gemm_impl == 0 && conv_tc_supported(g, 1);
+    l->conv_tc[i] = l->cfg.conv_impl == 0 && l->cfg.gemm_impl == 0 && conv_tc_supported(geom_of(l, i), 1);
     if (l->conv_tc[i]) {
       const int m = L.k / L.s;
-      l->wD[i] = take_planes(ar, 3, (size_t)L.s * L.s * L.cin, pad8(m * m * L.C));   // rows (py,px,ci), K = (i,j,co)
+      l->wD[i] = take_planes(ar, 3, (size_t)L.s * L.s * L.cin, pad8(m * m * l->blk[i].C));   // rows (py,px,ci), K = (i,j,co)
     }
   }
   l->conv_tc[0] = l->conv_tc[3] = false;
@@ -377,11 +200,11 @@ static size_t layout(acx_learner* l, uint8_t* base) {
   l->P3 = take_planes(ar, np, (size_t)R * 49, 576);
   l->act3 = take_planes(ar, np, (size_t)R * 49, c3);
   l->act4 = take_planes(ar, np, (size_t)R, 512);
-  l->logits = f32((size_t)R * A);
-  l->values = f32(R);
-  l->targets = f32(N);
-  l->adv = f32(N);
-  l->dheads = f32(B2 * (A + 1));
+  l->logits = ar.f32((size_t)R * A);
+  l->values = ar.f32(R);
+  l->targets = ar.f32(N);
+  l->adv = ar.f32(N);
+  l->dheads = ar.f32(B2 * (A + 1));
   const int ng = l->grad_planes;
   l->dpre4 = take_planes(ar, ng, B2, 512);
   l->dpre3 = take_planes(ar, ng, B2 * 49, c3);
@@ -393,22 +216,22 @@ static size_t layout(acx_learner* l, uint8_t* base) {
     const size_t whole = std::max(B2 * 49 * 576, B2 * 81 * 512) * sizeof(float);
     l->dgrad_chunk_bytes = (mb == 0 || (mb << 20) > whole) ? whole : (mb << 20);
   }
-  l->dP = f32(l->dgrad_chunk_bytes / sizeof(float) + 81 * 512);   // one chunk of patch gradients
+  l->dP = ar.f32(l->dgrad_chunk_bytes / sizeof(float) + 81 * 512);   // one chunk of patch gradients
   // ---- preconditioning scratch
   int dmax = 0, cmax = 0;
   for (int i = 0; i < 6; ++i) {
-    dmax = std::max(dmax, l->L[i].K + 1);
-    cmax = std::max(cmax, l->L[i].C);
+    dmax = std::max(dmax, l->blk[i].K + 1);
+    cmax = std::max(cmax, l->blk[i].C);
   }
   l->Vp = take_planes(ar, 3, dmax, pad8(cmax));
   l->Wt = take_planes(ar, 3, cmax, pad8(dmax));
-  l->dot_partials = f32(kDotPartials);
+  l->dot_partials = ar.f32(kDotPartials);
   const size_t kpad = align_up((size_t)49 * c3, 128);
   for (int i = 0; i < kMaxLanes; ++i) {
     Scratch& sc = l->scr[i];
-    sc.colsum_partial = f32(std::max(std::max((size_t)kColsumChunks * (size_t)std::max(49 * c3, 576), (size_t)kBorderChunks * 28224),
-                                     (size_t)kGramChunks * 4096));
-    sc.colsum_tmp = f32(4096 + 28224 + 8);   // [0,4096): border / column-sum vectors, then the batch-summed conv input
+    sc.colsum_partial = ar.f32(std::max(std::max((size_t)kColsumChunks * (size_t)std::max(49 * c3, 576), (size_t)kBorderChunks * 28224),
+                                        (size_t)kGramChunks * 4096));
+    sc.colsum_tmp = ar.f32(4096 + 28224 + 8);   // [0,4096): border / column-sum vectors, then the batch-summed conv input
     sc.ws_bytes = std::max<size_t>((size_t)48 << 20, kpad * kpad * sizeof(float) + (1 << 20));
     sc.ws = reinterpret_cast<float*>(ar.take(sc.ws_bytes));
   }
@@ -478,70 +301,39 @@ static void setup_gather(acx_learner* l) {
   for (int li = 0; li < 3; ++li) {
     acx_gather_t& g = l->gat_g[li];
     const Layer& L = l->L[li];
+    const int C = l->blk[li].C;
     fill(g, *dp[li], dp[li]->n);
-    const long long px = (long long)L.C * 2;
-    const long long dim[5] = {L.C, L.hw_out, 1, L.hw_out, N}, st[4] = {px, px, L.hw_out * px, (long long)L.hw_out * L.hw_out * px};
+    const long long px = (long long)C * 2;
+    const long long dim[5] = {C, L.hw_out, 1, L.hw_out, N}, st[4] = {px, px, L.hw_out * px, (long long)L.hw_out * L.hw_out * px};
     for (int i = 0; i < 5; ++i) g.dim[i] = dim[i];
     for (int i = 0; i < 4; ++i) g.stride_bytes[i] = st[i];
     g.gx = g.gy = L.hw_out;
     g.samples = N;
-    g.num_chunks = (L.C + 63) / 64;
+    g.num_chunks = (C + 63) / 64;
     for (int j = 0; j < g.num_chunks; ++j) g.c0[j] = (signed char)(64 * j);
   }
 }
 
 static void register_buffers(acx_learner* l) {
-  const size_t P = l->num_params;
-  reg(l, "params", l->params, P * 4);
-  reg(l, "velocity", l->velocity, P * 4);
-  reg(l, "accum", l->accum, P * 4);
-  reg(l, "precon", l->precon, P * 4);
-  reg(l, "grads", l->grads, P * 4);
-  reg(l, "reduce_bucket", l->bucket, l->bucket_floats * 4);
-  reg(l, "factor_stats", l->stats, l->factor_floats * 4);
-  reg(l, "input_factor_stats", l->stats, l->goff[0] * 4);   // the A part = the prefix of the reduce bucket
-  reg(l, "factor_sums", l->sums, l->factor_floats * 4);
-  reg(l, "inverses", l->inv, l->inv_floats * 4);
-  reg(l, "dampings", l->damp, 12 * 4);
-  reg(l, "scalars", l->scalars, 16 * 4);
-  reg(l, "sched", l->sched, sizeof(Sched));
-  reg(l, "observations", l->obs, (size_t)l->R * 28224);
-  reg(l, "actions", l->actions, l->N);
-  reg(l, "terminals", l->terminals, l->N);
-  reg(l, "rewards", l->rewards, (size_t)l->N * 4);
-  reg(l, "logits", l->logits, (size_t)l->R * l->A * 4);
-  reg(l, "values", l->values, (size_t)l->R * 4);
-  reg(l, "targets", l->targets, (size_t)l->N * 4);
-  reg(l, "advantages", l->adv, (size_t)l->N * 4);
-  reg(l, "patches/conv1", l->P1.p[0], (size_t)l->R * 400 * 256 * 2);   // bf16 [R*400, 256], raw byte values (ACX_GATHER=0 only)
-  reg(l, "obs_pairs", l->obs_pairs, (size_t)l->R * 28224 * 2);         // bf16 [R, 42, 84, 2, 4]: the row-pair copy of the observations
+  l->register_buffers();
+  l->reg("input_factor_stats", l->stats, l->goff[0] * 4);   // the A part = the prefix of the reduce bucket
+  l->reg("observations", l->obs, (size_t)l->R * 28224);
+  l->reg("actions", l->actions, l->N);
+  l->reg("terminals", l->terminals, l->N);
+  l->reg("rewards", l->rewards, (size_t)l->N * 4);
+  l->reg("logits", l->logits, (size_t)l->R * l->A * 4);
+  l->reg("values", l->values, (size_t)l->R * 4);
+  l->reg("targets", l->targets, (size_t)l->N * 4);
+  l->reg("advantages", l->adv, (size_t)l->N * 4);
+  l->reg("patches/conv1", l->P1.p[0], (size_t)l->R * 400 * 256 * 2);   // bf16 [R*400, 256], raw byte values (ACX_GATHER=0 only)
+  l->reg("obs_pairs", l->obs_pairs, (size_t)l->R * 28224 * 2);         // bf16 [R, 42, 84, 2, 4]: the row-pair copy of the observations
   // hi planes of the forward activations = the ReLU masks the backward pass applies (act > 0); exposed so that the parity
   // tests can tell arithmetic error from units whose pre-activation is within rounding of zero
-  reg(l, "act_hi/conv1", l->act1.p[0], (size_t)l->R * 400 * 32 * 2);
-  reg(l, "act_hi/conv2", l->act2.p[0], (size_t)l->R * 81 * 64 * 2);
-  reg(l, "act_hi/conv3", l->act3.p[0], (size_t)l->R * 49 * l->c3 * 2);
-  reg(l, "act_hi/fc4", l->act4.p[0], (size_t)l->R * 512 * 2);
-  reg(l, "dheads", l->dheads, (size_t)2 * l->N * (l->A + 1) * 4);
-  static const char* an[5] = {"conv1", "conv2", "conv3", "fc4", "heads"};
-  for (int i = 0; i < 5; ++i) {
-    const size_t b = (size_t)l->adim[i] * l->adim[i] * 4;
-    reg(l, (std::string("stats/A/") + an[i]).c_str(), l->stats + l->aoff[i], b);
-    reg(l, (std::string("sums/A/") + an[i]).c_str(), l->sums + l->aoff[i], b);
-  }
-  for (int i = 0; i < 6; ++i) {
-    const size_t b = (size_t)l->L[i].C * l->L[i].C * 4;
-    reg(l, (std::string("stats/G/") + l->L[i].name).c_str(), l->stats + l->goff[i], b);
-    reg(l, (std::string("sums/G/") + l->L[i].name).c_str(), l->sums + l->goff[i], b);
-    const int d = l->L[i].K + 1;
-    reg(l, (std::string("inv/A/") + l->L[i].name).c_str(), l->inv + l->ainv_off[i], (size_t)d * d * 4);
-    reg(l, (std::string("inv/G/") + l->L[i].name).c_str(), l->inv + l->ginv_off[i], b);
-    const size_t vb = (size_t)d * l->L[i].C * 4;
-    reg(l, (std::string("params/") + l->L[i].name).c_str(), l->params + l->L[i].off, vb);
-    reg(l, (std::string("grads/") + l->L[i].name).c_str(), l->grads + l->L[i].off, vb);
-    reg(l, (std::string("precon/") + l->L[i].name).c_str(), l->precon + l->L[i].off, vb);
-    reg(l, (std::string("velocity/") + l->L[i].name).c_str(), l->velocity + l->L[i].off, vb);
-    reg(l, (std::string("accum/") + l->L[i].name).c_str(), l->accum + l->L[i].off, vb);
-  }
+  l->reg("act_hi/conv1", l->act1.p[0], (size_t)l->R * 400 * 32 * 2);
+  l->reg("act_hi/conv2", l->act2.p[0], (size_t)l->R * 81 * 64 * 2);
+  l->reg("act_hi/conv3", l->act3.p[0], (size_t)l->R * 49 * l->c3 * 2);
+  l->reg("act_hi/fc4", l->act4.p[0], (size_t)l->R * 512 * 2);
+  l->reg("dheads", l->dheads, (size_t)2 * l->N * (l->A + 1) * 4);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -595,39 +387,6 @@ static int join_lane(acx_learner* l, const Lane& ln, cudaStream_t main_st) {
   return order_after(l, ln.st, main_st);
 }
 
-// ------------------------------------------------------------------------------------------------
-// GEMM helper: picks the plane pairs from the precision level (pairs (i,j) with i + j <= level)
-// ------------------------------------------------------------------------------------------------
-struct GemmOut {
-  float* c = nullptr;
-  int ldc = 0;
-  const Planes* planes = nullptr;
-  const float* bias = nullptr;
-  int relu = 0;
-  const bf16* mask = nullptr;
-  int mask_ld = 0, mask_rows = 0;
-  const uint8_t* a_patch = nullptr;   // A = conv1 patch matrix generated in the kernel from these observations
-  int a_patch_samples = 0;
-  const acx_gather_t* a_gather = nullptr;   // operands read in place from NHWC tensors (acx.h)
-  const acx_gather_t* b_gather = nullptr;
-  int perm_m = 0, perm_n = 0;
-};
-
-// plane pairs (i, j) with i + j <= level, low orders first
-static int level_pairs(int level, int a_planes, int b_planes, int* pa, int* pb) {
-  int np = 0;
-  for (int s = 0; s <= level && np < 6; ++s)
-    for (int i = 0; i <= s && np < 6; ++i) {
-      const int j = s - i;
-      if (i < a_planes && j < b_planes) {
-        pa[np] = i;
-        pb[np] = j;
-        ++np;
-      }
-    }
-  return np;
-}
-
 // triage: ACX_MAIN_CTAS / ACX_SIDE_CTAS cap the persistent grids of the tensor-core kernels of lane 0 / the side lanes
 static int lane_cta_cap(const acx_learner* l, int lane_index) {
   static int caps[2] = {-2, -2};
@@ -646,49 +405,10 @@ static int lane_cta_cap(const acx_learner* l, int lane_index) {
   return (l->cfg.acktr && l->lanes > 1 && !l->profiling) ? 132 : 0;
 }
 
-static ConvGeom geom_of(const Layer& L) { return ConvGeom{L.hw_in, L.cin, L.k, L.s, L.hw_out, L.C}; }
-
 static int run_gemm(acx_learner* l, const Planes& a, const Planes& b, int trans, int m, int n, int k, int level, float alpha,
                     int symmetric, const GemmOut& o, const Lane& ln) {
   acx_gemm_t g;
-  memset(&g, 0, sizeof(g));
-  for (int i = 0; i < a.n; ++i) g.a.planes[i] = a.p[i];
-  for (int i = 0; i < b.n; ++i) g.b.planes[i] = b.p[i];
-  g.a.num_planes = a.n;
-  g.b.num_planes = b.n;
-  g.a.ld = a.ld;
-  g.b.ld = b.ld;
-  if (trans) {
-    g.a.rows = k; g.a.cols = m; g.b.rows = k; g.b.cols = n;
-  } else {
-    g.a.rows = m; g.a.cols = k; g.b.rows = n; g.b.cols = k;
-  }
-  g.trans_a = g.trans_b = trans;
-  g.m = m; g.n = n; g.k = k;
-  g.num_pairs = level_pairs(level, a.n, b.n, g.pair_a, g.pair_b);
-  g.alpha = alpha;
-  g.bias = o.bias;
-  g.relu = o.relu;
-  g.symmetric = symmetric;
-  g.c = o.c;
-  g.ldc = o.ldc;
-  if (o.planes) {
-    for (int i = 0; i < o.planes->n; ++i) g.c_planes[i] = o.planes->p[i];
-    g.c_num_planes = o.planes->n;
-    g.ldc_planes = o.planes->ld;
-  }
-  g.mask_plane = o.mask;
-  g.mask_ld = o.mask_ld;
-  g.mask_rows = o.mask_rows;
-  g.a_patch_u8 = o.a_patch;
-  g.a_patch_samples = o.a_patch_samples;
-  g.a_gather = o.a_gather;
-  g.b_gather = o.b_gather;
-  g.perm_m = o.perm_m;
-  g.perm_n = o.perm_n;
-  g.splits = 0;
-  g.workspace = ln.sc->ws;
-  g.workspace_bytes = ln.sc->ws_bytes;
+  fill_gemm(&g, a, b, trans, m, n, k, level, alpha, symmetric, o, ln.sc->ws, ln.sc->ws_bytes);
   set_cta_cap(lane_cta_cap(l, ln.index));
   const int r = gemm_dispatch(&g, l->cfg.gemm_impl, ln.st);
   set_cta_cap(0);
@@ -702,19 +422,13 @@ static void mark(acx_learner* l, int k, cudaStream_t st) {
   l->ev_set[k] = true;
 }
 
-#define ACX_TRY(expr)        \
-  do {                       \
-    int _r = (expr);         \
-    if (_r) return _r;       \
-  } while (0)
-
 static int refresh_weight_planes(acx_learner* l, cudaStream_t st, bool on_lanes = false) {
   const float* w[4];
   int kr[4], cc[4], ldt[4], ldn[4];
   bf16* t[4][3];
   bf16* n[4][3];
   for (int i = 0; i < 4; ++i) {
-    const Layer& L = l->L[i];
+    const Block& L = l->blk[i];
     w[i] = l->params + L.off;
     kr[i] = L.K;
     cc[i] = L.C;
@@ -731,14 +445,13 @@ static int refresh_weight_planes(acx_learner* l, cudaStream_t st, bool on_lanes 
   const bool fork = on_lanes && l->lanes > 1 && !l->profiling && st != nullptr;
   for (int i = 1; i <= 2; ++i)
     if (l->conv_tc[i]) {
-      const Layer& L = l->L[i];
-      const ConvGeom g = {L.hw_in, L.cin, L.k, L.s, L.hw_out, L.C};
+      const float* w = l->params + l->blk[i].off;
       const Lane& ln = side[i - 1];
       if (fork && ln.index != 0) {
         ACX_TRY(fork_lane(l, st, ln));
-        ACX_TRY(conv_dgrad_weight_planes(l->params + L.off, g, l->wD[i], ln.st));
+        ACX_TRY(conv_dgrad_weight_planes(w, geom_of(l, i), l->wD[i], ln.st));
       } else {
-        ACX_TRY(conv_dgrad_weight_planes(l->params + L.off, g, l->wD[i], st));
+        ACX_TRY(conv_dgrad_weight_planes(w, geom_of(l, i), l->wD[i], st));
       }
     }
   ACX_TRY(weight_planes(w, kr, cc, t, ldt, n, ldn, 4, st, l->gather ? 1 : 0));   // gather: conv1's W^T columns in the row-pair copy's order
@@ -768,7 +481,8 @@ static int input_factor(acx_learner* l, int fac, const Planes& x, int rows, int 
 static int conv_input_factor(acx_learner* l, int li, const Planes& patches, const uint8_t* obs_u8, const Planes* act_in,
                              float scale_sq, float border_scale, const Lane& ln, const Lane& lb) {
   const Layer& L = l->L[li];
-  const int d = L.K + 1, rows = l->N * L.T;
+  const Block& B = l->blk[li];
+  const int d = B.K + 1, rows = l->N * L.T;
   float* dst = l->stats + l->aoff[li];
   GemmOut o;
   o.c = dst;
@@ -786,9 +500,9 @@ static int conv_input_factor(acx_learner* l, int li, const Planes& patches, cons
     x.n = l->gat_x[li].num_planes;
     x.ld = 8;
     for (int i = 0; i < x.n; ++i) x.p[i] = reinterpret_cast<bf16*>(const_cast<void*>(l->gat_x[li].planes[i]));
-    ACX_TRY(run_gemm(l, x, x, 1, L.K, L.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
+    ACX_TRY(run_gemm(l, x, x, 1, B.K, B.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
   } else {
-    ACX_TRY(run_gemm(l, first_planes(patches, o.a_patch ? 1 : patches.n), patches, 1, L.K, L.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
+    ACX_TRY(run_gemm(l, first_planes(patches, o.a_patch ? 1 : patches.n), patches, 1, B.K, B.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
   }
   ACX_TRY(conv_border(obs_u8, act_in, l->N, L.hw_in, L.cin, L.k, L.s, L.hw_out, border_scale, lb.sc->colsum_partial, kBorderChunks,
                       lb.sc->colsum_tmp + 4096, dst, d, lb.st));
@@ -848,14 +562,15 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
   };
   auto conv_layer = [&](int li, const Planes& in, const Planes& patches, const Planes& out) -> int {
     const Layer& L = l->L[li];
+    const Block& B = l->blk[li];
     GemmOut o;
     o.relu = 1;
-    o.bias = l->params + L.off + (size_t)L.K * L.C;
+    o.bias = l->params + B.off + (size_t)B.K * B.C;
     o.planes = &out;
     if (!l->conv_fwd_tc[li]) {
       ACX_TRY(im2col_bf16(in, patches, rows * L.T, L.hw_in, L.cin, L.k, L.s, L.hw_out, st));
       ACX_TRY(factor(li));
-      return run_gemm(l, patches, l->wT[li], 0, rows * L.T, L.C, L.K, l->lvl_fwd, 1.0f, 0, o, ln);
+      return run_gemm(l, patches, l->wT[li], 0, rows * L.T, B.C, B.K, l->lvl_fwd, 1.0f, 0, o, ln);
     }
     if (aux && ((l->gather_mask >> li) & 1)) {
       ACX_TRY(factor(li));   // the input factor reads the layer's input in place: nothing to build
@@ -868,7 +583,7 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
     int pa[6], pb[6];
     const int np = level_pairs(l->lvl_fwd, in.n, l->wT[li].n, pa, pb);
     set_cta_cap(lane_cta_cap(l, 0));
-    const int rc = conv_tc_forward(in, l->wT[li], geom_of(L), rows, o.bias, 1, out, np, pa, pb, st);
+    const int rc = conv_tc_forward(in, l->wT[li], geom_of(l, li), rows, o.bias, 1, out, np, pa, pb, st);
     set_cta_cap(0);
     return rc;
   };
@@ -876,7 +591,7 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
   o.relu = 1;
   // conv1: raw bytes are exact in bf16; the /255 of envs/atari/model.py:93 is the GEMM alpha
   // (with conv1_patch the GEMMs build the patch tiles themselves from `obs`: no im2col pass, no P1)
-  o.bias = l->params + l->L[0].off + (size_t)l->L[0].K * l->L[0].C;
+  o.bias = l->params + l->blk[0].off + (size_t)l->blk[0].K * l->blk[0].C;
   o.planes = &l->act1;
   if (l->gather) {
     // the row-pair interleaved bf16 copy of the observations replaces P1 (2x instead of 7.2x the observations, L2 resident);
@@ -903,22 +618,22 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
   ACX_TRY(conv_layer(2, l->act2, l->P3, l->act3));
   ACX_TRY(factor(3));
   // fc4 on the (h, w, c)-flattened conv3 output (nn.py:125-126)
-  o.bias = l->params + l->L[3].off + (size_t)l->L[3].K * l->L[3].C;
+  o.bias = l->params + l->blk[3].off + (size_t)l->blk[3].K * l->blk[3].C;
   o.planes = &l->act4;
   ACX_TRY(run_gemm(l, with_ld(l->act3, 49 * c3), l->wT[3], 0, rows, 512, 49 * c3, l->lvl_fwd, 1.0f, 0, o, ln));
   ACX_TRY(factor(4));
-  ACX_TRY(heads_fwd(l->act4, l->params + l->L[4].off, l->params + l->L[5].off, rows, l->A, l->logits, l->values, st));
+  ACX_TRY(heads_fwd(l->act4, l->params + l->blk[4].off, l->params + l->blk[5].off, rows, l->A, l->logits, l->values, st));
   return 0;
 }
 
 // weight gradient V_l[:K] = X^T g over the true-loss rows, bias row = column sums of g
 static int bias_grad(acx_learner* l, int li, const Planes& g, int rows, const Lane& ln) {
-  const Layer& L = l->L[li];
+  const Block& L = l->blk[li];
   return colsum(g, rows, L.C, 1.0f, ln.sc->colsum_partial, kColsumChunks, l->grads + L.off + (size_t)L.K * L.C, 1, ln.st);
 }
 static int weight_grad(acx_learner* l, int li, const Planes& x, const Planes& g, int rows, float alpha, const Lane& ln,
                        bool with_bias = true) {
-  const Layer& L = l->L[li];
+  const Block& L = l->blk[li];
   GemmOut o;
   o.c = l->grads + L.off;
   o.ldc = L.C;
@@ -948,6 +663,7 @@ static int weight_grad(acx_learner* l, int li, const Planes& x, const Planes& g,
 static int conv_dgrad(acx_learner* l, int li, const Planes& g, const bf16* act_below_hi, const Planes& g_below, int samples,
                       const Lane& ln) {
   const Layer& L = l->L[li];
+  const Block& B = l->blk[li];
   if (l->conv_tc[li]) {   // gather form on the tensor cores: no dP matrix, no col2im pass (conv.cu)
     int pa[6], pb[6];
     const int np = level_pairs(l->lvl_bwd, g.n, l->wD[li].n, pa, pb);
@@ -958,20 +674,20 @@ static int conv_dgrad(acx_learner* l, int li, const Planes& g, const bf16* act_b
     const int np_lo = level_pairs(l->lvl_fisher, g.n, l->wD[li].n, pa2, pb2);
     const bool lo = samples > l->N && np_lo < np;
     set_cta_cap(lane_cta_cap(l, ln.index));
-    const int rc = conv_tc_dgrad(g, l->wD[li], geom_of(L), samples, act_below_hi, l->N, g_below, np, pa, pb, ln.st, lo ? l->N : -1,
+    const int rc = conv_tc_dgrad(g, l->wD[li], geom_of(l, li), samples, act_below_hi, l->N, g_below, np, pa, pb, ln.st, lo ? l->N : -1,
                                  np_lo);
     set_cta_cap(0);
     return rc;
   }
-  const size_t per_sample = (size_t)L.T * L.K * sizeof(float);
+  const size_t per_sample = (size_t)L.T * B.K * sizeof(float);
   int chunk = (int)(l->dgrad_chunk_bytes / per_sample);
   if (chunk < 1) chunk = 1;
   for (int n0 = 0; n0 < samples; n0 += chunk) {
     const int ns = std::min(chunk, samples - n0);
     GemmOut o;
     o.c = l->dP;
-    o.ldc = L.K;
-    ACX_TRY(run_gemm(l, offset_rows(g, (size_t)n0 * L.T), l->wN[li], 0, ns * L.T, L.K, L.C, l->lvl_bwd, 1.0f, 0, o, ln));
+    o.ldc = B.K;
+    ACX_TRY(run_gemm(l, offset_rows(g, (size_t)n0 * L.T), l->wN[li], 0, ns * L.T, B.K, B.C, l->lvl_bwd, 1.0f, 0, o, ln));
     ACX_TRY(col2im_mask_split(l->dP, act_below_hi, g_below, n0, ns, l->N, L.hw_in, L.cin, L.k, L.s, L.hw_out, ln.st));
   }
   return 0;
@@ -979,7 +695,7 @@ static int conv_dgrad(acx_learner* l, int li, const Planes& g, const bf16* act_b
 
 // output factor G_l = g^T g / rows over the Fisher-sample rows
 static int output_factor(acx_learner* l, int li, const Planes& g_fisher, int rows, const Lane& ln) {
-  const Layer& L = l->L[li];
+  const Block& L = l->blk[li];
   // Narrow output factors (C = 32 / 64 fill a 128 x 64 MMA tile to 1/8 .. 1/2) still run faster as a split-K SYRK on the
   // tensor cores than on the fp32 SIMT Gram kernel (measured: 1.067 -> 1.043 ms/update; the MMAs are nearly free next to
   // the one pass over g).  ACX_GRAM_TC=0 selects the SIMT kernel.
@@ -1003,8 +719,7 @@ static int output_factor(acx_learner* l, int li, const Planes& g_fisher, int row
 // With one lane (profiling, ACX lanes = 1) the same calls run back to back on the caller's stream.
 static int issue_phase1(acx_learner* l, const int32_t* fisher_labels, const float* fisher_eps, cudaStream_t st) {
   const int N = l->N, E = l->E, T = l->T, A = l->A, c3 = l->c3;
-  const bool acktr = l->cfg.acktr != 0;
-  const bool fisher = acktr && l->gs >= l->cfg.num_cold_updates;   // kfac_utils.py:42-44: covariances only after the cold phase
+  const bool fisher = l->sch.fisher();
   const int RB = fisher ? 2 * N : N;
   l->ev_next = 0;
   for (cudaEvent_t& e : l->patches_ready) e = nullptr;
@@ -1027,8 +742,8 @@ static int issue_phase1(acx_learner* l, const int32_t* fisher_labels, const floa
   ACX_TRY(returns_loss_grad(l->rewards, l->terminals, l->values + N, l->cfg.gamma, E, T, l->targets, l->adv, l->logits, l->values,
                             l->actions, fisher_labels, fisher_eps, l->cfg.seed, l->sched, A, l->cfg.entropy_beta, l->value_weight,
                             l->dheads, l->bscalars, fisher ? 1 : 0, st, l->policy_weight));
-  ACX_TRY(heads_bwd(l->dheads, l->params + l->L[4].off, l->params + l->L[5].off, l->act4, N, RB, A, l->dpre4,
-                    l->grads + l->L[4].off, l->grads + l->L[5].off, st));
+  ACX_TRY(heads_bwd(l->dheads, l->params + l->blk[4].off, l->params + l->blk[5].off, l->act4, N, RB, A, l->dpre4,
+                    l->grads + l->blk[4].off, l->grads + l->blk[5].off, st));
   const Planes flat3 = with_ld(l->act3, 49 * c3);
   mark(l, 2, st);
   // ---- fc4
@@ -1095,7 +810,7 @@ static int precondition(acx_learner* l, cudaStream_t st) {
   ACX_TRY(fork_lane(l, st, small_ln));
   ACX_TRY(precondition_small(l->d_pjobs, l->num_pjobs, l->pjobs_max_d, small_ln.st));
   for (int i = 0; i < 6; ++i) {
-    const Layer& L = l->L[i];
+    const Block& L = l->blk[i];
     const int d = L.K + 1, C = L.C;
     if (C <= 64) continue;   // done above
     Planes vp = l->Vp;
@@ -1118,41 +833,7 @@ static int precondition(acx_learner* l, cudaStream_t st) {
 // SURVEY A.7-U3: the 1 / (1 - decay^n) factor belongs to zero-initialised running sums
 static bool zero_debias_on(const acx_learner_config_t& c) { return !c.no_zero_debias && !c.cov_init_identity; }
 
-// what one phase-2 call does, decided on the host from the schedule counters (kfac_utils.py:38-53)
-struct Plan2 {
-  bool a2c, cold, invert, kfac_apply, refresh;
-  int key() const { return (a2c ? 1 : 0) | (cold ? 2 : 0) | (invert ? 4 : 0) | (kfac_apply ? 8 : 0) | (refresh ? 16 : 0); }
-};
-
-static Plan2 plan_phase2(const acx_learner* l) {
-  const acx_learner_config_t& c = l->cfg;
-  Plan2 p = {false, false, false, false, false};
-  if (!c.acktr) {
-    p.a2c = true;
-    p.refresh = true;
-    return p;
-  }
-  p.cold = l->gs < c.num_cold_updates;
-  const int64_t gs1 = l->gs + (p.cold ? 1 : 0);   // the cold optimizer increments global_step itself (kfac_utils.py:43)
-  p.invert = gs1 > c.num_cold_updates && (gs1 - c.num_cold_updates) % c.invert_every == 0;   // kfac_utils.py:47-50
-  // kfac_utils.py:52-53 runs always; with kfac's zero-initialised inverses it is exactly a no-op (U = 0, v stays 0)
-  // until the first refresh, so only the step counter moves.
-  p.kfac_apply = l->inverses_valid || p.invert;
-  p.refresh = p.cold || p.kfac_apply;
-  return p;
-}
-
-static void advance_phase2(acx_learner* l, const Plan2& p) {
-  if (p.a2c) {
-    l->gs += 1;
-    return;
-  }
-  if (p.cold) l->gs += 1; else l->ncov += 1;
-  if (p.invert) l->inverses_valid = true;
-  l->gs += 1;
-}
-
-static int issue_phase2(acx_learner* l, const Plan2& p, cudaStream_t st) {
+static int issue_phase2(acx_learner* l, const Plan& p, cudaStream_t st) {
   const acx_learner_config_t& c = l->cfg;
   const size_t P = l->num_params;
   l->ev_next = 0;
@@ -1227,22 +908,15 @@ static int issue_phase2(acx_learner* l, const Plan2& p, cudaStream_t st) {
       const char* e = getenv("ACX_INV_IMPL");
       inv_impl = e ? atoi(e) : 2;
     }
-    int done = 0;
-    if (inv_impl == 2) {
-      const int r = spd_inverse_resident(l->h_jobs, 12, l->sched, l->damp, l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims, l->d_g_dims,
-                                         l->lambdas, 6, l->inv_bar, st);
-      if (r > 0) return r;
-      done = r == 0;
-    } else if (inv_impl == 1) {
+    // (the serial pivot-block inversions of the chain run on a side lane next to the trailing updates, joined inside, step by step)
+    const cudaStream_t side = lane_of(l, 1, st).st;
+    if (inv_impl == 2)
+      ACX_TRY(l->invert(st, side));
+    else if (inv_impl == 1)
       ACX_TRY(spd_inverse_persistent(l->h_jobs, l->d_jobs, 12, l->sched, l->damp, l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims,
                                      l->d_g_dims, l->lambdas, 6, l->inv_bar, st));
-      done = 1;
-    }
-    if (!done) {
-      ACX_TRY(compute_dampings(l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims, l->d_g_dims, l->lambdas, 6, l->damp, st));
-      // the serial pivot-block inversions run on a side lane next to the trailing updates (joined inside, step by step)
-      ACX_TRY(spd_inverse_batched(l->h_jobs, l->d_jobs, 12, l->sched, l->damp, st, lane_of(l, 1, st).st));
-    }
+    else
+      ACX_TRY(l->invert_chain(st, side));
   }
   mark(l, 7, st);
   if (p.kfac_apply) {
@@ -1261,60 +935,17 @@ static int issue_phase2(acx_learner* l, const Plan2& p, cudaStream_t st) {
   return 0;
 }
 
-// ------------------------------------------------------------------------------------------------
-// CUDA-graph cache: the first use of a (phase, variant) runs eagerly (it also performs one-time host work such as
-// tensor-map encoding and function attributes), the second is captured and instantiated, later uses replay the graph.
-// Valid because no kernel takes a step-dependent scalar by value (see Sched).
-// ------------------------------------------------------------------------------------------------
-template <typename F>
-static int run_cached(acx_learner* l, const GraphKey& key, cudaStream_t st, F&& issue) {
-  if (!l->cfg.use_graphs || l->profiling || st == nullptr) return issue();
-  {
-    // the caller is capturing this stream itself (e.g. a whole rollout as one graph): the launches simply become nodes
-    // of the caller's graph
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) return issue();
-  }
-  GraphEntry& ge = l->graphs[key];
-  if (ge.uses == 0) {
-    ge.uses = 1;
-    return issue();
-  }
-  if (ge.exec == nullptr) {
-    const uint64_t before = g_launch_count;
-    ACX_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    const int r = issue();
-    cudaGraph_t graph = nullptr;
-    const cudaError_t e = cudaStreamEndCapture(st, &graph);
-    if (r != 0 || e != cudaSuccess || graph == nullptr) {
-      if (graph) cudaGraphDestroy(graph);
-      if (r == 0) set_error(std::string("graph capture failed: ") + cudaGetErrorString(e));
-      return r ? r : 4;
-    }
-    ge.launches = g_launch_count - before;
-    g_launch_count = before;
-    const cudaError_t e2 = cudaGraphInstantiate(&ge.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (e2 != cudaSuccess) {
-      ge.exec = nullptr;
-      set_error(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e2));
-      return 4;
-    }
-  }
-  ACX_CUDA(cudaGraphLaunch(ge.exec, st));
-  count_launch((int)ge.launches);
-  ge.uses += 1;
-  return 0;
-}
+// graphs are off, or stage timing brackets the work with events on the caller's stream
+static bool eager_graphs(const acx_learner* l) { return !l->cfg.use_graphs || l->profiling; }
 
 static int phase2(acx_learner* l, cudaStream_t st) {
-  const Plan2 p = plan_phase2(l);
+  const Plan p = l->sch.plan();
   if (p.a2c || p.cold) l->deferred = 0;   // no covariance update in this phase: nothing can have been left to it
   GraphKey key = {2, p.key() | (l->deferred << 5) | (l->external_ema ? 1 << 10 : 0) | (l->peer.world > 1 ? 1 << 11 : 0), nullptr, nullptr};
-  const int r = run_cached(l, key, st, [&]() { return issue_phase2(l, p, st); });
+  const int r = l->graphs.run(key, st, eager_graphs(l), [&]() { return issue_phase2(l, p, st); });
   if (r) return r;
   l->deferred = 0;
-  advance_phase2(l, p);
+  l->sch.advance(p);
   return 0;
 }
 
@@ -1382,6 +1013,9 @@ static void init_dims(acx_learner* l, const acx_learner_config_t* cfg) {
   l->A = cfg->num_actions;
   l->c3 = cfg->conv3_filters;
   setup_layers(l);
+  l->sch.acktr = cfg->acktr != 0;
+  l->sch.num_cold_updates = cfg->num_cold_updates;
+  l->sch.invert_every = cfg->invert_every;
 }
 
 size_t acx_learner_arena_bytes(const acx_learner_config_t* cfg) {
@@ -1405,16 +1039,13 @@ acx_learner_t* acx_learner_create(const acx_learner_config_t* cfg, void* d_arena
   l->arena_base = reinterpret_cast<uint8_t*>(d_arena);
   setup_gather(l);
   register_buffers(l);
-  l->gs = 0;
-  l->ncov = 0;
   l->value_weight = cfg->value_loss_weight;
-  l->inverses_valid = false;
   l->act_calls = 0;
   l->lanes = cfg->num_lanes <= 0 ? kMaxLanes : std::min(cfg->num_lanes, kMaxLanes);
   if (cudaEventCreateWithFlags(&l->a_ready, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&l->reduced, cudaEventDisableTiming) != cudaSuccess) {
     acx::set_error("acx_learner_create: cudaEventCreateWithFlags failed");
-    delete l;
+    acx_learner_destroy(l);
     return nullptr;
   }
   {
@@ -1426,11 +1057,9 @@ acx_learner_t* acx_learner_create(const acx_learner_config_t* cfg, void* d_arena
     l->conv1_patch = cfg->gemm_impl == 0 && e != nullptr && atoi(e) != 0;
   }
   // implicit-GEMM forward of conv2 / conv3 only pays when its patch matrix can be built concurrently on another lane
-  for (int i = 0; i < 4; ++i) {
-    const ConvGeom g = {l->L[i].hw_in, l->L[i].cin, l->L[i].k, l->L[i].s, l->L[i].hw_out, l->L[i].C};
+  for (int i = 0; i < 4; ++i)
     l->conv_fwd_tc[i] = (i == 1 || i == 2) && l->cfg.conv_impl == 0 && l->cfg.gemm_impl == 0 && (l->lanes > 1 || l->gather) && fwd_tc_enabled() &&
-                        conv_tc_supported(g, 0);
-  }
+                        conv_tc_supported(geom_of(l, i), 0);
   int prio_lo = 0, prio_hi = 0;
   cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // (numerically lowest = highest priority)
   const char* pe = getenv("ACX_SIDE_PRIO");               // 1: side lanes at the lowest stream priority (triage)
@@ -1438,69 +1067,42 @@ acx_learner_t* acx_learner_create(const acx_learner_config_t* cfg, void* d_arena
   for (int i = 0; i + 1 < l->lanes; ++i)
     if (cudaStreamCreateWithPriority(&l->side[i], cudaStreamNonBlocking, side_prio) != cudaSuccess) {
       acx::set_error("acx_learner_create: cudaStreamCreateWithFlags failed");
-      delete l;
+      acx_learner_destroy(l);
       return nullptr;
     }
-  // zero everything persistent; RMSProp's ms starts at one (TF-1 default)
-  cudaError_t e = cudaMemset(d_arena, 0, need);
-  if (e != cudaSuccess) {
-    acx::set_error(std::string("acx_learner_create: cudaMemset: ") + cudaGetErrorString(e));
-    delete l;
+  // zero everything persistent, then the initial schedule, optimizer slots and K-FAC tables
+  if (l->upload(d_arena, need, !cfg->acktr, cfg->lr_start, cfg->damping) != 0) {
+    acx_learner_destroy(l);
     return nullptr;
   }
-  std::vector<float> ones;
-  if (!cfg->acktr) {
-    ones.assign(l->params_pad, 1.0f);
-    cudaMemcpy(l->accum, ones.data(), l->params_pad * 4, cudaMemcpyHostToDevice);
-  }
-  Sched s0 = {0ull, 0ull, cfg->lr_start, 1.0f};
-  cudaMemcpy(l->sched, &s0, sizeof(s0), cudaMemcpyHostToDevice);
   if (cfg->acktr && (cfg->cov_init_identity || cfg->inv_init_identity)) {   // SURVEY A.7-U3 (the arena is zero so far)
     std::vector<float> eye;
+    cudaError_t e = cudaSuccess;
     auto put_eye = [&](float* dst, int d) {
       eye.assign((size_t)d * d, 0.0f);
       for (int i = 0; i < d; ++i) eye[(size_t)i * d + i] = 1.0f;
-      cudaMemcpy(dst, eye.data(), eye.size() * sizeof(float), cudaMemcpyHostToDevice);
+      if (e == cudaSuccess) e = cudaMemcpy(dst, eye.data(), eye.size() * sizeof(float), cudaMemcpyHostToDevice);
     };
     if (cfg->cov_init_identity) {
       for (int i = 0; i < 5; ++i) put_eye(l->sums + l->aoff[i], l->adim[i]);
-      for (int i = 0; i < 6; ++i) put_eye(l->sums + l->goff[i], l->L[i].C);
+      for (int i = 0; i < 6; ++i) put_eye(l->sums + l->goff[i], l->blk[i].C);
     }
     if (cfg->inv_init_identity) {
       for (int i = 0; i < 6; ++i) {
-        put_eye(l->inv + l->ainv_off[i], l->L[i].K + 1);
-        put_eye(l->inv + l->ginv_off[i], l->L[i].C);
+        put_eye(l->inv + l->ainv_off[i], l->blk[i].K + 1);
+        put_eye(l->inv + l->ginv_off[i], l->blk[i].C);
       }
-      l->inverses_valid = true;   // the K-FAC apply is a real step from the first update on
+      l->sch.inverses_valid = true;   // the K-FAC apply is a real step from the first update on
     }
-  }
-  const float* ap[6];
-  const float* gp[6];
-  int ad[6], gd[6];
-  float lam[8] = {0};
-  for (int i = 0; i < 6; ++i) {
-    ap[i] = l->sums + l->aoff[l->L[i].afac];
-    gp[i] = l->sums + l->goff[i];
-    ad[i] = l->adim[l->L[i].afac];
-    gd[i] = l->L[i].C;
-    lam[i] = cfg->damping / (float)l->L[i].Tnorm;
-  }
-  cudaMemcpy(l->d_a_ptrs, ap, sizeof(ap), cudaMemcpyHostToDevice);
-  cudaMemcpy(l->d_g_ptrs, gp, sizeof(gp), cudaMemcpyHostToDevice);
-  cudaMemcpy(l->d_a_dims, ad, sizeof(ad), cudaMemcpyHostToDevice);
-  cudaMemcpy(l->d_g_dims, gd, sizeof(gd), cudaMemcpyHostToDevice);
-  cudaMemcpy(l->lambdas, lam, sizeof(lam), cudaMemcpyHostToDevice);
-  std::stable_sort(l->h_jobs, l->h_jobs + 12, [](const InvJob& a, const InvJob& b) { return a.n > b.n; });
-  cudaMemcpy(l->d_pjobs, l->h_pjobs, sizeof(l->h_pjobs), cudaMemcpyHostToDevice);
-  e = cudaMemcpy(l->d_jobs, l->h_jobs, sizeof(l->h_jobs), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) {
-    acx::set_error(std::string("acx_learner_create: cudaMemcpy: ") + cudaGetErrorString(e));
-    delete l;
-    return nullptr;
+    if (e != cudaSuccess) {
+      acx::set_error(std::string("acx_learner_create: cudaMemcpy: ") + cudaGetErrorString(e));
+      acx_learner_destroy(l);
+      return nullptr;
+    }
   }
   if (cfg->acktr && cfg->inv_init_identity) {   // bf16 operand planes of the identity inverses
     if (acx_learner_refresh_weights(l, nullptr) != 0 || cudaDeviceSynchronize() != cudaSuccess) {
-      delete l;
+      acx_learner_destroy(l);
       return nullptr;
     }
   }
@@ -1508,18 +1110,15 @@ acx_learner_t* acx_learner_create(const acx_learner_config_t* cfg, void* d_arena
 }
 
 void acx_learner_destroy(acx_learner_t* l) {
-  if (l)
-    for (auto& kv : l->graphs)
-      if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-  if (l && l->profiling)
+  if (!l) return;
+  if (l->profiling)
     for (int k = 0; k < ACX_NUM_STAGES + 2; ++k) cudaEventDestroy(l->ev[k]);
-  if (l) {
-    for (cudaEvent_t e : l->lane_events) cudaEventDestroy(e);
-    if (l->a_ready) cudaEventDestroy(l->a_ready);
-    for (cudaStream_t s : l->side)
-      if (s) cudaStreamDestroy(s);
-  }
-  delete l;
+  for (cudaEvent_t e : l->lane_events) cudaEventDestroy(e);
+  if (l->a_ready) cudaEventDestroy(l->a_ready);
+  if (l->reduced) cudaEventDestroy(l->reduced);
+  for (cudaStream_t s : l->side)
+    if (s) cudaStreamDestroy(s);
+  delete l;   // the graph cache destroys its executable graphs
 }
 
 int acx_learner_set_profiling(acx_learner_t* l, int enable) {
@@ -1559,58 +1158,37 @@ size_t acx_learner_num_params(const acx_learner_t* l) { return l ? l->num_params
 int acx_learner_set_params(acx_learner_t* l, const float* h_params, void* stream) {
   ACX_CHECK(l && h_params, "null argument");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  ACX_CUDA(cudaMemcpyAsync(l->params, h_params, l->num_params * sizeof(float), cudaMemcpyHostToDevice, st));
-  int r = refresh_weight_planes(l, st);
-  if (r) return r;
+  ACX_TRY(l->set_params(h_params, st));
+  ACX_TRY(refresh_weight_planes(l, st));
   ACX_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
 
 int acx_learner_get_params(acx_learner_t* l, float* h_params, void* stream) {
   ACX_CHECK(l && h_params, "null argument");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  ACX_CUDA(cudaMemcpyAsync(h_params, l->params, l->num_params * sizeof(float), cudaMemcpyDeviceToHost, st));
-  ACX_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return l->get_params(h_params, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int acx_learner_refresh_weights(acx_learner_t* l, void* stream) {
   ACX_CHECK(l, "null learner");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  int r = refresh_weight_planes(l, st);
-  if (r) return r;
-  for (int i = 0; i < 6; ++i) {   // the bf16 planes of the stored inverses are derived state too
-    const int d = l->L[i].K + 1, c = l->L[i].C;
-    r = split_planes(l->inv + l->ainv_off[i], d, d, d, 1.0f, l->ainv_pl[i].p[0], l->ainv_pl[i].p[1], l->ainv_pl[i].p[2], 3,
-                     l->ainv_pl[i].ld, st);
-    if (r) return r;
-    r = split_planes(l->inv + l->ginv_off[i], c, c, c, 1.0f, l->ginv_pl[i].p[0], l->ginv_pl[i].p[1], l->ginv_pl[i].p[2], 3,
-                     l->ginv_pl[i].ld, st);
-    if (r) return r;
-  }
-  return 0;
+  ACX_TRY(refresh_weight_planes(l, st));
+  return l->split_inverses(st);
 }
 
 void* acx_learner_buffer(acx_learner_t* l, const char* name, size_t* num_bytes) {
-  if (!l || !name) return nullptr;
-  auto it = l->named.find(name);
-  if (it == l->named.end()) {
-    acx::set_error(std::string("acx_learner_buffer: unknown buffer '") + name + "'");
-    return nullptr;
-  }
-  if (num_bytes) *num_bytes = it->second.bytes;
-  return it->second.ptr;
+  return l ? l->buffer("acx_learner_buffer", name, num_bytes) : nullptr;
 }
 
 int acx_learner_phase1(acx_learner_t* l, const int32_t* d_fisher_labels, const float* d_fisher_eps, void* stream) {
   ACX_CHECK(l, "null learner");
   ACX_CHECK((d_fisher_labels == nullptr) == (d_fisher_eps == nullptr), "inject both Fisher labels and eps, or neither");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const bool fisher = l->cfg.acktr != 0 && l->gs >= l->cfg.num_cold_updates;
+  const bool fisher = l->sch.fisher();
   l->deferred = fisher ? resolve_deferred(l) : 0;
   l->defer_request = 0;   // one-shot
   GraphKey key = {1, (fisher ? 1 : 0) | (l->deferred << 1) | (l->loss_variant << 8), d_fisher_labels, d_fisher_eps};
-  const int r = run_cached(l, key, st, [&]() { return issue_phase1(l, d_fisher_labels, d_fisher_eps, st); });
+  const int r = l->graphs.run(key, st, eager_graphs(l), [&]() { return issue_phase1(l, d_fisher_labels, d_fisher_eps, st); });
   l->a_ready_valid = r == 0 && fisher && l->lanes > 1 && !l->profiling;
   return r;
 }
@@ -1638,28 +1216,28 @@ int acx_learner_update(acx_learner_t* l, const int32_t* d_fisher_labels, const f
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   // both phases as ONE captured graph per schedule variant (nothing has to happen between them unless the caller runs a
   // collective there): one graph launch per update
-  const bool fisher = l->cfg.acktr != 0 && l->gs >= l->cfg.num_cold_updates;
+  const bool fisher = l->sch.fisher();
   l->deferred = fisher ? resolve_deferred(l) : 0;
   l->defer_request = 0;
-  const Plan2 p = plan_phase2(l);
+  const Plan p = l->sch.plan();
   if (p.a2c || p.cold) l->deferred = 0;
   const int k1 = (fisher ? 1 : 0) | (l->deferred << 1) | (l->loss_variant << 8);
   const int k2 = p.key() | (l->external_ema ? 1 << 10 : 0) | (l->peer.world > 1 ? 1 << 11 : 0);
   GraphKey key = {4, k1 | (k2 << 16), d_fisher_labels, d_fisher_eps};
-  const int r = run_cached(l, key, st, [&]() {
+  const int r = l->graphs.run(key, st, eager_graphs(l), [&]() {
     const int r1 = issue_phase1(l, d_fisher_labels, d_fisher_eps, st);
     return r1 ? r1 : issue_phase2(l, p, st);
   });
   l->a_ready_valid = false;
   if (r) return r;
   l->deferred = 0;
-  advance_phase2(l, p);
+  l->sch.advance(p);
   return 0;
 }
 
 int acx_learner_update_plan(const acx_learner_t* l, int* has_factors, int* will_invert) {
   ACX_CHECK(l, "null learner");
-  const Plan2 p = plan_phase2(l);
+  const Plan p = l->sch.plan();
   if (has_factors) *has_factors = (!p.a2c && !p.cold) ? 1 : 0;
   if (will_invert) *will_invert = p.invert ? 1 : 0;
   return 0;
@@ -1735,31 +1313,18 @@ int acx_learner_phase2(acx_learner_t* l, void* stream) {
   return phase2(l, reinterpret_cast<cudaStream_t>(stream));
 }
 
-int64_t acx_learner_global_step(const acx_learner_t* l) { return l ? l->gs : -1; }
+int64_t acx_learner_global_step(const acx_learner_t* l) { return l ? l->sch.gs : -1; }
 
 int acx_learner_set_state(acx_learner_t* l, int64_t global_step, int64_t num_cov_updates, int inverses_valid, void* stream) {
   ACX_CHECK(l, "null learner");
   ACX_CHECK(global_step >= 0 && num_cov_updates >= 0, "negative counters");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  l->gs = global_step;
-  l->ncov = num_cov_updates;
-  l->inverses_valid = inverses_valid != 0;
-  Sched s;
-  s.gs = (unsigned long long)global_step;
-  s.ncov = (unsigned long long)num_cov_updates;
-  s.lr = l->cfg.lr_start;
-  s.debias = (num_cov_updates > 0 && zero_debias_on(l->cfg))
-                 ? (float)(1.0 / (1.0 - pow((double)l->cfg.cov_ema_decay, (double)num_cov_updates))) : 1.0f;
-  ACX_CUDA(cudaMemcpyAsync(l->sched, &s, sizeof(s), cudaMemcpyHostToDevice, st));
-  ACX_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return l->sch.set(global_step, num_cov_updates, inverses_valid, l->cfg.lr_start, l->cfg.cov_ema_decay, zero_debias_on(l->cfg),
+                    l->sched, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int acx_learner_get_state(const acx_learner_t* l, int64_t* global_step, int64_t* num_cov_updates, int* inverses_valid) {
   ACX_CHECK(l, "null learner");
-  if (global_step) *global_step = l->gs;
-  if (num_cov_updates) *num_cov_updates = l->ncov;
-  if (inverses_valid) *inverses_valid = l->inverses_valid ? 1 : 0;
+  l->sch.get(global_step, num_cov_updates, inverses_valid);
   return 0;
 }
 
@@ -1796,8 +1361,7 @@ int acx_learner_act(acx_learner_t* l, const uint8_t* d_obs, int rows, const floa
   };
   l->act_calls++;
   GraphKey key = {3, (greedy ? 1 : 0) | (rows << 1), d_obs, d_actions, d_uniform, d_logits, d_values};
-  if (l->graphs.size() > 512 && l->graphs.find(key) == l->graphs.end()) return issue();   // ever-changing buffers: do not hoard graphs
-  return run_cached(l, key, st, issue);
+  return l->graphs.run_bounded(key, st, eager_graphs(l), issue);
 }
 
 }  // extern "C"

@@ -4,7 +4,8 @@
 // kernels: every matrix product on the tcgen05 GEMM (gemm.cu), the loss / column sums / sampling of layers.cu, the EMA,
 // inverse refresh, preconditioning and optimizer steps of kfac.cu / kfac_inv.cu.  Only the two heads (any width, any
 // action count) have kernels of their own here.  Everything runs in order on the caller's stream; acx_mlp_update is one
-// captured CUDA graph per schedule variant.
+// captured CUDA graph per schedule variant.  The host code it shares with learner.cu (arena, K-FAC blocks and their state,
+// schedule, inverse refresh, graph cache) lives in learner_core.cuh / learner_core.cu.
 //   forward   obs -> bf16 planes; fc_i: GEMM with bias + ReLU + plane split in the epilogue; heads (one warp per row)
 //   loss      K-RET + A2C loss + output gradients + Fisher-sample output gradients (loss_grad_kernel), rows [0,N) true
 //             loss, rows [N,2N) Fisher samples
@@ -15,84 +16,16 @@
 //   phase 2   as learner.cu issue_phase2: schedule step, cold momentum / EMA, scheduled inverse refresh, preconditioning,
 //             KL clip + momentum + apply, or the A2C RMSProp step; then the weight operand planes
 #include <algorithm>
-#include <cmath>
-#include <map>
 #include <string>
-#include <tuple>
-#include <vector>
 
-#include "layers.cuh"
+#include "learner_core.cuh"
 
 namespace acx {
 namespace {
 
-constexpr int kMaxLayers = 6;        // 4 hidden layers + the two heads
-constexpr int kColsumChunks = 592;
-constexpr int kDotPartials = 296;
 constexpr int kActPlanes = 2;        // default preset: activations and gradients on 2 planes, 3 plane pairs ...
 constexpr int kLvl = 1;
 constexpr int kLvlPrecon = 2;        // ... weights, inverses and preconditioning operands on 3 planes, 6 pairs
-
-struct Block {
-  std::string name;
-  int K, C;          // V_l = [K+1, C]
-  size_t off;        // offset in the flat parameter vector
-  int afac;          // input factor (the two heads share one)
-};
-
-struct Buf {
-  void* ptr;
-  size_t bytes;
-};
-
-struct Arena {
-  uint8_t* base = nullptr;
-  size_t used = 0;
-  void* take(size_t bytes) {
-    used = align_up(used, 256);
-    void* p = base ? base + used : nullptr;
-    used += bytes;
-    return p;
-  }
-};
-
-struct GraphEntry {
-  int uses = 0;
-  cudaGraphExec_t exec = nullptr;
-  uint64_t launches = 0;
-};
-typedef std::tuple<int, const void*, const void*, const void*, const void*, const void*> GraphKey;
-
-int pad8(int x) { return (x + 7) / 8 * 8; }
-
-Planes take_planes(Arena& ar, int nplanes, size_t rows, int ld) {
-  Planes pl;
-  pl.n = nplanes;
-  pl.ld = ld;
-  for (int i = 0; i < nplanes; ++i) pl.p[i] = reinterpret_cast<bf16*>(ar.take(rows * (size_t)ld * sizeof(bf16)));
-  return pl;
-}
-
-Planes offset_rows(const Planes& p, size_t rows) {
-  Planes q = p;
-  for (int i = 0; i < p.n; ++i) q.p[i] = p.p[i] + rows * (size_t)p.ld;
-  return q;
-}
-
-// plane pairs (i, j) with i + j <= level, low orders first
-int level_pairs(int level, int a_planes, int b_planes, int* pa, int* pb) {
-  int np = 0;
-  for (int s = 0; s <= level && np < 6; ++s)
-    for (int i = 0; i <= s && np < 6; ++i) {
-      const int j = s - i;
-      if (i < a_planes && j < b_planes) {
-        pa[np] = i;
-        pb[np] = j;
-        ++np;
-      }
-    }
-  return np;
-}
 
 // ------------------------------------------------------------------------------------------------
 // heads of any width H and 1..31 actions (the Atari head kernels of layers.cu are fixed at 512 inputs)
@@ -198,31 +131,10 @@ __global__ void __launch_bounds__(128) mlp_heads_wgrad_kernel(const float* __res
 
 using namespace acx;
 
-struct acx_mlp {
+// the K-FAC blocks fc1 .. fcL, fc_policy, fc_baseline and their state (KfacBlocks), plus this model's activations
+struct acx_mlp : KfacBlocks {
   acx_mlp_config_t cfg;
-  int E, T, N, R, A, D, L, NL;
-  Block blk[kMaxLayers];
-  size_t num_params, params_pad;
-  int adim[kMaxLayers - 1];
-  size_t aoff[kMaxLayers - 1], goff[kMaxLayers], factor_floats;
-  size_t ainv_off[kMaxLayers], ginv_off[kMaxLayers], inv_floats;
-  // fp32 state
-  float *params, *velocity, *accum, *precon, *precon_w;
-  float *bucket, *stats, *grads, *bscalars;
-  size_t bucket_floats;
-  float *sums, *inv, *damp, *lambdas, *scalars;
-  Planes ainv_pl[kMaxLayers], ginv_pl[kMaxLayers];
-  Sched* sched;
-  const float** d_a_ptrs;
-  const float** d_g_ptrs;
-  int *d_a_dims, *d_g_dims;
-  InvJob h_jobs[2 * kMaxLayers];
-  InvJob* d_jobs;
-  unsigned int* inv_bar;
-  unsigned long long* act_counter;
-  PreconJob h_pjobs[kMaxLayers];
-  PreconJob* d_pjobs;
-  int num_pjobs, pjobs_max_d;
+  int E, T, N, R, A, D, L;
   // inputs
   float* obs;
   uint8_t *actions, *terminals;
@@ -236,21 +148,12 @@ struct acx_mlp {
   Planes Vp, Wt;             // preconditioning operands of blocks with C > 64
   float *dot_partials, *colsum_partial, *colsum_tmp, *ws;
   size_t ws_bytes;
-  // host mirror of the schedule
-  int64_t gs, ncov;
-  bool inverses_valid;
-  std::map<std::string, Buf> named;
-  std::map<GraphKey, GraphEntry> graphs;
+  Schedule sch;
+  GraphCache graphs;
 };
 
 namespace acx {
 namespace {
-
-#define ACX_TRY(expr)        \
-  do {                       \
-    int _r = (expr);         \
-    if (_r) return _r;       \
-  } while (0)
 
 void init_dims(acx_mlp* l, const acx_mlp_config_t* c) {
   l->cfg = *c;
@@ -261,10 +164,8 @@ void init_dims(acx_mlp* l, const acx_mlp_config_t* c) {
   l->A = c->num_actions;
   l->D = c->obs_dim;
   l->L = c->num_hidden;
-  l->NL = l->L + 2;
-  size_t off = 0;
   int in = l->D;
-  for (int i = 0; i < l->NL; ++i) {
+  for (int i = 0; i < l->L + 2; ++i) {
     Block& b = l->blk[i];
     if (i < l->L) {
       b.name = "fc" + std::to_string(i + 1);
@@ -278,111 +179,25 @@ void init_dims(acx_mlp* l, const acx_mlp_config_t* c) {
       b.C = i == l->L ? l->A : 1;
       b.afac = l->L;
     }
-    b.off = off;
-    off += (size_t)(b.K + 1) * b.C;
   }
-  l->num_params = off;
-  l->params_pad = align_up(off, 4);
-  size_t f = 0;
-  for (int i = 0; i <= l->L; ++i) {
-    l->adim[i] = (i < l->L ? l->blk[i].K : l->blk[l->L].K) + 1;
-    l->aoff[i] = f;
-    f += align_up((size_t)l->adim[i] * l->adim[i], 4);
-  }
-  for (int i = 0; i < l->NL; ++i) {
-    l->goff[i] = f;
-    f += align_up((size_t)l->blk[i].C * l->blk[i].C, 4);
-  }
-  l->factor_floats = f;
-  size_t v = 0;
-  for (int i = 0; i < l->NL; ++i) {
-    l->ainv_off[i] = v;
-    v += align_up((size_t)(l->blk[i].K + 1) * (l->blk[i].K + 1), 4);
-  }
-  for (int i = 0; i < l->NL; ++i) {
-    l->ginv_off[i] = v;
-    v += align_up((size_t)l->blk[i].C * l->blk[i].C, 4);
-  }
-  l->inv_floats = v;
+  l->set_blocks(l->L + 2);
+  l->sch.acktr = c->acktr != 0;
+  l->sch.num_cold_updates = c->num_cold_updates;
+  l->sch.invert_every = c->invert_every;
 }
 
 // lay the arena out (base == nullptr: size pass only)
 size_t layout(acx_mlp* l, uint8_t* base) {
   Arena ar;
   ar.base = base;
-  const int N = l->N, R = l->R, A = l->A, NL = l->NL;
-  const size_t P = l->params_pad, F = l->factor_floats;
-  auto f32 = [&](size_t n) { return reinterpret_cast<float*>(ar.take(n * sizeof(float))); };
-  l->params = f32(P);
-  l->velocity = f32(P);
-  l->accum = f32(P);
-  l->precon = f32(P);
-  l->bucket_floats = P + F + 4;
-  l->bucket = f32(l->bucket_floats);   // [A | G | grads | 4 loss scalars], as acx_learner's reduce bucket
-  l->stats = l->bucket;
-  l->grads = l->bucket + F;
-  l->bscalars = l->bucket + F + P;
-  l->sums = f32(F);
-  l->inv = f32(l->inv_floats);
-  l->damp = f32(16);
-  l->lambdas = f32(8);
-  l->scalars = f32(16);
-  l->sched = reinterpret_cast<Sched*>(ar.take(sizeof(Sched)));
-  l->d_a_ptrs = reinterpret_cast<const float**>(ar.take(kMaxLayers * sizeof(float*)));
-  l->d_g_ptrs = reinterpret_cast<const float**>(ar.take(kMaxLayers * sizeof(float*)));
-  l->d_a_dims = reinterpret_cast<int*>(ar.take(kMaxLayers * sizeof(int)));
-  l->d_g_dims = reinterpret_cast<int*>(ar.take(kMaxLayers * sizeof(int)));
-  l->d_jobs = reinterpret_cast<InvJob*>(ar.take(2 * kMaxLayers * sizeof(InvJob)));
-  l->d_pjobs = reinterpret_cast<PreconJob*>(ar.take(kMaxLayers * sizeof(PreconJob)));
-  l->inv_bar = reinterpret_cast<unsigned int*>(ar.take(256));
-  l->act_counter = reinterpret_cast<unsigned long long*>(ar.take(256));
-  l->precon_w = f32(P);
-  for (int i = 0; i < NL; ++i) {
-    const int d = l->blk[i].K + 1, c = l->blk[i].C;
-    l->ainv_pl[i] = take_planes(ar, 3, d, pad8(d));
-    l->ginv_pl[i] = take_planes(ar, 3, c, pad8(c));
-  }
-  for (int i = 0; i < NL; ++i) {   // inverse jobs (sorted by decreasing n at create)
-    const int d = l->blk[i].K + 1, c = l->blk[i].C;
-    InvJob& ja = l->h_jobs[i];
-    ja.s = l->sums + l->aoff[l->blk[i].afac];
-    ja.n = d;
-    ja.damp_index = 2 * i;
-    ja.work_m = reinterpret_cast<double*>(ar.take((size_t)d * d * sizeof(double)));
-    ja.work_x = reinterpret_cast<double*>(ar.take(((size_t)3 * 32 * d + 2 * 32 * 32 + 2048) * sizeof(double)));
-    ja.inv = l->inv + l->ainv_off[i];
-    for (int q = 0; q < 3; ++q) ja.planes[q] = l->ainv_pl[i].p[q];
-    ja.ld_planes = l->ainv_pl[i].ld;
-    InvJob& jg = l->h_jobs[NL + i];
-    jg.s = l->sums + l->goff[i];
-    jg.n = c;
-    jg.damp_index = 2 * i + 1;
-    jg.work_m = reinterpret_cast<double*>(ar.take((size_t)c * c * sizeof(double)));
-    jg.work_x = reinterpret_cast<double*>(ar.take(((size_t)3 * 32 * c + 2 * 32 * 32 + 2048) * sizeof(double)));
-    jg.inv = l->inv + l->ginv_off[i];
-    for (int q = 0; q < 3; ++q) jg.planes[q] = l->ginv_pl[i].p[q];
-    jg.ld_planes = l->ginv_pl[i].ld;
-  }
-  l->num_pjobs = 0;
-  l->pjobs_max_d = 0;
-  for (int i = 0; i < NL; ++i) {   // blocks with C <= 64: batched fp32 SIMT preconditioning
-    if (l->blk[i].C > 64) continue;
-    PreconJob& pj = l->h_pjobs[l->num_pjobs++];
-    pj.v = l->grads + l->blk[i].off;
-    pj.ginv = l->inv + l->ginv_off[i];
-    pj.ainv = l->inv + l->ainv_off[i];
-    pj.w = l->precon_w + l->blk[i].off;
-    pj.u = l->precon + l->blk[i].off;
-    pj.d = l->blk[i].K + 1;
-    pj.c = l->blk[i].C;
-    pj.scale = 1.0f;   // fully connected: T~ = 1
-    l->pjobs_max_d = std::max(l->pjobs_max_d, pj.d);
-  }
+  const int N = l->N, R = l->R, A = l->A;
+  l->take_state(ar);
+  l->take_tables(ar);
   // inputs
-  l->obs = f32((size_t)R * l->D);
+  l->obs = ar.f32((size_t)R * l->D);
   l->actions = reinterpret_cast<uint8_t*>(ar.take(N));
   l->terminals = reinterpret_cast<uint8_t*>(ar.take(N));
-  l->rewards = f32(N);
+  l->rewards = ar.f32(N);
   // weights as GEMM operands
   for (int i = 0; i < l->L; ++i) {
     l->wT[i] = take_planes(ar, 3, l->blk[i].C, pad8(l->blk[i].K));
@@ -394,119 +209,45 @@ size_t layout(acx_mlp* l, uint8_t* base) {
     l->act[i] = take_planes(ar, kActPlanes, R, l->blk[i].C);
     l->dpre[i] = take_planes(ar, kActPlanes, 2 * (size_t)N, l->blk[i].C);
   }
-  l->logits = f32((size_t)R * A);
-  l->values = f32(R);
-  l->targets = f32(N);
-  l->adv = f32(N);
-  l->dheads = f32(2 * (size_t)N * (A + 1));
+  l->logits = ar.f32((size_t)R * A);
+  l->values = ar.f32(R);
+  l->targets = ar.f32(N);
+  l->adv = ar.f32(N);
+  l->dheads = ar.f32(2 * (size_t)N * (A + 1));
   int dmax = 0, cmax = 0;
-  for (int i = 0; i < NL; ++i) {
+  for (int i = 0; i < l->nb; ++i) {
     dmax = std::max(dmax, l->blk[i].K + 1);
     cmax = std::max(cmax, l->blk[i].C);
   }
   l->Vp = take_planes(ar, 3, dmax, pad8(cmax));
   l->Wt = take_planes(ar, 3, cmax, pad8(dmax));
-  l->dot_partials = f32(kDotPartials);
-  l->colsum_partial = f32((size_t)kColsumChunks * pad8(dmax));
-  l->colsum_tmp = f32(pad8(dmax) + 8);
+  l->dot_partials = ar.f32(kDotPartials);
+  l->colsum_partial = ar.f32((size_t)kColsumChunks * pad8(dmax));
+  l->colsum_tmp = ar.f32(pad8(dmax) + 8);
   const size_t kpad = align_up((size_t)dmax, 128);
   l->ws_bytes = std::max<size_t>((size_t)48 << 20, kpad * kpad * sizeof(float) + (1 << 20));
   l->ws = reinterpret_cast<float*>(ar.take(l->ws_bytes));   // split-K partials; its arrival counters start zero
   return align_up(ar.used, 256);
 }
 
-void reg(acx_mlp* l, const std::string& name, void* p, size_t bytes) { l->named[name] = Buf{p, bytes}; }
-
 void register_buffers(acx_mlp* l) {
-  const size_t P = l->num_params;
-  reg(l, "params", l->params, P * 4);
-  reg(l, "velocity", l->velocity, P * 4);
-  reg(l, "accum", l->accum, P * 4);
-  reg(l, "precon", l->precon, P * 4);
-  reg(l, "grads", l->grads, P * 4);
-  reg(l, "reduce_bucket", l->bucket, l->bucket_floats * 4);
-  reg(l, "factor_stats", l->stats, l->factor_floats * 4);
-  reg(l, "factor_sums", l->sums, l->factor_floats * 4);
-  reg(l, "inverses", l->inv, l->inv_floats * 4);
-  reg(l, "dampings", l->damp, 2 * l->NL * 4);
-  reg(l, "scalars", l->scalars, 16 * 4);
-  reg(l, "sched", l->sched, sizeof(Sched));
-  reg(l, "observations", l->obs, (size_t)l->R * l->D * 4);
-  reg(l, "actions", l->actions, l->N);
-  reg(l, "terminals", l->terminals, l->N);
-  reg(l, "rewards", l->rewards, (size_t)l->N * 4);
-  reg(l, "logits", l->logits, (size_t)l->R * l->A * 4);
-  reg(l, "values", l->values, (size_t)l->R * 4);
-  reg(l, "targets", l->targets, (size_t)l->N * 4);
-  reg(l, "advantages", l->adv, (size_t)l->N * 4);
-  reg(l, "dheads", l->dheads, (size_t)2 * l->N * (l->A + 1) * 4);
-  for (int i = 0; i < l->L; ++i)
-    reg(l, "act_hi/" + l->blk[i].name, l->act[i].p[0], (size_t)l->R * l->act[i].ld * 2);
-  for (int f = 0; f <= l->L; ++f) {
-    const std::string fn = f < l->L ? l->blk[f].name : "heads";
-    const size_t b = (size_t)l->adim[f] * l->adim[f] * 4;
-    reg(l, "stats/A/" + fn, l->stats + l->aoff[f], b);
-    reg(l, "sums/A/" + fn, l->sums + l->aoff[f], b);
-  }
-  for (int i = 0; i < l->NL; ++i) {
-    const Block& B = l->blk[i];
-    const size_t gb = (size_t)B.C * B.C * 4, vb = (size_t)(B.K + 1) * B.C * 4;
-    reg(l, "stats/G/" + B.name, l->stats + l->goff[i], gb);
-    reg(l, "sums/G/" + B.name, l->sums + l->goff[i], gb);
-    reg(l, "inv/A/" + B.name, l->inv + l->ainv_off[i], (size_t)(B.K + 1) * (B.K + 1) * 4);
-    reg(l, "inv/G/" + B.name, l->inv + l->ginv_off[i], gb);
-    reg(l, "params/" + B.name, l->params + B.off, vb);
-    reg(l, "grads/" + B.name, l->grads + B.off, vb);
-    reg(l, "precon/" + B.name, l->precon + B.off, vb);
-    reg(l, "velocity/" + B.name, l->velocity + B.off, vb);
-    reg(l, "accum/" + B.name, l->accum + B.off, vb);
-  }
+  l->register_buffers();
+  l->reg("observations", l->obs, (size_t)l->R * l->D * 4);
+  l->reg("actions", l->actions, l->N);
+  l->reg("terminals", l->terminals, l->N);
+  l->reg("rewards", l->rewards, (size_t)l->N * 4);
+  l->reg("logits", l->logits, (size_t)l->R * l->A * 4);
+  l->reg("values", l->values, (size_t)l->R * 4);
+  l->reg("targets", l->targets, (size_t)l->N * 4);
+  l->reg("advantages", l->adv, (size_t)l->N * 4);
+  l->reg("dheads", l->dheads, (size_t)2 * l->N * (l->A + 1) * 4);
+  for (int i = 0; i < l->L; ++i) l->reg("act_hi/" + l->blk[i].name, l->act[i].p[0], (size_t)l->R * l->act[i].ld * 2);
 }
-
-struct GemmOut {
-  float* c = nullptr;
-  int ldc = 0;
-  const Planes* planes = nullptr;
-  const float* bias = nullptr;
-  int relu = 0;
-  const bf16* mask = nullptr;
-  int mask_ld = 0, mask_rows = 0;
-};
 
 int run_gemm(acx_mlp* l, const Planes& a, const Planes& b, int trans, int m, int n, int k, int level, float alpha, int symmetric,
              const GemmOut& o, cudaStream_t st) {
   acx_gemm_t g;
-  memset(&g, 0, sizeof(g));
-  for (int i = 0; i < a.n; ++i) g.a.planes[i] = a.p[i];
-  for (int i = 0; i < b.n; ++i) g.b.planes[i] = b.p[i];
-  g.a.num_planes = a.n;
-  g.b.num_planes = b.n;
-  g.a.ld = a.ld;
-  g.b.ld = b.ld;
-  if (trans) {
-    g.a.rows = k; g.a.cols = m; g.b.rows = k; g.b.cols = n;
-  } else {
-    g.a.rows = m; g.a.cols = k; g.b.rows = n; g.b.cols = k;
-  }
-  g.trans_a = g.trans_b = trans;
-  g.m = m; g.n = n; g.k = k;
-  g.num_pairs = level_pairs(level, a.n, b.n, g.pair_a, g.pair_b);
-  g.alpha = alpha;
-  g.bias = o.bias;
-  g.relu = o.relu;
-  g.symmetric = symmetric;
-  g.c = o.c;
-  g.ldc = o.ldc;
-  if (o.planes) {
-    for (int i = 0; i < o.planes->n; ++i) g.c_planes[i] = o.planes->p[i];
-    g.c_num_planes = o.planes->n;
-    g.ldc_planes = o.planes->ld;
-  }
-  g.mask_plane = o.mask;
-  g.mask_ld = o.mask_ld;
-  g.mask_rows = o.mask_rows;
-  g.workspace = l->ws;
-  g.workspace_bytes = l->ws_bytes;
+  fill_gemm(&g, a, b, trans, m, n, k, level, alpha, symmetric, o, l->ws, l->ws_bytes);
   return gemm_dispatch(&g, 0, st);
 }
 
@@ -609,42 +350,9 @@ int issue_update_phase1(acx_mlp* l, const int32_t* fl, const float* fe, bool fis
   return 0;
 }
 
-// what one update's optimizer step does, decided on the host from the schedule counters (kfac_utils.py:38-53)
-struct Plan {
-  bool a2c, cold, invert, kfac_apply, refresh;
-  int key() const { return (a2c ? 1 : 0) | (cold ? 2 : 0) | (invert ? 4 : 0) | (kfac_apply ? 8 : 0) | (refresh ? 16 : 0); }
-};
-
-Plan plan_update(const acx_mlp* l) {
-  const acx_mlp_config_t& c = l->cfg;
-  Plan p = {false, false, false, false, false};
-  if (!c.acktr) {
-    p.a2c = true;
-    p.refresh = true;
-    return p;
-  }
-  p.cold = l->gs < c.num_cold_updates;
-  const int64_t gs1 = l->gs + (p.cold ? 1 : 0);   // the cold optimizer increments global_step itself (kfac_utils.py:43)
-  p.invert = gs1 > c.num_cold_updates && (gs1 - c.num_cold_updates) % c.invert_every == 0;
-  // the always-run K-FAC apply (kfac_utils.py:52-53) is a no-op with zero inverses until the first refresh
-  p.kfac_apply = l->inverses_valid || p.invert;
-  p.refresh = p.cold || p.kfac_apply;
-  return p;
-}
-
-void advance(acx_mlp* l, const Plan& p) {
-  if (p.a2c) {
-    l->gs += 1;
-    return;
-  }
-  if (p.cold) l->gs += 1; else l->ncov += 1;
-  if (p.invert) l->inverses_valid = true;
-  l->gs += 1;
-}
-
 int precondition(acx_mlp* l, cudaStream_t st) {
   ACX_TRY(precondition_small(l->d_pjobs, l->num_pjobs, l->pjobs_max_d, st));
-  for (int i = 0; i < l->NL; ++i) {
+  for (int i = 0; i < l->nb; ++i) {
     const Block& B = l->blk[i];
     const int d = B.K + 1, C = B.C;
     if (C <= 64) continue;
@@ -684,16 +392,7 @@ int issue_update_phase2(acx_mlp* l, const Plan& p, cudaStream_t st) {
   } else {        // :44 covariance updates
     ACX_TRY(ema_update(l->sums, l->stats, l->factor_floats, c.cov_ema_decay, 1.0f, st));
   }
-  if (p.invert) {   // the Atari learner's selection: factor tiles resident in shared memory, else the fp64 chain
-    const int jobs = 2 * l->NL;
-    const int r = spd_inverse_resident(l->h_jobs, jobs, l->sched, l->damp, l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims, l->d_g_dims,
-                                       l->lambdas, l->NL, l->inv_bar, st);
-    if (r > 0) return r;
-    if (r < 0) {
-      ACX_TRY(compute_dampings(l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims, l->d_g_dims, l->lambdas, l->NL, l->damp, st));
-      ACX_TRY(spd_inverse_batched(l->h_jobs, l->d_jobs, jobs, l->sched, l->damp, st));
-    }
-  }
+  if (p.invert) ACX_TRY(l->invert(st));   // as the Atari learner: factor tiles resident in shared memory, else the fp64 chain
   if (p.kfac_apply) {
     ACX_TRY(precondition(l, st));
     ACX_TRY(dot_partial(l->grads, l->precon, P, l->dot_partials, kDotPartials, st));
@@ -701,48 +400,6 @@ int issue_update_phase2(acx_mlp* l, const Plan& p, cudaStream_t st) {
                       l->scalars + 4, st));
   }
   if (p.refresh) ACX_TRY(refresh_weight_planes(l, st));
-  return 0;
-}
-
-// CUDA-graph cache as learner.cu's run_cached: the first use of a variant runs eagerly (one-time host work such as tensor-map
-// encoding), the second is captured and instantiated, later uses replay it.  Valid because no kernel takes a step-dependent
-// scalar by value (Sched).
-template <typename F>
-int run_cached(acx_mlp* l, const GraphKey& key, cudaStream_t st, F&& issue) {
-  if (!l->cfg.use_graphs || st == nullptr) return issue();
-  {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive) return issue();
-  }
-  GraphEntry& ge = l->graphs[key];
-  if (ge.uses == 0) {
-    ge.uses = 1;
-    return issue();
-  }
-  if (ge.exec == nullptr) {
-    const uint64_t before = g_launch_count;
-    ACX_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    const int r = issue();
-    cudaGraph_t graph = nullptr;
-    const cudaError_t e = cudaStreamEndCapture(st, &graph);
-    if (r != 0 || e != cudaSuccess || graph == nullptr) {
-      if (graph) cudaGraphDestroy(graph);
-      if (r == 0) set_error(std::string("graph capture failed: ") + cudaGetErrorString(e));
-      return r ? r : 4;
-    }
-    ge.launches = g_launch_count - before;
-    g_launch_count = before;
-    const cudaError_t e2 = cudaGraphInstantiate(&ge.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    if (e2 != cudaSuccess) {
-      ge.exec = nullptr;
-      set_error(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e2));
-      return 4;
-    }
-  }
-  ACX_CUDA(cudaGraphLaunch(ge.exec, st));
-  count_launch((int)ge.launches);
-  ge.uses += 1;
   return 0;
 }
 
@@ -783,59 +440,22 @@ acx_mlp_t* acx_mlp_create(const acx_mlp_config_t* cfg, void* d_arena, size_t are
   }
   layout(l, reinterpret_cast<uint8_t*>(d_arena));
   register_buffers(l);
-  l->gs = 0;
-  l->ncov = 0;
-  l->inverses_valid = false;
-  // zero everything persistent (pad columns of the operand planes included); RMSProp's ms starts at one (TF-1 default)
-  cudaError_t e = cudaMemset(d_arena, 0, need);
-  std::vector<float> ones;
-  if (e == cudaSuccess && !cfg->acktr) {
-    ones.assign(l->params_pad, 1.0f);
-    e = cudaMemcpy(l->accum, ones.data(), l->params_pad * 4, cudaMemcpyHostToDevice);
-  }
-  Sched s0 = {0ull, 0ull, cfg->lr_start, 1.0f};
-  if (e == cudaSuccess) e = cudaMemcpy(l->sched, &s0, sizeof(s0), cudaMemcpyHostToDevice);
-  const float* ap[kMaxLayers];
-  const float* gp[kMaxLayers];
-  int ad[kMaxLayers], gd[kMaxLayers];
-  float lam[8] = {0};
-  for (int i = 0; i < l->NL; ++i) {
-    ap[i] = l->sums + l->aoff[l->blk[i].afac];
-    gp[i] = l->sums + l->goff[i];
-    ad[i] = l->adim[l->blk[i].afac];
-    gd[i] = l->blk[i].C;
-    lam[i] = cfg->damping;   // lambda / T~ with T~ = 1
-  }
-  const int NL = l->NL;
-  std::stable_sort(l->h_jobs, l->h_jobs + 2 * NL, [](const InvJob& a, const InvJob& b) { return a.n > b.n; });
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_a_ptrs, ap, NL * sizeof(float*), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_g_ptrs, gp, NL * sizeof(float*), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_a_dims, ad, NL * sizeof(int), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_g_dims, gd, NL * sizeof(int), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->lambdas, lam, sizeof(lam), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_pjobs, l->h_pjobs, sizeof(l->h_pjobs), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(l->d_jobs, l->h_jobs, sizeof(l->h_jobs), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) {
-    set_error(std::string("acx_mlp_create: ") + cudaGetErrorString(e));
+  // zero everything persistent (pad columns of the operand planes included)
+  if (l->upload(d_arena, need, !cfg->acktr, cfg->lr_start, cfg->damping) != 0) {
     delete l;
     return nullptr;
   }
   return l;
 }
 
-void acx_mlp_destroy(acx_mlp_t* l) {
-  if (l)
-    for (auto& kv : l->graphs)
-      if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-  delete l;
-}
+void acx_mlp_destroy(acx_mlp_t* l) { delete l; }
 
 size_t acx_mlp_num_params(const acx_mlp_t* l) { return l ? l->num_params : 0; }
 
 int acx_mlp_set_params(acx_mlp_t* l, const float* h_params, void* stream) {
   ACX_CHECK(l && h_params, "null argument");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  ACX_CUDA(cudaMemcpyAsync(l->params, h_params, l->num_params * sizeof(float), cudaMemcpyHostToDevice, st));
+  ACX_TRY(l->set_params(h_params, st));
   ACX_TRY(refresh_weight_planes(l, st));
   ACX_CUDA(cudaStreamSynchronize(st));
   return 0;
@@ -843,76 +463,47 @@ int acx_mlp_set_params(acx_mlp_t* l, const float* h_params, void* stream) {
 
 int acx_mlp_get_params(acx_mlp_t* l, float* h_params, void* stream) {
   ACX_CHECK(l && h_params, "null argument");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  ACX_CUDA(cudaMemcpyAsync(h_params, l->params, l->num_params * sizeof(float), cudaMemcpyDeviceToHost, st));
-  ACX_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return l->get_params(h_params, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int acx_mlp_refresh_weights(acx_mlp_t* l, void* stream) {
   ACX_CHECK(l, "null learner");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   ACX_TRY(refresh_weight_planes(l, st));
-  for (int i = 0; i < l->NL; ++i) {   // the bf16 planes of the stored inverses are derived state too
-    const int d = l->blk[i].K + 1, c = l->blk[i].C;
-    ACX_TRY(split_planes(l->inv + l->ainv_off[i], d, d, d, 1.0f, l->ainv_pl[i].p[0], l->ainv_pl[i].p[1], l->ainv_pl[i].p[2], 3,
-                         l->ainv_pl[i].ld, st));
-    ACX_TRY(split_planes(l->inv + l->ginv_off[i], c, c, c, 1.0f, l->ginv_pl[i].p[0], l->ginv_pl[i].p[1], l->ginv_pl[i].p[2], 3,
-                         l->ginv_pl[i].ld, st));
-  }
-  return 0;
+  return l->split_inverses(st);
 }
 
 void* acx_mlp_buffer(acx_mlp_t* l, const char* name, size_t* num_bytes) {
-  if (!l || !name) return nullptr;
-  auto it = l->named.find(name);
-  if (it == l->named.end()) {
-    set_error(std::string("acx_mlp_buffer: unknown buffer '") + name + "'");
-    return nullptr;
-  }
-  if (num_bytes) *num_bytes = it->second.bytes;
-  return it->second.ptr;
+  return l ? l->buffer("acx_mlp_buffer", name, num_bytes) : nullptr;
 }
 
 int acx_mlp_update(acx_mlp_t* l, const int32_t* d_fisher_labels, const float* d_fisher_eps, void* stream) {
   ACX_CHECK(l, "null learner");
   ACX_CHECK((d_fisher_labels == nullptr) == (d_fisher_eps == nullptr), "inject both Fisher labels and eps, or neither");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const bool fisher = l->cfg.acktr != 0 && l->gs >= l->cfg.num_cold_updates;   // kfac_utils.py:42-44
-  const Plan p = plan_update(l);
-  const GraphKey key(p.key() | (fisher ? 32 : 0), d_fisher_labels, d_fisher_eps, nullptr, nullptr, nullptr);
-  ACX_TRY(run_cached(l, key, st, [&]() {
+  const bool fisher = l->sch.fisher();
+  const Plan p = l->sch.plan();
+  const GraphKey key = {0, p.key() | (fisher ? 32 : 0), d_fisher_labels, d_fisher_eps};
+  ACX_TRY(l->graphs.run(key, st, !l->cfg.use_graphs, [&]() {
     const int r1 = issue_update_phase1(l, d_fisher_labels, d_fisher_eps, fisher, st);
     return r1 ? r1 : issue_update_phase2(l, p, st);
   }));
-  advance(l, p);
+  l->sch.advance(p);
   return 0;
 }
 
-int64_t acx_mlp_global_step(const acx_mlp_t* l) { return l ? l->gs : -1; }
+int64_t acx_mlp_global_step(const acx_mlp_t* l) { return l ? l->sch.gs : -1; }
 
 int acx_mlp_set_state(acx_mlp_t* l, int64_t global_step, int64_t num_cov_updates, int inverses_valid, void* stream) {
   ACX_CHECK(l, "null learner");
   ACX_CHECK(global_step >= 0 && num_cov_updates >= 0, "negative counters");
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  l->gs = global_step;
-  l->ncov = num_cov_updates;
-  l->inverses_valid = inverses_valid != 0;
-  Sched s;
-  s.gs = (unsigned long long)global_step;
-  s.ncov = (unsigned long long)num_cov_updates;
-  s.lr = l->cfg.lr_start;
-  s.debias = num_cov_updates > 0 ? (float)(1.0 / (1.0 - pow((double)l->cfg.cov_ema_decay, (double)num_cov_updates))) : 1.0f;
-  ACX_CUDA(cudaMemcpyAsync(l->sched, &s, sizeof(s), cudaMemcpyHostToDevice, st));
-  ACX_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return l->sch.set(global_step, num_cov_updates, inverses_valid, l->cfg.lr_start, l->cfg.cov_ema_decay, true, l->sched,
+                    reinterpret_cast<cudaStream_t>(stream));
 }
 
 int acx_mlp_get_state(const acx_mlp_t* l, int64_t* global_step, int64_t* num_cov_updates, int* inverses_valid) {
   ACX_CHECK(l, "null learner");
-  if (global_step) *global_step = l->gs;
-  if (num_cov_updates) *num_cov_updates = l->ncov;
-  if (inverses_valid) *inverses_valid = l->inverses_valid ? 1 : 0;
+  l->sch.get(global_step, num_cov_updates, inverses_valid);
   return 0;
 }
 
@@ -928,9 +519,8 @@ int acx_mlp_act(acx_mlp_t* l, const float* d_obs, int rows, const float* d_unifo
     if (d_values) ACX_CUDA(cudaMemcpyAsync(d_values, l->values, (size_t)rows * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return 0;
   };
-  const GraphKey key(64 | (greedy ? 1 : 0) | (rows << 7), d_obs, d_actions, d_uniform, d_logits, d_values);
-  if (l->graphs.size() > 512 && l->graphs.find(key) == l->graphs.end()) return issue();   // ever-changing buffers
-  return run_cached(l, key, st, issue);
+  const GraphKey key = {1, (greedy ? 1 : 0) | (rows << 1), d_obs, d_actions, d_uniform, d_logits, d_values};
+  return l->graphs.run_bounded(key, st, !l->cfg.use_graphs, issue);
 }
 
 }  // extern "C"

@@ -38,7 +38,6 @@ class Gemm(ctypes.Structure):
                 ("c_planes", ctypes.c_void_p * MAX_PLANES), ("c_num_planes", ctypes.c_int), ("ldc_planes", ctypes.c_int),
                 ("mask_plane", ctypes.c_void_p), ("mask_ld", ctypes.c_int), ("mask_rows", ctypes.c_int),
                 ("splits", ctypes.c_int), ("workspace", ctypes.c_void_p), ("workspace_bytes", ctypes.c_size_t),
-                ("a_patch_u8", ctypes.c_void_p), ("a_patch_samples", ctypes.c_int),
                 ("a_gather", ctypes.POINTER(Gather)), ("b_gather", ctypes.POINTER(Gather)),
                 ("perm_m", ctypes.c_int), ("perm_n", ctypes.c_int)]
 
@@ -135,7 +134,6 @@ SIGNATURES = {
     "acx_learner_peer_reduce_prefix": (ctypes.c_int, [_P, _P]),
     "acx_peer_error": (ctypes.c_int, []),
     "acx_learner_ema": (ctypes.c_int, [_P, _P]),
-    "acx_learner_defer_input_factors": (ctypes.c_int, [_P, ctypes.c_int]),
     "acx_learner_set_profiling": (ctypes.c_int, [_P, ctypes.c_int]),
     "acx_learner_stage_ms": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_float)]),
     "acx_learner_global_step": (ctypes.c_int64, [_P]),

@@ -50,10 +50,6 @@ struct TcParams {
   int bn;                // tile width (32, 64, 128)
   int bk;                // k-block depth (64 or 32)
   int trace;             // triage: record where CTA 0's MMA warp spends its cycles (ACX_GEMM_TRACE=1)
-  // A operand built in shared memory by the patch-producer warps instead of TMA: the conv1 patch matrix
-  // P1[(r, oy, ox)][(kh, kw, c)] = obs[r, 4 oy + kh, 4 ox + kw, c] (uint8 -> bf16, exact) is never materialised
-  const uint8_t* patch_src;   // uint8 [samples, 84, 84, 4] or null
-  int patch_limit;            // number of patch rows (patches beyond it read as zero)
   int stages;            // shared-memory ring depth
   int tiles_m, tiles_n, num_tiles, splits, total_work;
   int symmetric;
@@ -220,9 +216,6 @@ __device__ __forceinline__ void reduce_block(const float* __restrict__ src, long
 
 constexpr int MAX_STAGES = 8;
 constexpr int GEMM_THREADS = 320;                       // warp 0 TMA producer, warp 1 MMA, warps 2..9 epilogue
-constexpr int PATCH_WARPS = 8;                          // PATCH instantiation: + warps 10..17 build the conv1 patch tiles
-constexpr int PATCH_WARP0 = 10;
-constexpr int PATCH_THREADS = 32 * PATCH_WARPS;
 constexpr int EPI_BYTES = 8 * 32 * 32 * 4;              // one XOR-swizzled 32 x 32 fp32 staging tile per epilogue warp
 
 // ------------------------------------------------------------------------------------------------
@@ -236,8 +229,8 @@ constexpr int EPI_BYTES = 8 * 32 * 32 * 4;              // one XOR-swizzled 32 x
 // ------------------------------------------------------------------------------------------------
 __device__ long long g_gemm_trace[12];   // triage: total / waiting for operands / waiting for an accumulator / k-blocks
 
-template <int MAJOR, bool PATCH>
-__global__ void __launch_bounds__(GEMM_THREADS + (PATCH ? PATCH_THREADS : 0), 1)
+template <int MAJOR>
+__global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ CUtensorMap ta1,
                const __grid_constant__ CUtensorMap ta2, const __grid_constant__ CUtensorMap tb0,
                const __grid_constant__ CUtensorMap tb1, const __grid_constant__ CUtensorMap tb2,
@@ -272,7 +265,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ 
 
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < p.stages; ++s) {
-      mbar_init(&full_bar[s], PATCH ? 1 + PATCH_WARPS : 1);   // the TMA thread's expect_tx arrival (+ one per patch-producer warp)
+      mbar_init(&full_bar[s], 1);   // the TMA thread's expect_tx arrival
       mbar_init(&empty_bar[s], 1);
     }
     for (int b = 0; b < 2; ++b) {
@@ -329,11 +322,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ 
         const int na = MAJOR == 0 ? 0 : min(BM / 64, (p.out.m - m0 + 63) / 64);
         const int nb = MAJOR == 0 ? 0 : min(BN / 64, (p.out.n - n0 + 63) / 64);
         const int nch = (p.out.n + 63) / 64;   // panel mode: 64-column chunks of X
-        constexpr bool patch = PATCH;   // the A tiles (all tiles in panel mode) come from the patch warps
         const bool diag = MAJOR == 1 && p.same_operand && tm == tn;   // B tile = A tile: loaded once
-        const uint32_t tx = p.panel ? (patch ? 0u : (uint32_t)(p.npa * nch * bk * 128))
-                                    : (MAJOR == 0 ? (uint32_t)(stage_bytes - (patch ? p.npa * a_tile_bytes : 0))
-                                                  : (uint32_t)(((patch ? 0 : p.npa * na) + (diag ? 0 : p.npb * nb)) * bk * 128));
+        const uint32_t tx = p.panel ? (uint32_t)(p.npa * nch * bk * 128)
+                                    : (MAJOR == 0 ? (uint32_t)stage_bytes
+                                                  : (uint32_t)((p.npa * na + (diag ? 0 : p.npb * nb)) * bk * 128));
         // gathered operands: the chunk coordinates of this work item's (up to 4) A and (up to 2) B chunks are fixed - read them
         // from the parameters once, not per load (the issuing thread is alone: dependent parameter loads with run-time indices
         // cost it hundreds of cycles per k-block)
@@ -381,7 +373,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ 
           mbar_expect_tx(&full_bar[s], tx);
           uint8_t* a_s = smem + s * stage_bytes;
           if (p.panel) {
-            for (int i = 0; i < p.npa && !patch; ++i) {
+            for (int i = 0; i < p.npa; ++i) {
               const CUtensorMap* ma = i == 0 ? &ta0 : (i == 1 ? &ta1 : &ta2);
 #pragma unroll
               for (int j = 0; j < 4; ++j) {   // (a panel is at most 256 columns = 4 chunks)
@@ -396,7 +388,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ 
             continue;
           }
           uint8_t* b_s = a_s + p.npa * a_tile_bytes;
-          for (int i = 0; i < p.npa && !patch; ++i) {
+          for (int i = 0; i < p.npa; ++i) {
             const CUtensorMap* ma = i == 0 ? &ta0 : (i == 1 ? &ta1 : &ta2);
             uint8_t* dst = a_s + i * a_tile_bytes;
             if (MAJOR == 0) {
@@ -568,115 +560,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap ta0, const __grid_constant__ 
       g_gemm_trace[1] = w_full;
       g_gemm_trace[2] = w_acc;
       g_gemm_trace[3] = it;
-    }
-  } else if (PATCH && warp >= PATCH_WARP0) {
-    // ===== patch producers (8 warps): build the conv1 patch tiles straight from the uint8 observations =====
-    // A 64-element chunk of a patch row is two kernel rows kh = 2c, 2c + 1: twice 32 contiguous bytes
-    // obs[r, 4 oy + kh, 4 ox .. 4 ox + 7, 0 .. 3], converted to bf16 (exact) and stored as one 128-byte row in the
-    // SWIZZLE_128B order TMA would have produced (16-byte group g of row i at position g ^ (i & 7)).
-    //   K-major  (forward):      tile = 128 patch rows m0.., chunk = k-block kb
-    //   MN-major (wgrad / SYRK): per 64-feature chunk j, 64 patch rows kb*64..
-    // 256 threads, one half-row (one kernel row, 32 bytes -> 64 bytes of bf16) per thread and item; the loads of the next
-    // k-block are issued before the current one is converted, so their L2 latency hides behind the ring.
-    const int pt = (warp - PATCH_WARP0) * 32 + lane;   // 0 .. 255
-    const uint8_t* __restrict__ obs = p.patch_src;
-    // flattened (work item, k-block) sequence of this CTA
-    int w = blockIdx.x, kb = 0, kb1 = 0, m0 = 0, items = 0, rows_per_chunk = MAJOR == 0 ? BM : bk;
-    auto open_work = [&]() -> bool {
-      while (w < p.total_work) {
-        int tm, tn, split;
-        decode(w, tm, tn, split);
-        m0 = tm * BM;
-        kb = split * p.kb_per_split;
-        kb1 = min(p.kb_total, kb + p.kb_per_split);
-        const int nchunks = MAJOR == 0 ? 1 : (p.panel ? (p.out.n + 63) / 64 : min(BM / 64, (p.out.m - m0 + 63) / 64));
-        items = 2 * nchunks * rows_per_chunk;   // half rows
-        if (kb < kb1) return true;
-        w += gridDim.x;
-      }
-      return false;
-    };
-    constexpr int MAX_PER_THREAD = 2;   // panel mode: 4 chunks x 64 rows x 2 halves = 512 half rows over 256 threads
-    auto load_block = [&](uint4 (*q)[2]) {
-#pragma unroll
-      for (int u = 0; u < MAX_PER_THREAD; ++u) {
-        q[u][0] = q[u][1] = make_uint4(0u, 0u, 0u, 0u);
-        const int item = pt + u * 256;
-        if (item < items) {
-          const int half = item & 1, ri = item >> 1;
-          const int j = ri / rows_per_chunk, row = ri - j * rows_per_chunk;
-          const int patch = MAJOR == 0 ? m0 + row : kb * bk + row;
-          const int khp = MAJOR == 0 ? kb : (p.panel ? j : m0 / 64 + j);   // kernel-row pair = 64-feature chunk index
-          if (patch < p.patch_limit) {
-            const int r = patch / 400, loc = patch - r * 400;
-            const int oy = loc / 20, ox = loc - oy * 20;
-            const uint4* src = reinterpret_cast<const uint4*>(obs + ((size_t)(r * 84 + 4 * oy + 2 * khp + half) * 84 + 4 * ox) * 4);
-            q[u][0] = __ldg(src);
-            q[u][1] = __ldg(src + 1);
-          }
-        }
-      }
-    };
-    uint4 cur[MAX_PER_THREAD][2], nxt[MAX_PER_THREAD][2];
-    bool have = open_work();
-    if (have) load_block(cur);
-    int it = 0;
-    int ring_s = 0;
-    uint32_t ring_ph = 0u;
-    while (have) {
-      // remember where the current block goes, then advance and prefetch
-      const int c_items = items, c_rpc = rows_per_chunk;
-      ++kb;
-      if (kb >= kb1) {
-        w += gridDim.x;
-        have = open_work();
-      }
-      if (have) load_block(nxt);
-      const int s = ring_s;   // ring position and phase advance without a division (this thread is the bottleneck)
-      const uint32_t ph = ring_ph;
-      if (++ring_s == p.stages) {
-        ring_s = 0;
-        ring_ph ^= 1u;
-      }
-      mbar_wait(&empty_bar[s], ph ^ 1u, 6);
-      uint8_t* a_s = smem + s * stage_bytes;
-#pragma unroll
-      for (int u = 0; u < MAX_PER_THREAD; ++u) {
-        const int item = pt + u * 256;
-        if (item < c_items) {
-          const int half = item & 1, ri = item >> 1;
-          const int j = ri / c_rpc, row = ri - j * c_rpc;
-          uint8_t* dst = a_s + j * (c_rpc * 128) + row * 128;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {   // 16 bytes -> 16 bf16 = two 16-byte groups
-            const uint32_t wv[4] = {cur[u][h].x, cur[u][h].y, cur[u][h].z, cur[u][h].w};
-            uint32_t o[8];
-#pragma unroll
-            for (int t = 0; t < 4; ++t) {
-              // byte -> bf16: the integer 0..255 as fp32 (exact) is 0x4B000000 + v - 2^23; its bf16 is the high half
-              const float f0 = __uint_as_float(0x4B000000u | (wv[t] & 0xffu)) - 8388608.0f;
-              const float f1 = __uint_as_float(0x4B000000u | ((wv[t] >> 8) & 0xffu)) - 8388608.0f;
-              const float f2 = __uint_as_float(0x4B000000u | ((wv[t] >> 16) & 0xffu)) - 8388608.0f;
-              const float f3 = __uint_as_float(0x4B000000u | (wv[t] >> 24)) - 8388608.0f;
-              o[2 * t] = (__float_as_uint(f0) >> 16) | (__float_as_uint(f1) & 0xffff0000u);
-              o[2 * t + 1] = (__float_as_uint(f2) >> 16) | (__float_as_uint(f3) & 0xffff0000u);
-            }
-            const int g0 = 4 * half + 2 * h, g1 = g0 + 1;
-            *reinterpret_cast<uint4*>(dst + ((g0 ^ (row & 7)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
-            *reinterpret_cast<uint4*>(dst + ((g1 ^ (row & 7)) << 4)) = make_uint4(o[4], o[5], o[6], o[7]);
-          }
-        }
-      }
-      // generic-proxy writes -> visible to the tensor core's async-proxy reads, then one arrival per warp
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&full_bar[s]);
-      ++it;
-#pragma unroll
-      for (int u = 0; u < MAX_PER_THREAD; ++u) {
-        cur[u][0] = nxt[u][0];
-        cur[u][1] = nxt[u][1];
-      }
     }
   } else {
     // ===== epilogue: TMEM -> registers -> shared-memory transpose -> global =====
@@ -1369,8 +1252,7 @@ static void plan_tc(const acx_gemm_t* g, TcPlan* pl) {
   if (g->symmetric) tiles = pl->tiles_n * (pl->tiles_n + 1) / 2;
   // SYRK panel mode: X^T X with 128 < n <= 256 (MN-major): every CTA streams its k-range of X once and feeds all three
   // upper sub-tiles from the same shared memory
-  const bool same_operand = g->a_gather ? (g->b_gather == nullptr || g->b_gather == g->a_gather)
-                                        : (g->a_patch_u8 != nullptr || g->a.planes[0] == g->b.planes[0]);
+  const bool same_operand = g->a_gather ? (g->b_gather == nullptr || g->b_gather == g->a_gather) : g->a.planes[0] == g->b.planes[0];
   pl->panel = (g->symmetric && g->trans_a && pl->bn == 128 && pl->tiles_n == 2 && same_operand) ? 1 : 0;
   if (pl->panel) tiles = 1;
   // planes each side loads per k-block, and the ring depth they leave
@@ -1391,7 +1273,7 @@ static void plan_tc(const acx_gemm_t* g, TcPlan* pl) {
   // 128-deep k-blocks for MN-major products whose stages are small (the deep-split conv weight gradients and output-factor
   // SYRKs: 8 MMAs per 64-deep k-block): the hand-off between producer, issuing thread and tensor pipe costs ~250 cycles per
   // k-block whatever its depth (tools/micro/mma_rate3.cu).  ACX_GEMM_BK=128 forces it wherever two stages fit, =64 forbids it.
-  if (g->trans_a && g->a_patch_u8 == nullptr && force_bk() != 64 && force_bk() != 32) {
+  if (g->trans_a && force_bk() != 64 && force_bk() != 32) {
     const int st128 = stages_for(128);
     if (force_bk() == 128 ? st128 >= 2 : st128 >= bk128_min_stages()) pl->bk = 128;
   }
@@ -1443,7 +1325,7 @@ static void plan_tc(const acx_gemm_t* g, TcPlan* pl) {
   // The reduction runs inside the kernel where ONE SM can sum a tile's partials in a few microseconds (measured: a single
   // SM reads its peers' partials at some tens of GB/s, so deep splits of large tiles - the conv factor SYRKs and weight
   // gradients - reduce faster in a finalize launch that spreads the sums over all SMs: 0.80 vs 1.32 ms/update with
-  // everything fused).  ACX_GEMM_FUSE_REDUCE: 0 = never, 1 = where cheap (default), 2 = always (two-level for > 8 splits).
+  // everything fused).  ACX_GEMM_FUSE_REDUCE: 0 = never (default), 1 = where cheap, 2 = always (two-level for > 8 splits).
   const size_t tile_bytes = (size_t)(pl->panel ? 4 : 1) * BM * pl->bn * sizeof(float);
   const bool cheap = pl->groups == 1 && (size_t)pl->splits * tile_bytes <= kFusedReduceBytes;
   const int mode = fuse_reduce_enabled();
@@ -1458,23 +1340,21 @@ static void plan_tc(const acx_gemm_t* g, TcPlan* pl) {
 static bool g_probe_on = false;
 static cudaEvent_t g_probe_ev[2] = {nullptr, nullptr};
 
-template <int MAJOR, bool PATCH>
+template <int MAJOR>
 static int launch_tc(const CUtensorMap* ta, const CUtensorMap* tb, const TcParams& p, int grid, int smem, cudaStream_t st) {
   static bool configured = false;
   if (!configured) {
-    ACX_CUDA((cudaFuncSetAttribute(gemm_tc_kernel<MAJOR, PATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT)));
+    ACX_CUDA((cudaFuncSetAttribute(gemm_tc_kernel<MAJOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT)));
     configured = true;
   }
   if (g_probe_on) ACX_CUDA(cudaEventRecord(g_probe_ev[0], st));
-  ACX_CUDA(launch_pdl(gemm_tc_kernel<MAJOR, PATCH>, dim3(grid), dim3(GEMM_THREADS + (PATCH ? PATCH_THREADS : 0)), (size_t)smem, st, ta[0], ta[1],
-                      ta[2], tb[0], tb[1], tb[2], p));
+  ACX_CUDA(launch_pdl(gemm_tc_kernel<MAJOR>, dim3(grid), dim3(GEMM_THREADS), (size_t)smem, st, ta[0], ta[1], ta[2], tb[0], tb[1],
+                      tb[2], p));
     acx::count_launch();
   if (g_probe_on) ACX_CUDA(cudaEventRecord(g_probe_ev[1], st));
   return 0;
 }
 
-// triage knob (ACX_MAIN_CTAS / ACX_SIDE_CTAS, learner.cu): cap on the persistent grid of the next tensor-core launches, so
-// that kernels of different lanes can share the SMs instead of queueing behind each other (0 = all SMs)
 static int g_pdl_override = -1;
 void set_pdl_override(int level) { g_pdl_override = level; }
 int pdl_level() {
@@ -1486,6 +1366,8 @@ int pdl_level() {
   return (v > 0 && g_pdl_override >= 0) ? g_pdl_override : v;
 }
 
+// cap on the persistent grid of the next tensor-core launches (learner.cu: lane 0 of K-FAC learners), so that kernels of
+// different lanes can share the SMs instead of queueing behind each other (0 = all SMs)
 int g_cta_cap = 0;
 void set_cta_cap(int cap) { g_cta_cap = cap; }
 
@@ -1516,7 +1398,6 @@ static int validate(const acx_gemm_t* g) {
     const acx_gather_t* ga = g->a_gather;
     ACX_CHECK(ga != nullptr && gb_eff != nullptr, "gathered operands: both sides must be gathered (or the product symmetric with B = A)");
     ACX_CHECK(g->trans_a == 1 && g->trans_b == 1, "gathered operands are MN-major (trans_a = trans_b = 1)");
-    ACX_CHECK(g->a_patch_u8 == nullptr, "a_gather and a_patch_u8 are exclusive");
     ACX_CHECK(ga->gx >= 1 && ga->gy >= 1 && ga->samples >= 1 && (long long)ga->samples * ga->gx * ga->gy == (long long)g->k,
               "gathered operands: k must be samples * gy * gx");
     ACX_CHECK(gb_eff->gx == ga->gx && gb_eff->gy == ga->gy && gb_eff->samples == ga->samples, "gathered operands: A and B enumerate different locations");
@@ -1525,16 +1406,6 @@ static int validate(const acx_gemm_t* g) {
   }
   if (g->perm_m || g->perm_n) ACX_CHECK(g->bias == nullptr && g->mask_plane == nullptr, "perm_m / perm_n: no bias or mask");
   ACX_CHECK(g->trans_a == g->trans_b, "only (K-major,K-major) and (MN-major,MN-major) operand pairs are supported");
-  if (g->a_patch_u8) {
-    // A = the conv1 patch matrix of uint8 observations [samples, 84, 84, 4] (8x8 kernel, stride 4: 400 patch rows of 256
-    // features per sample), generated inside the kernel
-    ACX_CHECK(g->a.num_planes == 1, "a_patch_u8: the patch operand has one (exact) plane");
-    ACX_CHECK((g->trans_a ? g->m : g->k) == 256, "a_patch_u8: the patch matrix has 256 feature columns");
-    ACX_CHECK((long long)(g->trans_a ? g->k : g->m) <= (long long)g->a_patch_samples * 400, "a_patch_u8: more patch rows than samples * 400");
-    ACX_CHECK((reinterpret_cast<uintptr_t>(g->a_patch_u8) & 15) == 0, "a_patch_u8 must be 16-byte aligned");
-    for (int i = 0; i < g->num_pairs; ++i) ACX_CHECK(g->pair_a[i] == 0, "a_patch_u8: pair_a must be 0");
-    if (g->symmetric) ACX_CHECK(g->trans_a && g->n == 256, "a_patch_u8: the symmetric product is P^T P (256 x 256)");
-  }
   ACX_CHECK(g->c != nullptr || g->c_num_planes > 0, "no output requested");
   ACX_CHECK(g->c_num_planes >= 0 && g->c_num_planes <= ACX_MAX_PLANES, "c_num_planes");
   if (g->symmetric) ACX_CHECK(g->m == g->n, "symmetric needs m == n");
@@ -1549,8 +1420,6 @@ static int gemm_tc(const acx_gemm_t* g, cudaStream_t st) {
   }
   CUtensorMap ta[3], tb[3];
   const int major = g->trans_a ? 1 : 0;
-  const bool patch = g->a_patch_u8 != nullptr;
-  const bool b_patch = patch && pl.panel;   // SYRK panel mode: both operand sides are the patch tiles
   const acx_gather_t* ga = g->a_gather;
   const acx_gather_t* gb = ga ? (g->b_gather ? g->b_gather : ga) : nullptr;
   for (int i = 0; i < 3 && ga; ++i) {   // gathered operands: 5-D views, one box = the 64 locations of a k-block x one 64-column chunk
@@ -1562,21 +1431,12 @@ static int gemm_tc(const acx_gemm_t* g, cudaStream_t st) {
   }
   for (int i = 0; i < 3 && !ga; ++i) {
     const int ia = i < g->a.num_planes ? i : 0, ib = i < g->b.num_planes ? i : 0;
-    int r;
-    if (!b_patch) {
-      r = major == 0 ? get_tensor_map(g->b.planes[ib], g->n, g->k, g->b.ld, pl.bk, pl.bn, &tb[i])
-                     : get_tensor_map(g->b.planes[ib], g->k, g->n, g->b.ld, 64, pl.bk, &tb[i]);
-      if (r) return r;
-    }
-    if (!patch) {
-      r = major == 0 ? get_tensor_map(g->a.planes[ia], g->m, g->k, g->a.ld, pl.bk, BM, &ta[i])
-                     : get_tensor_map(g->a.planes[ia], g->k, g->m, g->a.ld, 64, pl.bk, &ta[i]);
-      if (r) return r;
-    }
-  }
-  if (patch) {   // unused tensor maps still travel as kernel parameters: give them valid contents
-    if (b_patch) memset(tb, 0, sizeof(tb));
-    for (int i = 0; i < 3; ++i) ta[i] = tb[0];
+    int r = major == 0 ? get_tensor_map(g->b.planes[ib], g->n, g->k, g->b.ld, pl.bk, pl.bn, &tb[i])
+                       : get_tensor_map(g->b.planes[ib], g->k, g->n, g->b.ld, 64, pl.bk, &tb[i]);
+    if (r) return r;
+    r = major == 0 ? get_tensor_map(g->a.planes[ia], g->m, g->k, g->a.ld, pl.bk, BM, &ta[i])
+                   : get_tensor_map(g->a.planes[ia], g->k, g->m, g->a.ld, 64, pl.bk, &ta[i]);
+    if (r) return r;
   }
   TcParams p;
   fill_out(g, &p.out);
@@ -1590,7 +1450,7 @@ static int gemm_tc(const acx_gemm_t* g, cudaStream_t st) {
       const char* e = getenv("ACX_SYRK_DIAG");   // 0: diagonal tiles load both operand sides (round 1)
       dg = e ? atoi(e) : 1;
     }
-    p.same_operand = (dg && g->symmetric && major == 1 && !patch && one && pl.npa >= pl.npb) ? 1 : 0;
+    p.same_operand = (dg && g->symmetric && major == 1 && one && pl.npa >= pl.npb) ? 1 : 0;
   }
   p.gather_a = p.gather_b = ga ? 1 : 0;
   p.g_cells = pl.g_cells;
@@ -1642,8 +1502,6 @@ static int gemm_tc(const acx_gemm_t* g, cudaStream_t st) {
     }
     p.trace = tr;
   }
-  p.patch_src = g->a_patch_u8;
-  p.patch_limit = major == 0 ? g->m : g->k;
   p.mn_lbo = g_mn_lbo ? g_mn_lbo : (uint32_t)(pl.bk * 128);
   p.mn_sbo = g_mn_sbo ? g_mn_sbo : 1024u;
   p.mn_kstep = g_mn_kstep ? g_mn_kstep : 2048u;
@@ -1651,11 +1509,7 @@ static int gemm_tc(const acx_gemm_t* g, cudaStream_t st) {
   if (g_cta_cap > 0 && grid > g_cta_cap) grid = g_cta_cap;
   grid = ceil_div(p.total_work, ceil_div(p.total_work, grid));   // the smallest grid with the same number of rounds
   const int smem = SMEM_FIXED + p.stages * stage_bytes;
-  int r;
-  if (patch)
-    r = major == 0 ? launch_tc<0, true>(ta, tb, p, grid, smem, st) : launch_tc<1, true>(ta, tb, p, grid, smem, st);
-  else
-    r = major == 0 ? launch_tc<0, false>(ta, tb, p, grid, smem, st) : launch_tc<1, false>(ta, tb, p, grid, smem, st);
+  const int r = major == 0 ? launch_tc<0>(ta, tb, p, grid, smem, st) : launch_tc<1>(ta, tb, p, grid, smem, st);
   if (r) return r;
   if (pl.fuse) return 0;   // the kernel reduced and finished its own split-K partials
   if (pl.to_ws && g->symmetric && g->n > 64) {

@@ -603,77 +603,6 @@ static int launch_colsum_stage2(const float* partial, int chunks, int cols, floa
   return 0;
 }
 
-// ------------------------------------------------------------------------------------------------
-// small Gram matrices G = x^T x over a tall row range (the conv output factors: C = 32 / 64 columns, 10^4..10^5 rows).
-// Far too narrow for the tensor core (a 128-wide MMA tile would be 3/4..15/16 padding), so: fp32 SIMT, each CTA owns
-// a contiguous chunk of rows, stages them as fp32 in shared memory (planes summed) and accumulates its C x C partial in
-// registers; partial[chunk][C*C] is then reduced in a fixed order by colsum_stage2_kernel.
-// ------------------------------------------------------------------------------------------------
-template <int C>
-__global__ void __launch_bounds__(256) gram_stage1_kernel(const Planes x, int rows, int rows_per_chunk, float* __restrict__ partial) {
-  constexpr int RT = 64;                 // rows staged per iteration
-  constexpr int TG = C / 4;              // thread grid edge: every thread owns a 4 x 4 block of G
-  constexpr int RG = 256 / (TG * TG);    // row groups (C=32: 4 groups of 64 threads, C=64: 1); group g takes rows r % RG == g
-  constexpr int LD = C + 4;              // padded row (16-byte multiple)
-  __shared__ __align__(16) float xs[RT][LD];
-  const int g = threadIdx.x / (TG * TG);
-  const int tt = threadIdx.x - g * (TG * TG);
-  const int ti = tt / TG, tj = tt - ti * TG;
-  float acc[4][4];
-#pragma unroll
-  for (int a = 0; a < 4; ++a)
-#pragma unroll
-    for (int b = 0; b < 4; ++b) acc[a][b] = 0.f;
-  const int r0 = blockIdx.x * rows_per_chunk;
-  const int r1 = min(rows, r0 + rows_per_chunk);
-  constexpr int VPR = C / 8;             // 16-byte vectors per row
-  constexpr int LOADS = RT * VPR / 256;  // C=32: 1, C=64: 2
-  for (int rb = r0; rb < r1; rb += RT) {
-    uint4 q[LOADS][3];                   // every global load is issued before the first shared store
-#pragma unroll
-    for (int t = 0; t < LOADS; ++t) {
-      const int v = threadIdx.x + 256 * t;
-      const int rr = v / VPR, cv = v % VPR;
-      const int r = rb + rr;
-      const size_t idx = (size_t)r * x.ld + (size_t)cv * 8;
-      const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-      q[t][0] = r < r1 ? __ldg(reinterpret_cast<const uint4*>(x.p[0] + idx)) : z;
-      q[t][1] = (r < r1 && x.n > 1) ? __ldg(reinterpret_cast<const uint4*>(x.p[1] + idx)) : z;
-      q[t][2] = (r < r1 && x.n > 2) ? __ldg(reinterpret_cast<const uint4*>(x.p[2] + idx)) : z;
-    }
-    __syncthreads();   // previous iteration's reads of xs are done
-#pragma unroll
-    for (int t = 0; t < LOADS; ++t) {
-      const int v = threadIdx.x + 256 * t;
-      const int rr = v / VPR, cv = v % VPR;
-      float f[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      add8(f, q[t][0]);
-      add8(f, q[t][1]);
-      add8(f, q[t][2]);
-      *reinterpret_cast<float4*>(&xs[rr][cv * 8]) = make_float4(f[0], f[1], f[2], f[3]);
-      *reinterpret_cast<float4*>(&xs[rr][cv * 8 + 4]) = make_float4(f[4], f[5], f[6], f[7]);
-    }
-    __syncthreads();
-    const int nr = min(RT, r1 - rb);
-#pragma unroll 4
-    for (int r = g; r < nr; r += RG) {
-      const float4 a4 = *reinterpret_cast<const float4*>(&xs[r][4 * ti]);
-      const float4 b4 = *reinterpret_cast<const float4*>(&xs[r][4 * tj]);
-      const float a[4] = {a4.x, a4.y, a4.z, a4.w};
-      const float b[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-      for (int t = 0; t < 4; ++t)
-#pragma unroll
-        for (int u = 0; u < 4; ++u) acc[t][u] = fmaf(a[t], b[u], acc[t][u]);
-    }
-  }
-  // one partial per (chunk, row group); the fixed-order reduction over all of them happens in stage 2
-  float* dst = partial + ((size_t)blockIdx.x * RG + g) * (C * C);
-#pragma unroll
-  for (int t = 0; t < 4; ++t)
-    *reinterpret_cast<float4*>(dst + (4 * ti + t) * C + 4 * tj) = make_float4(acc[t][0], acc[t][1], acc[t][2], acc[t][3]);
-}
-
 // fp32 [K, C] (row-major, the V-layout weight rows) -> transposed bf16 planes [C, ld_out]
 __global__ void transpose_split_kernel(const float* __restrict__ in, int k_rows, int c_cols, bf16* __restrict__ p0,
                                        bf16* __restrict__ p1, bf16* __restrict__ p2, int num_planes, int ld_out) {
@@ -901,25 +830,6 @@ int colsum(const Planes& x, int rows, int cols, float scale, float* partial, int
   }
   ACX_PDL_LAUNCH(colsum_stage1_kernel, dim3(chunks, ceil_div(cols, CS_COLBLOCK)), CS_THREADS, smem, st, x, rows, cols, rpc, partial);
   if (int r2 = launch_colsum_stage2(partial, chunks, cols, scale, out, out_stride, out2, out2_stride, corner, st)) return r2;
-  return 0;
-}
-
-// G = scale * x^T x over rows [0, rows) of a C-column planes matrix (C = 32 or 64) -> out [C, C]
-int gram_small(const Planes& x, int rows, int c, float scale, float* partial, int max_chunks, float* out, cudaStream_t st) {
-  ACX_CHECK(c == 32 || c == 64, "gram_small: 32 or 64 columns");
-  int chunks = ceil_div(rows, 256);
-  const int cap = c == 32 ? max_chunks / 2 : max_chunks;   // C = 32 writes four partials per chunk: keep stage 2 short
-  if (chunks > cap) chunks = cap;
-  if (chunks < 1) chunks = 1;
-  const int rpc = ceil_div(rows, chunks);
-  chunks = ceil_div(rows, rpc);
-  if (c == 32)
-    gram_stage1_kernel<32><<<chunks, 256, 0, st>>>(x, rows, rpc, partial);
-  else
-    gram_stage1_kernel<64><<<chunks, 256, 0, st>>>(x, rows, rpc, partial);
-  ACX_LAUNCH_CHECK();
-  const int parts = chunks * (c == 32 ? 4 : 1);   // C = 32: four row groups per chunk
-  if (int r2 = launch_colsum_stage2(partial, parts, c * c, scale, out, 1, nullptr, 0, nullptr, st)) return r2;
   return 0;
 }
 

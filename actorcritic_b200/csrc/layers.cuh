@@ -44,7 +44,6 @@ int heads_bwd(const float* dheads, const float* vpol, const float* vval, const P
 int heads_gfactor(const float* dheads_fisher, int n_rows, int num_actions, float* g_pol, float* g_val, cudaStream_t st);
 int colsum(const Planes& x, int rows, int cols, float scale, float* partial, int max_chunks, float* out, int out_stride,
            cudaStream_t st, float* out2 = nullptr, int out2_stride = 0, float* corner = nullptr);
-int gram_small(const Planes& x, int rows, int c, float scale, float* partial, int max_chunks, float* out, cudaStream_t st);
 int conv_border(const uint8_t* obs_u8, const Planes* act, int n_rows, int hw_in, int c, int k, int s, int hw_out, float scale,
                 float* partial, int max_chunks, float* sum_tmp, float* a, int d, cudaStream_t st);
 int transpose_split(const float* in, int k_rows, int c_cols, bf16* p0, bf16* p1, bf16* p2, int num_planes, int ld_out,

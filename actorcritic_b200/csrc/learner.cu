@@ -69,18 +69,15 @@ struct acx_learner : KfacBlocks {
   Planes P1, act1, P2, act2, P3, act3, act4;
   Planes dpre4, dpre3, dpre2, dpre1;
   float *dP, *logits, *values, *targets, *adv, *dheads;
-  size_t dgrad_chunk_bytes;
   Planes wT[4], wN[4];
   Planes wD[4];              // gather-form dgrad operand of conv2 / conv3 (conv.cu), unused otherwise
   bool conv_tc[4];           // layer computes its input gradient with the gather-form tensor-core kernel (conv.cu)
-  bool conv_fwd_tc[4];       // layer runs its forward on the implicit-GEMM kernel (patch matrix built on the aux lane)
-  bool conv1_patch;          // conv1's patch matrix P1 is generated inside the GEMMs from the uint8 observations (never stored)
+  bool conv_fwd_tc[4];       // layer runs its forward on the implicit-GEMM kernel (conv.cu)
   PeerState peer;            // world > 1: phase 2 sums the ranks' buckets itself (peer.cu) - the caller issues no collective for them
   uint8_t* arena_base = nullptr;
   unsigned int* peer_flags = nullptr;
   unsigned int* peer_epochs = nullptr;
   cudaEvent_t reduced = nullptr;   // [G | grads | scalars] of this update are summed over the ranks (external event, split exchange)
-  int gather_mask;           // bit l: conv layer l reads its patch operand in place (bit 0 = `gather`)
   bool gather;               // no patch matrix is ever stored: the conv GEMMs read their patch operands in place (TMA box loads from
                              // the activations; conv1 from the row-pair interleaved bf16 copy `obs_pairs` of the observations)
   bf16* obs_pairs;           // [R, 42, 84, 2, 4] (layers.cu: obs_pairs_bf16)
@@ -94,7 +91,6 @@ struct acx_learner : KfacBlocks {
   std::vector<cudaEvent_t> lane_events;   // fork / join events (timing disabled), reused every update
   size_t ev_next = 0;
   bool lane_forked[kMaxLanes] = {false, false, false, false, false};
-  cudaEvent_t patches_ready[4] = {nullptr, nullptr, nullptr, nullptr};   // P_l complete on the aux lane (this update)
   cudaEvent_t a_ready = nullptr;     // all input-factor statistics of the current phase 1 are complete (external event)
   bool a_ready_valid = false;        // the last phase 1 recorded it
   Schedule sch;
@@ -105,8 +101,6 @@ struct acx_learner : KfacBlocks {
   float policy_weight = 1.0f, value_weight = 0.0f;   // acx_learner_set_loss_weights (value_weight is set from cfg at create)
   int loss_variant = 0;                   // 0 = the configured weights; other values key separate CUDA graphs
   bool external_ema = false;              // acx_learner_set_external_ema: phase 2 leaves statistics scaling + EMA to acx_learner_ema
-  int defer_request = 0;                  // acx_learner_defer_input_factors: mask for the next phase 1
-  int deferred = 0;                       // what the last phase 1 actually left to phase 2
   cudaEvent_t ev[ACX_NUM_STAGES + 2];
   bool ev_set[ACX_NUM_STAGES + 2];
   GraphCache graphs;
@@ -115,25 +109,11 @@ struct acx_learner : KfacBlocks {
 namespace acx {
 
 static const int kBorderChunks = 160;   // row chunks of the batch-sum pass over a conv input (4 samples per CTA at 32 x 20)
-static const int kGramChunks = 444;   // 3 CTAs per SM
-static const size_t kDgradChunkBytes = 0;   // 0 = whole batch in one piece.  Measured on B200 at 32x20 (ACX_DGRAD_CHUNK_MB sweep):
-                                            // whole 1.510 ms/update, 128 MB 1.533, 64 MB 1.551, 32 MB 1.599, 16 MB 1.681 - the
-                                            // extra launches and wave tails cost more than the HBM round trip saves
 
 static Planes with_ld(const Planes& p, int ld) {
   Planes q = p;
   q.ld = ld;
   return q;
-}
-static Planes first_planes(const Planes& p, int n) {
-  Planes q = p;
-  q.n = n < p.n ? n : p.n;
-  return q;
-}
-
-static bool fwd_tc_enabled() {   // tuning knob: ACX_CONV_FWD=0 keeps im2col + GEMM for the conv2 / conv3 forward
-  const char* e = getenv("ACX_CONV_FWD");
-  return e == nullptr || atoi(e) != 0;
 }
 
 static void setup_layers(acx_learner* l) {
@@ -210,13 +190,7 @@ static size_t layout(acx_learner* l, uint8_t* base) {
   l->dpre3 = take_planes(ar, ng, B2 * 49, c3);
   l->dpre2 = take_planes(ar, ng, B2 * 81, 64);
   l->dpre1 = take_planes(ar, ng, B2 * 400, 32);
-  {
-    const char* env = getenv("ACX_DGRAD_CHUNK_MB");   // tuning knob (0 = whole batch in one piece)
-    size_t mb = env ? (size_t)atoi(env) : (size_t)(kDgradChunkBytes >> 20);
-    const size_t whole = std::max(B2 * 49 * 576, B2 * 81 * 512) * sizeof(float);
-    l->dgrad_chunk_bytes = (mb == 0 || (mb << 20) > whole) ? whole : (mb << 20);
-  }
-  l->dP = ar.f32(l->dgrad_chunk_bytes / sizeof(float) + 81 * 512);   // one chunk of patch gradients
+  l->dP = ar.f32(std::max(B2 * 49 * 576, B2 * 81 * 512) + 81 * 512);   // patch gradients of the conv3 / conv2 input gradient
   // ---- preconditioning scratch
   int dmax = 0, cmax = 0;
   for (int i = 0; i < 6; ++i) {
@@ -229,8 +203,7 @@ static size_t layout(acx_learner* l, uint8_t* base) {
   const size_t kpad = align_up((size_t)49 * c3, 128);
   for (int i = 0; i < kMaxLanes; ++i) {
     Scratch& sc = l->scr[i];
-    sc.colsum_partial = ar.f32(std::max(std::max((size_t)kColsumChunks * (size_t)std::max(49 * c3, 576), (size_t)kBorderChunks * 28224),
-                                        (size_t)kGramChunks * 4096));
+    sc.colsum_partial = ar.f32(std::max((size_t)kColsumChunks * (size_t)std::max(49 * c3, 576), (size_t)kBorderChunks * 28224));
     sc.colsum_tmp = ar.f32(4096 + 28224 + 8);   // [0,4096): border / column-sum vectors, then the batch-summed conv input
     sc.ws_bytes = std::max<size_t>((size_t)48 << 20, kpad * kpad * sizeof(float) + (1 << 20));
     sc.ws = reinterpret_cast<float*>(ar.take(sc.ws_bytes));
@@ -325,7 +298,7 @@ static void register_buffers(acx_learner* l) {
   l->reg("values", l->values, (size_t)l->R * 4);
   l->reg("targets", l->targets, (size_t)l->N * 4);
   l->reg("advantages", l->adv, (size_t)l->N * 4);
-  l->reg("patches/conv1", l->P1.p[0], (size_t)l->R * 400 * 256 * 2);   // bf16 [R*400, 256], raw byte values (ACX_GATHER=0 only)
+  l->reg("patches/conv1", l->P1.p[0], (size_t)l->R * 400 * 256 * 2);   // bf16 [R*400, 256], raw byte values (conv_impl / gemm_impl = 1 only)
   l->reg("obs_pairs", l->obs_pairs, (size_t)l->R * 28224 * 2);         // bf16 [R, 42, 84, 2, 4]: the row-pair copy of the observations
   // hi planes of the forward activations = the ReLU masks the backward pass applies (act > 0); exposed so that the parity
   // tests can tell arithmetic error from units whose pre-activation is within rounding of zero
@@ -387,18 +360,10 @@ static int join_lane(acx_learner* l, const Lane& ln, cudaStream_t main_st) {
   return order_after(l, ln.st, main_st);
 }
 
-// triage: ACX_MAIN_CTAS / ACX_SIDE_CTAS cap the persistent grids of the tensor-core kernels of lane 0 / the side lanes
+// cap on the persistent grids of the tensor-core kernels of a lane (0 = all SMs)
 static int lane_cta_cap(const acx_learner* l, int lane_index) {
-  static int caps[2] = {-2, -2};
-  if (caps[0] == -2) {
-    const char* a = getenv("ACX_MAIN_CTAS");
-    const char* b = getenv("ACX_SIDE_CTAS");
-    caps[0] = a ? atoi(a) : -1;
-    caps[1] = b ? atoi(b) : 0;
-  }
-  if (lane_index != 0) return caps[1];
-  if (caps[0] >= 0) return caps[0];
-  // Default for K-FAC learners: the persistent grids of the caller's lane (forward, input gradients, conv1 weight gradient,
+  if (lane_index != 0) return 0;
+  // K-FAC learners: the persistent grids of the caller's lane (forward, input gradients, conv1 weight gradient,
   // preconditioning) leave 16 SMs to the factor / weight-gradient lanes, so that their kernels start beside the critical chain
   // instead of queueing behind it: 0.674 -> 0.656 ms/update at 32 x 20 (measured 96 / 112 / 120 / 132 / 140 CTAs: 0.671 / 0.660 /
   // 0.656 / 0.656 / 0.657; capping the side lanes instead is slower).  Learners without K-FAC side work keep every SM.
@@ -487,22 +452,16 @@ static int conv_input_factor(acx_learner* l, int li, const Planes& patches, cons
   GemmOut o;
   o.c = dst;
   o.ldc = d;
-  const bool gathered = ((l->gather_mask >> li) & 1) != 0;
-  if (gathered) {                    // P^T P read in place from the layer's input (conv1: columns in the row-pair copy's order)
+  if (l->gather) {                   // P^T P read in place from the layer's input (conv1: columns in the row-pair copy's order)
     o.a_gather = &l->gat_x[li];
     o.perm_m = o.perm_n = li == 0 ? 1 : 0;
-  } else if (li == 0 && l->conv1_patch) {   // P1^T P1 straight from the uint8 observations
-    o.a_patch = obs_u8;
-    o.a_patch_samples = l->N;
-  }
-  if (gathered) {
     Planes x;   // only the plane count matters
     x.n = l->gat_x[li].num_planes;
     x.ld = 8;
     for (int i = 0; i < x.n; ++i) x.p[i] = reinterpret_cast<bf16*>(const_cast<void*>(l->gat_x[li].planes[i]));
     ACX_TRY(run_gemm(l, x, x, 1, B.K, B.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
   } else {
-    ACX_TRY(run_gemm(l, first_planes(patches, o.a_patch ? 1 : patches.n), patches, 1, B.K, B.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
+    ACX_TRY(run_gemm(l, patches, patches, 1, B.K, B.K, rows, l->lvl_factor, scale_sq, 1, o, ln));
   }
   ACX_TRY(conv_border(obs_u8, act_in, l->N, L.hw_in, L.cin, L.k, L.s, L.hw_out, border_scale, lb.sc->colsum_partial, kBorderChunks,
                       lb.sc->colsum_tmp + 4096, dst, d, lb.st));
@@ -525,37 +484,16 @@ static int input_factor_stage(acx_learner* l, int stage, const Lane& ln, const L
 }
 
 // Nature-CNN forward on `rows` observations (envs/atari/model.py:173-217).  conv1 and fc4: im2col / flatten + GEMM with
-// bias/ReLU epilogues.  conv2 / conv3 (`conv_fwd_tc`): implicit-GEMM kernel straight from the activation planes
-// (conv.cu); their patch matrices - still the MN-major operands of wgrad and of the factor SYRKs - are then built on the
-// `aux` lane, off the forward's critical path (`patches_ready[l]` is raised on that lane), and acting (aux == nullptr)
-// skips them altogether.  Otherwise im2col + GEMM on the caller's stream.
+// bias/ReLU epilogues (conv1 with `gather`: implicit GEMM on the row-pair copy of the observations).  conv2 / conv3
+// (`conv_fwd_tc`): implicit-GEMM kernel straight from the activation planes (conv.cu); their input factors and weight
+// gradients read the same activations in place, so no patch matrix is built.  Otherwise im2col + GEMM on the caller's stream.
 // With `factors` every input factor is issued on the aux lane the moment its operand is complete, so the factor SYRKs
 // overlap the rest of the forward and the whole backward.
-// Input-factor stages (bit s = input_factor_stage s) that phase 1 leaves to phase 2.  Only the next inverse refresh reads
-// the factor statistics, while the parameter update needs nothing but the gradients: on a single GPU the big conv SYRKs
-// therefore run on a side lane of phase 2, under its chain of small latency-bound kernels (preconditioning, KL clip,
-// apply, operand planes - ~90 us during which the SMs were mostly idle), instead of queueing behind the other heavy
-// kernels of phase 1.  Their operands (patch matrices, activations) stay intact until the next update's forward pass.
-// Data-parallel learners all-reduce the statistics between the phases and keep everything in phase 1; so does a caller
-// that runs phase 1 alone (acx_learner_defer_input_factors is opt-in per update).
-static int deferred_factors(const acx_learner* l) { return l->deferred; }
-static int resolve_deferred(const acx_learner* l) {
-  if (l->cfg.world_size > 1 || l->lanes < 3 || l->profiling || !l->cfg.acktr || l->defer_request == 0) return 0;
-  if (l->defer_request > 0) return l->defer_request & 31;
-  static int mask = -1;
-  if (mask < 0) {
-    const char* e = getenv("ACX_DEFER_FACTORS");
-    mask = e ? atoi(e) & 31 : 6;   // the library's choice: the conv2 and conv3 input factors
-  }
-  return mask;
-}
-
 static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln, const Lane* aux, const Lane* aux2, bool factors) {
   const int c3 = l->c3;
   cudaStream_t st = ln.st;
   auto factor = [&](int stage) -> int {   // SYRK on aux, its border on aux2 (idle until the backward pass starts)
     if (!aux || !factors) return 0;
-    if (deferred_factors(l) & (1 << stage)) return 0;   // issued next to phase 2's latency-bound chain instead
     ACX_TRY(fork_lane(l, st, *aux));
     ACX_TRY(fork_lane(l, st, *aux2));
     return input_factor_stage(l, stage, *aux, *aux2);
@@ -572,14 +510,7 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
       ACX_TRY(factor(li));
       return run_gemm(l, patches, l->wT[li], 0, rows * L.T, B.C, B.K, l->lvl_fwd, 1.0f, 0, o, ln);
     }
-    if (aux && ((l->gather_mask >> li) & 1)) {
-      ACX_TRY(factor(li));   // the input factor reads the layer's input in place: nothing to build
-    } else if (aux) {
-      ACX_TRY(fork_lane(l, st, *aux));
-      ACX_TRY(im2col_bf16(in, patches, rows * L.T, L.hw_in, L.cin, L.k, L.s, L.hw_out, aux->st));
-      if (aux->st != st) ACX_TRY(record_tail(l, aux->st, &l->patches_ready[li]));
-      ACX_TRY(factor(li));
-    }
+    ACX_TRY(factor(li));   // the input factor reads the layer's input in place: nothing to build
     int pa[6], pb[6];
     const int np = level_pairs(l->lvl_fwd, in.n, l->wT[li].n, pa, pb);
     set_cta_cap(lane_cta_cap(l, 0));
@@ -590,7 +521,6 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
   GemmOut o;
   o.relu = 1;
   // conv1: raw bytes are exact in bf16; the /255 of envs/atari/model.py:93 is the GEMM alpha
-  // (with conv1_patch the GEMMs build the patch tiles themselves from `obs`: no im2col pass, no P1)
   o.bias = l->params + l->blk[0].off + (size_t)l->blk[0].K * l->blk[0].C;
   o.planes = &l->act1;
   if (l->gather) {
@@ -605,14 +535,9 @@ static int forward(acx_learner* l, const uint8_t* obs, int rows, const Lane& ln,
     set_cta_cap(0);
     ACX_TRY(rc);
   } else {
-    if (!l->conv1_patch) ACX_TRY(im2col_conv1(obs, l->P1.p[0], rows * 400, st));
+    ACX_TRY(im2col_conv1(obs, l->P1.p[0], rows * 400, st));
     ACX_TRY(factor(0));
-    if (l->conv1_patch) {
-      o.a_patch = obs;
-      o.a_patch_samples = rows;
-    }
     ACX_TRY(run_gemm(l, l->P1, l->wT[0], 0, rows * 400, 32, 256, l->lvl_fwd, 1.0f / 255.0f, 0, o, ln));
-    o.a_patch = nullptr;
   }
   ACX_TRY(conv_layer(1, l->act1, l->P2, l->act2));
   ACX_TRY(conv_layer(2, l->act2, l->P3, l->act3));
@@ -637,7 +562,7 @@ static int weight_grad(acx_learner* l, int li, const Planes& x, const Planes& g,
   GemmOut o;
   o.c = l->grads + L.off;
   o.ldc = L.C;
-  if (li < 3 && ((l->gather_mask >> li) & 1)) {   // X^T g with both operands read in place over the same locations
+  if (li < 3 && l->gather) {   // X^T g with both operands read in place over the same locations
     o.a_gather = &l->gat_x[li];
     o.b_gather = &l->gat_g[li];
     o.perm_m = li == 0 ? 1 : 0;
@@ -649,17 +574,14 @@ static int weight_grad(acx_learner* l, int li, const Planes& x, const Planes& g,
     if (with_bias) ACX_TRY(bias_grad(l, li, g, rows, ln));
     return 0;
   }
-  if (li == 0 && l->conv1_patch) {
-    o.a_patch = l->obs;
-    o.a_patch_samples = l->N;
-  }
   ACX_TRY(run_gemm(l, x, g, 1, L.K, L.C, rows, l->lvl_bwd, alpha, 0, o, ln));
   if (with_bias) ACX_TRY(bias_grad(l, li, g, rows, ln));
   return 0;
 }
 
-// input gradient of conv layer li: dP = g W^T (fp32) then col2im + ReLU mask of the layer below + bf16 split.  Done in
-// chunks of samples (optional, see kDgradChunkBytes: an L2-sized chunk keeps dP on chip, but measured slower).
+// input gradient of conv layer li: dP = g W^T (fp32) then col2im + ReLU mask of the layer below + bf16 split, over the whole
+// batch at once.  Chunks of samples small enough to keep dP in L2 measured slower on B200 at 32x20 (whole 1.510 ms/update,
+// 128 MB 1.533, 64 MB 1.551, 32 MB 1.599, 16 MB 1.681): the extra launches and wave tails cost more than the HBM round trip.
 static int conv_dgrad(acx_learner* l, int li, const Planes& g, const bf16* act_below_hi, const Planes& g_below, int samples,
                       const Lane& ln) {
   const Layer& L = l->L[li];
@@ -679,33 +601,19 @@ static int conv_dgrad(acx_learner* l, int li, const Planes& g, const bf16* act_b
     set_cta_cap(0);
     return rc;
   }
-  const size_t per_sample = (size_t)L.T * B.K * sizeof(float);
-  int chunk = (int)(l->dgrad_chunk_bytes / per_sample);
-  if (chunk < 1) chunk = 1;
-  for (int n0 = 0; n0 < samples; n0 += chunk) {
-    const int ns = std::min(chunk, samples - n0);
-    GemmOut o;
-    o.c = l->dP;
-    o.ldc = B.K;
-    ACX_TRY(run_gemm(l, offset_rows(g, (size_t)n0 * L.T), l->wN[li], 0, ns * L.T, B.K, B.C, l->lvl_bwd, 1.0f, 0, o, ln));
-    ACX_TRY(col2im_mask_split(l->dP, act_below_hi, g_below, n0, ns, l->N, L.hw_in, L.cin, L.k, L.s, L.hw_out, ln.st));
-  }
-  return 0;
+  GemmOut o;
+  o.c = l->dP;
+  o.ldc = B.K;
+  ACX_TRY(run_gemm(l, g, l->wN[li], 0, samples * L.T, B.K, B.C, l->lvl_bwd, 1.0f, 0, o, ln));
+  return col2im_mask_split(l->dP, act_below_hi, g_below, 0, samples, l->N, L.hw_in, L.cin, L.k, L.s, L.hw_out, ln.st);
 }
 
 // output factor G_l = g^T g / rows over the Fisher-sample rows
 static int output_factor(acx_learner* l, int li, const Planes& g_fisher, int rows, const Lane& ln) {
   const Block& L = l->blk[li];
   // Narrow output factors (C = 32 / 64 fill a 128 x 64 MMA tile to 1/8 .. 1/2) still run faster as a split-K SYRK on the
-  // tensor cores than on the fp32 SIMT Gram kernel (measured: 1.067 -> 1.043 ms/update; the MMAs are nearly free next to
-  // the one pass over g).  ACX_GRAM_TC=0 selects the SIMT kernel.
-  static int gram_tc = -1;
-  if (gram_tc < 0) {
-    const char* e = getenv("ACX_GRAM_TC");
-    gram_tc = e ? atoi(e) : 1;
-  }
-  if ((L.C == 32 || L.C == 64) && l->cfg.gemm_impl == 0 && !gram_tc)
-    return gram_small(g_fisher, rows, L.C, 1.0f / (float)rows, ln.sc->colsum_partial, kGramChunks, l->stats + l->goff[li], ln.st);
+  // tensor cores than on an fp32 SIMT Gram kernel (measured: 1.067 -> 1.043 ms/update; the MMAs are nearly free next to
+  // the one pass over g).
   GemmOut o;
   o.c = l->stats + l->goff[li];
   o.ldc = L.C;
@@ -722,7 +630,6 @@ static int issue_phase1(acx_learner* l, const int32_t* fisher_labels, const floa
   const bool fisher = l->sch.fisher();
   const int RB = fisher ? 2 * N : N;
   l->ev_next = 0;
-  for (cudaEvent_t& e : l->patches_ready) e = nullptr;
   const Lane main_ln = lane_of(l, 0, st), fac_ln = lane_of(l, 1, st), wg_ln = lane_of(l, 2, st), gf_ln = lane_of(l, 3, st),
              cs_ln = lane_of(l, 4, st);
   mark(l, 0, st);
@@ -771,18 +678,10 @@ static int issue_phase1(acx_learner* l, const int32_t* fisher_labels, const floa
     o.mask_rows = N;
     ACX_TRY(run_gemm(l, l->dpre4, l->wN[3], 0, RB, 49 * c3, 512, l->lvl_bwd, 1.0f, 0, o, main_ln));
   }
-  // ---- conv3  (patch matrices of implicit-GEMM forward layers come from the aux lane)
-  if (l->patches_ready[2] && wg_ln.st != fac_ln.st) {
-    ACX_TRY(fork_lane(l, st, wg_ln));
-    ACX_CUDA(cudaStreamWaitEvent(wg_ln.st, l->patches_ready[2], 0));
-  }
+  // ---- conv3
   ACX_TRY(fan_out(2, l->P3, l->dpre3, N * 49));
   ACX_TRY(conv_dgrad(l, 2, l->dpre3, l->act2.p[0], l->dpre2, RB, main_ln));
   // ---- conv2
-  if (l->patches_ready[1] && wg_ln.st != fac_ln.st) {
-    ACX_TRY(fork_lane(l, st, wg_ln));
-    ACX_CUDA(cudaStreamWaitEvent(wg_ln.st, l->patches_ready[1], 0));
-  }
   ACX_TRY(fan_out(1, l->P2, l->dpre2, N * 81));
   ACX_TRY(conv_dgrad(l, 1, l->dpre2, l->act1.p[0], l->dpre1, RB, main_ln));
   // ---- conv1 (no input gradient: observations are constants, envs/atari/model.py:101-104)
@@ -893,8 +792,6 @@ static int issue_phase2(acx_learner* l, const Plan& p, cudaStream_t st) {
       ema_ln = lane_of(l, 2, st);
       ACX_TRY(fork_lane(l, st, ema_ln));
     }
-    for (int stage = 0; stage < 5; ++stage)   // input factors that phase 1 left to this lane (see deferred_factors)
-      if (deferred_factors(l) & (1 << stage)) ACX_TRY(input_factor_stage(l, stage, ema_ln, ema_ln));
     ACX_TRY(ema_update(l->sums, l->stats, l->factor_floats, c.cov_ema_decay, 1.0f, ema_ln.st));
   }
   mark(l, 6, st);
@@ -940,11 +837,9 @@ static bool eager_graphs(const acx_learner* l) { return !l->cfg.use_graphs || l-
 
 static int phase2(acx_learner* l, cudaStream_t st) {
   const Plan p = l->sch.plan();
-  if (p.a2c || p.cold) l->deferred = 0;   // no covariance update in this phase: nothing can have been left to it
-  GraphKey key = {2, p.key() | (l->deferred << 5) | (l->external_ema ? 1 << 10 : 0) | (l->peer.world > 1 ? 1 << 11 : 0), nullptr, nullptr};
+  GraphKey key = {2, p.key() | (l->external_ema ? 1 << 10 : 0) | (l->peer.world > 1 ? 1 << 11 : 0), nullptr, nullptr};
   const int r = l->graphs.run(key, st, eager_graphs(l), [&]() { return issue_phase2(l, p, st); });
   if (r) return r;
-  l->deferred = 0;
   l->sch.advance(p);
   return 0;
 }
@@ -967,15 +862,7 @@ static int check_cfg(const acx_learner_config_t* c) {
 
 static void init_dims(acx_learner* l, const acx_learner_config_t* cfg) {
   l->cfg = *cfg;
-  {
-    // ACX_GATHER=0: round 1's materialised patch matrices P1 / P2 / P3 (im2col kernels)
-    const char* e = getenv("ACX_GATHER");
-    // ACX_GATHER = bit mask of the conv layers that read their patch operands in place (default 7 = all; 1 = conv1 only:
-    // conv2 / conv3 then build P2 / P3 with im2col_bf16 on a side lane as in round 1)
-    l->gather_mask = (cfg->gemm_impl == 0 && cfg->conv_impl == 0) ? (e == nullptr ? 7 : (atoi(e) & 7)) : 0;
-    if (l->gather_mask & 6) l->gather_mask |= 1;   // conv1 is the layer that pays most
-    l->gather = (l->gather_mask & 1) != 0;
-  }
+  l->gather = cfg->conv_impl == 0 && cfg->gemm_impl == 0;
   // precision: activations / gradients are kept as act_planes bf16 planes; a GEMM of level L accumulates the plane
   // pairs (i, j) with i + j <= L  (1 pair = bf16 inputs, 3 pairs ~ 2^-17, 6 pairs = fp32 class)
   switch (cfg->precision) {
@@ -1048,24 +935,10 @@ acx_learner_t* acx_learner_create(const acx_learner_config_t* cfg, void* d_arena
     acx_learner_destroy(l);
     return nullptr;
   }
-  {
-    // Opt-in (ACX_CONV1_PATCH=1): conv1's patch matrix generated inside the three GEMMs that read it (forward, wgrad, input
-    // factor) by eight producer warps from the uint8 observations - no im2col_conv1 pass, 550 MB less HBM traffic per
-    // update, bit-identical results - but measured slower on B200 (1.036 vs 1.016 ms/update: the ALU-built tiles arrive
-    // later than TMA's: forward 53 -> 67 us, wgrad 49 -> 60, SYRK 44 -> 53, against the 41 us im2col pass saved).
-    const char* e = getenv("ACX_CONV1_PATCH");
-    l->conv1_patch = cfg->gemm_impl == 0 && e != nullptr && atoi(e) != 0;
-  }
-  // implicit-GEMM forward of conv2 / conv3 only pays when its patch matrix can be built concurrently on another lane
   for (int i = 0; i < 4; ++i)
-    l->conv_fwd_tc[i] = (i == 1 || i == 2) && l->cfg.conv_impl == 0 && l->cfg.gemm_impl == 0 && (l->lanes > 1 || l->gather) && fwd_tc_enabled() &&
-                        conv_tc_supported(geom_of(l, i), 0);
-  int prio_lo = 0, prio_hi = 0;
-  cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);   // (numerically lowest = highest priority)
-  const char* pe = getenv("ACX_SIDE_PRIO");               // 1: side lanes at the lowest stream priority (triage)
-  const int side_prio = (pe && atoi(pe)) ? prio_lo : 0;
+    l->conv_fwd_tc[i] = (i == 1 || i == 2) && l->gather && conv_tc_supported(geom_of(l, i), 0);
   for (int i = 0; i + 1 < l->lanes; ++i)
-    if (cudaStreamCreateWithPriority(&l->side[i], cudaStreamNonBlocking, side_prio) != cudaSuccess) {
+    if (cudaStreamCreateWithFlags(&l->side[i], cudaStreamNonBlocking) != cudaSuccess) {
       acx::set_error("acx_learner_create: cudaStreamCreateWithFlags failed");
       acx_learner_destroy(l);
       return nullptr;
@@ -1185,9 +1058,7 @@ int acx_learner_phase1(acx_learner_t* l, const int32_t* d_fisher_labels, const f
   ACX_CHECK((d_fisher_labels == nullptr) == (d_fisher_eps == nullptr), "inject both Fisher labels and eps, or neither");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const bool fisher = l->sch.fisher();
-  l->deferred = fisher ? resolve_deferred(l) : 0;
-  l->defer_request = 0;   // one-shot
-  GraphKey key = {1, (fisher ? 1 : 0) | (l->deferred << 1) | (l->loss_variant << 8), d_fisher_labels, d_fisher_eps};
+  GraphKey key = {1, (fisher ? 1 : 0) | (l->loss_variant << 8), d_fisher_labels, d_fisher_eps};
   const int r = l->graphs.run(key, st, eager_graphs(l), [&]() { return issue_phase1(l, d_fisher_labels, d_fisher_eps, st); });
   l->a_ready_valid = r == 0 && fisher && l->lanes > 1 && !l->profiling;
   return r;
@@ -1217,11 +1088,8 @@ int acx_learner_update(acx_learner_t* l, const int32_t* d_fisher_labels, const f
   // both phases as ONE captured graph per schedule variant (nothing has to happen between them unless the caller runs a
   // collective there): one graph launch per update
   const bool fisher = l->sch.fisher();
-  l->deferred = fisher ? resolve_deferred(l) : 0;
-  l->defer_request = 0;
   const Plan p = l->sch.plan();
-  if (p.a2c || p.cold) l->deferred = 0;
-  const int k1 = (fisher ? 1 : 0) | (l->deferred << 1) | (l->loss_variant << 8);
+  const int k1 = (fisher ? 1 : 0) | (l->loss_variant << 8);
   const int k2 = p.key() | (l->external_ema ? 1 << 10 : 0) | (l->peer.world > 1 ? 1 << 11 : 0);
   GraphKey key = {4, k1 | (k2 << 16), d_fisher_labels, d_fisher_eps};
   const int r = l->graphs.run(key, st, eager_graphs(l), [&]() {
@@ -1230,7 +1098,6 @@ int acx_learner_update(acx_learner_t* l, const int32_t* d_fisher_labels, const f
   });
   l->a_ready_valid = false;
   if (r) return r;
-  l->deferred = 0;
   l->sch.advance(p);
   return 0;
 }
@@ -1294,13 +1161,6 @@ int acx_learner_wait_reduced(acx_learner_t* l, void* stream) {
   return 0;
 }
 
-int acx_learner_defer_input_factors(acx_learner_t* l, int stage_mask) {
-  ACX_CHECK(l, "null learner");
-  ACX_CHECK(stage_mask >= -1 && stage_mask <= 31, "stage_mask out of range");
-  l->defer_request = stage_mask;
-  return 0;
-}
-
 int acx_learner_wait_input_factors(acx_learner_t* l, void* stream) {
   ACX_CHECK(l, "null learner");
   if (!l->a_ready_valid) return -1;   // nothing was raised by the last phase 1: the prefix is complete only when phase 1 is
@@ -1328,15 +1188,6 @@ int acx_learner_get_state(const acx_learner_t* l, int64_t* global_step, int64_t*
   return 0;
 }
 
-static int act_pdl_level() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("ACX_ACT_PDL");
-    v = e ? atoi(e) : 2;
-  }
-  return v;
-}
-
 int acx_learner_act(acx_learner_t* l, const uint8_t* d_obs, int rows, const float* d_uniform, int greedy, int32_t* d_actions,
                     float* d_logits, float* d_values, void* stream) {
   ACX_CHECK(l && d_obs && d_actions, "null argument");
@@ -1349,7 +1200,7 @@ int acx_learner_act(acx_learner_t* l, const uint8_t* d_obs, int rows, const floa
     // the acting step is ONE serial chain of small launches on one stream: every kernel lets its successor be scheduled at
     // once (programmatic dependent launch, level 2) - inside an update the same setting gains nothing because the early
     // blocks compete with the other lanes
-    set_pdl_override(act_pdl_level());
+    set_pdl_override(2);
     int r = forward(l, d_obs, rows, lane_of(l, 0, st), nullptr, nullptr, false);
     if (r == 0) r = sample_actions(l->logits, d_uniform, l->cfg.seed, 0, rows, l->A, greedy, d_actions, st, l->act_counter);
     set_pdl_override(-1);

@@ -66,8 +66,6 @@ void fill_gemm(acx_gemm_t* g, const Planes& a, const Planes& b, int trans, int m
   g->mask_plane = o.mask;
   g->mask_ld = o.mask_ld;
   g->mask_rows = o.mask_rows;
-  g->a_patch_u8 = o.a_patch;
-  g->a_patch_samples = o.a_patch_samples;
   g->a_gather = o.a_gather;
   g->b_gather = o.b_gather;
   g->perm_m = o.perm_m;

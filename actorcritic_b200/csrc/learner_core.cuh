@@ -44,7 +44,7 @@ Planes offset_rows(const Planes& p, size_t rows);
 // plane pairs (i, j) with i + j <= level, low orders first
 int level_pairs(int level, int a_planes, int b_planes, int* pa, int* pb);
 
-// where a GEMM writes and what its epilogue does; the patch, gather and perm fields are the Atari learner's conv operands
+// where a GEMM writes and what its epilogue does; the gather and perm fields are the Atari learner's conv operands
 struct GemmOut {
   float* c = nullptr;
   int ldc = 0;
@@ -53,8 +53,6 @@ struct GemmOut {
   int relu = 0;
   const bf16* mask = nullptr;
   int mask_ld = 0, mask_rows = 0;
-  const uint8_t* a_patch = nullptr;   // A = conv1 patch matrix generated in the kernel from these observations
-  int a_patch_samples = 0;
   const acx_gather_t* a_gather = nullptr;   // operands read in place from NHWC tensors (acx.h)
   const acx_gather_t* b_gather = nullptr;
   int perm_m = 0, perm_n = 0;

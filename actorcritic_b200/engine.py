@@ -479,14 +479,9 @@ class Engine(_ArenaEngine):
             self._free[k].record(self.stream)
         self._stage_get += 1
 
-    def phase1(self, fisher_labels=None, fisher_eps=None, defer_factors=False):
-        """defer_factors: the caller runs `phase2` right after and reads no factor statistics in between - on a single
-        GPU the library then moves the conv2 / conv3 input-factor products under phase 2's chain of small kernels
-        (acx_learner_defer_input_factors)."""
+    def phase1(self, fisher_labels=None, fisher_eps=None):
         fl = ctypes.c_void_p(fisher_labels.data_ptr()) if fisher_labels is not None else None
         fe = ctypes.c_void_p(fisher_eps.data_ptr()) if fisher_eps is not None else None
-        if defer_factors and self.config.world_size == 1:
-            _lib.check(self.lib.acx_learner_defer_input_factors(self._h, -1))
         with self.on_stream():
             self.wait_pending_ema()      # the previous update's EMA (split exchange) still reads the statistics
             _lib.check(self.lib.acx_learner_phase1(self._h, fl, fe, self._stream()))
@@ -669,16 +664,14 @@ class Engine(_ArenaEngine):
         elif batch is not None:
             self.load_batch(batch["observations"], batch["bootstrap_observations"], batch["actions"], batch["rewards"],
                             batch["terminals"])
-        # ACX_DEFER_FACTORS=<mask>: opt-in (measured slower: the deferred SYRKs are persistent CTAs that hold an SM's whole
-        # shared memory, so phase 2's small kernels queue behind them instead of running beside them)
-        if self.config.world_size == 1 and "ACX_DEFER_FACTORS" not in os.environ and os.environ.get("ACX_ONE_GRAPH", "1") != "0":
+        if self.config.world_size == 1:
             # nothing happens between the phases on a single GPU: both as one captured graph (acx_learner_update)
             fl = ctypes.c_void_p(fisher_labels.data_ptr()) if fisher_labels is not None else None
             fe = ctypes.c_void_p(fisher_eps.data_ptr()) if fisher_eps is not None else None
             with self.on_stream():
                 _lib.check(self.lib.acx_learner_update(self._h, fl, fe, self._stream()))
         else:
-            self.phase1(fisher_labels, fisher_eps, defer_factors="ACX_DEFER_FACTORS" in os.environ)
+            self.phase1(fisher_labels, fisher_eps)
             self.allreduce(group)
             self.phase2()
         return self._fetched(fetch)

@@ -182,8 +182,8 @@ PAIRS = {1: [(0, 0)], 3: [(0, 0), (0, 1), (1, 0)], 6: [(0, 0), (0, 1), (1, 0), (
 
 
 def gemm(a_planes, b_planes, m, n, k, trans=False, pairs=None, alpha=1.0, bias=None, relu=False, symmetric=False,
-         out_planes=0, want_f32=True, mask=None, mask_rows=0, splits=0, impl=0, a_patch_obs=None, a_gather=None, b_gather=None,
-         perm_m=0, perm_n=0):
+         out_planes=0, want_f32=True, mask=None, mask_rows=0, splits=0, impl=0, a_gather=None, b_gather=None, perm_m=0,
+         perm_n=0):
     """C[m,n] = alpha * sum_pairs op(A_i) op(B_j) (+bias) via acx_gemm.
     trans=False: A planes stored [m,k], B planes stored [n,k];  trans=True: A stored [k,m], B stored [k,n]."""
     lib = _lib.load()
@@ -212,24 +212,11 @@ def gemm(a_planes, b_planes, m, n, k, trans=False, pairs=None, alpha=1.0, bias=N
         g.workspace, g.workspace_bytes = ws.data_ptr(), ws_bytes
         _lib.check(lib.acx_gemm(ctypes.byref(g), impl, _stream()))
         return c, []
-    dev = b_planes[0].device if a_patch_obs is None else a_patch_obs.device
-    if a_patch_obs is not None:
-        # A = the conv1 patch matrix of uint8 observations [samples, 84, 84, 4], generated inside the kernel (a_planes unused)
-        assert a_patch_obs.dtype == torch.uint8 and a_patch_obs.is_contiguous() and tuple(a_patch_obs.shape[1:]) == (84, 84, 4)
-        if pairs is None:
-            pairs = [(0, j) for j in range(len(b_planes))] if not symmetric else [(0, 0)]
-    elif pairs is None:
+    dev = b_planes[0].device
+    if pairs is None:
         pairs = PAIRS[{1: 1, 2: 3, 3: 6}[min(len(a_planes), len(b_planes))]]
     g = _lib.Gemm()
-    if a_patch_obs is not None:
-        g.a_patch_u8, g.a_patch_samples = a_patch_obs.data_ptr(), a_patch_obs.shape[0]
-        g.a.num_planes, g.a.ld = 1, 256
-        g.a.rows, g.a.cols = (k, m) if trans else (m, k)
-        if symmetric:
-            g.b.num_planes, g.b.ld, g.b.rows, g.b.cols = 1, 256, k, n
-        else:
-            g.b = _planes_struct(b_planes, k, n) if trans else _planes_struct(b_planes, n, k)
-    elif trans:
+    if trans:
         g.a = _planes_struct(a_planes, k, m)
         g.b = _planes_struct(b_planes, k, n)
     else:

@@ -124,12 +124,6 @@ typedef struct {
    * that may run concurrently need separate workspaces. */
   int splits;
   float* workspace; size_t workspace_bytes;
-  /* optional: A is NOT read from `a.planes` but generated inside the kernel as the conv1 patch matrix of uint8
-   * observations [a_patch_samples, 84, 84, 4] (8x8 kernel, stride 4 - envs/atari/model.py:173-179):
-   * P1[(r, oy, ox)][(kh, kw, c)] = obs[r, 4 oy + kh, 4 ox + kw, c], exact in one bf16 plane (a.num_planes = 1, pair_a = 0).
-   * trans_a == 0: A = P1 [m = patch rows, k = 256];  trans_a == 1: A = P1 [k = patch rows, m = 256]; with `symmetric`
-   * (n = 256) both sides are P1 and `b` is ignored.  Replaces extract_image_patches + the materialised patch matrix. */
-  const uint8_t* a_patch_u8; int a_patch_samples;
   /* optional (MN-major products only, trans_a == trans_b == 1): A and / or B are patch matrices read in place from NHWC
    * tensors (see acx_gather_t; `a.planes` / `b.planes` are then ignored and k = samples * gy * gx).  Both operands must
    * enumerate the same locations: either both are gathered over the same grid, or the product is `symmetric` and B = A.
@@ -173,9 +167,9 @@ int acx_debug_inv_trace(long long* h_out, int count);
 /* debug hook: override the UMMA shared-memory descriptor strides (bytes) used for MN-major operands;
  * 0 restores the built-in values. */
 void acx_debug_set_mn_desc(uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t kstep_bytes);
-/* where the split-K partials are summed: 0 = a finalize launch, 1 = inside the GEMM kernel where one SM can sum a tile's
- * partials in a few microseconds, else a finalize launch (default), 2 = always inside the kernel (two levels beyond 8
- * splits).  Every mode is deterministic.  Also ACX_GEMM_FUSE_REDUCE. */
+/* where the split-K partials are summed: 0 = a finalize launch (default), 1 = inside the GEMM kernel where one SM can sum a
+ * tile's partials in a few microseconds, else a finalize launch, 2 = always inside the kernel (two levels beyond 8 splits).
+ * Every mode is deterministic.  Also ACX_GEMM_FUSE_REDUCE. */
 void acx_debug_set_fuse_reduce(int mode);
 
 /* ---- implicit-GEMM convolution on bf16 planes (tcgen05 / TMEM / N-d TMA boxes) ---------------- */
@@ -327,15 +321,6 @@ int acx_learner_wait_reduced(acx_learner_t* l, void* stream);
 int acx_learner_peer_reduce_prefix(acx_learner_t* l, void* stream);
 int acx_peer_error(void);
 int acx_learner_ema(acx_learner_t* l, void* stream);
-/* Deferred input factors.  Only the next inverse refresh reads the K-FAC factor statistics, while the parameter update of
- * phase 2 needs nothing but the gradients.  With a non-zero `stage_mask` (bit s = input factor of conv1, conv2, conv3, fc4,
- * heads) the NEXT acx_learner_phase1 leaves those factor products to the following acx_learner_phase2, which runs them on
- * a side lane under its chain of small latency-bound kernels.  Callers that read the statistics, or all-reduce them,
- * between the two phases (data-parallel learners; world_size > 1 ignores the mask) keep the default 0.  -1 = the
- * library's choice (the conv2 and conv3 factors, or ACX_DEFER_FACTORS).  Measured on B200 (32 x 20): no gain - the factor
- * SYRKs are persistent CTAs that hold an SM's whole shared memory, so phase 2's small kernels queue behind them (end-to-end
- * 0.87 -> 0.93 .. 1.09 ms per update): opt-in only, results are identical either way (tests/test_gpu_learner.py). */
-int acx_learner_defer_input_factors(acx_learner_t* l, int stage_mask);
 /* optional stage timing with CUDA events on the launching stream (bench.py's live roofline numbers).
  * stages: 0 forward, 1 returns+loss+heads backward, 2 backward (dgrad+wgrad), 3 factor statistics,
  *         4 cold step / factor EMA, 5 inverse refresh, 6 preconditioning, 7 KL clip+momentum+apply+operand refresh.

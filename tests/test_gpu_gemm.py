@@ -5,6 +5,7 @@ contract of include/acx.h (arrival counters zero on entry, left zero).  The oper
 nn.py:110 (conv as patch GEMM), nn.py:48-52 (fully connected), tf.gradients of both (objectives.py:79) and kfac's
 factor statistics (SURVEY A.5)."""
 import ctypes
+import os
 
 import pytest
 import torch
@@ -55,11 +56,12 @@ CASES = [
 
 @pytest.fixture(params=[0, 1, 2], ids=["finalize_launch", "fused_where_cheap", "fused_always"])
 def reduce_mode(request):
-    """Where split-K partials are summed (acx.h: acx_debug_set_fuse_reduce); the library default is 1."""
+    """Where split-K partials are summed (acx.h: acx_debug_set_fuse_reduce).  Each case restores the library default
+    (ACX_GEMM_FUSE_REDUCE, else 0 = finalize launches), so the test files that run after this one see the mode users get."""
     _lib, _ = _ops()
     _lib.load().acx_debug_set_fuse_reduce(request.param)
     yield request.param
-    _lib.load().acx_debug_set_fuse_reduce(1)
+    _lib.load().acx_debug_set_fuse_reduce(int(os.environ.get("ACX_GEMM_FUSE_REDUCE", "0")))
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])

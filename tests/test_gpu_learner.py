@@ -97,28 +97,6 @@ def test_phase1_three_plane_preset_is_not_more_accurate():
     assert all(v["rel"] <= TOL_DEFAULT for v in a.values()) and all(v["rel"] <= TOL_DEFAULT for v in b.values())
 
 
-def test_deferred_input_factors_give_identical_updates():
-    """acx_learner_defer_input_factors moves the conv2 / conv3 factor products from phase 1 to a side lane of phase 2: the
-    learner state after every update must be bit-identical to the default schedule."""
-    eng = _engine_mod()
-    cfg = eng.EngineConfig(num_envs=4, num_steps=5, conv3_filters=32, num_cold_updates=2, invert_every=2)
-    states = []
-    for defer in (False, True):
-        e = eng.Engine(cfg)
-        e.set_params(onet.perturbed_params(4, 32, 3))
-        for u in range(6):
-            batch = synth.rollout(40 + u, 4, 5, 4, obs_kind="sparse")
-            y_hat, eps = synth.fisher_samples(70 + u, 20)
-            e.load_batch(batch["observations"], batch["bootstrap_observations"], batch["actions"], batch["rewards"],
-                         batch["terminals"])
-            e.phase1(torch.from_numpy(y_hat).cuda(), torch.from_numpy(eps).cuda(), defer_factors=defer)
-            e.phase2()
-        sd = e.state_dict()
-        states.append({k: sd[k] for k in ("params", "velocity", "factor_sums", "inverses")})
-    for k in states[0]:
-        assert torch.equal(states[0][k], states[1][k]), k
-
-
 def test_phase1_fast_precision_within_contract():
     errs = _compute(1, 8, 5, 32, "sparse")
     bad = {k: v for k, v in errs.items() if not v["rel"] <= TOL}

@@ -30,15 +30,8 @@ if name == "syrk_conv2_gather":   # the default path: A2 = P2^T P2 read in place
         durs.append(ms.value)
     print(name, "kernel-only us (library events):", " ".join("%.1f" % (1e3 * d) for d in durs))
     sys.exit(0)
-patch = name.endswith("_patch")
-if patch:
-    name = name[:-6]
 iters = int(sys.argv[2]) if len(sys.argv) > 2 else 3
 m, n, k, trans, sym, npl, outp = SHAPES[name]
-obs = None
-if patch:   # the A operand is generated inside the kernel from uint8 observations (conv1 shapes only)
-    rows = k if trans else m
-    obs = torch.randint(0, 256, (rows // 400, 84, 84, 4), dtype=torch.uint8, device="cuda")
 x = torch.randn((k, m) if trans else (m, k), device="cuda")
 a_pl = ops.split_planes(x, npl if name not in ("fwd_conv1", "wgrad_conv1") else 1)
 b_pl = a_pl if sym else ops.split_planes(torch.randn((k, n) if trans else (n, k), device="cuda"), npl)
@@ -47,7 +40,7 @@ if name in ("fwd_conv1", "wgrad_conv1"):
     pairs = [(0, 0), (0, 1), (0, 2)]
 bias = torch.randn(n, device="cuda") if outp else None
 for _ in range(iters):
-    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp), a_patch_obs=obs)
+    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp))
 torch.cuda.synchronize()
 import ctypes
 from actorcritic_b200 import _lib
@@ -55,7 +48,7 @@ lib = _lib.load()
 lib.acx_gemm_enable_timing(1)
 durs = []
 for _ in range(max(iters, 5)):
-    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp), a_patch_obs=obs)
+    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp))
     ms = ctypes.c_float(0)
     _lib.check(lib.acx_gemm_last_ms(ctypes.byref(ms)))
     durs.append(ms.value)
@@ -71,7 +64,7 @@ sys.exit(0)
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 e0.record()
 for _ in range(iters):
-    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp), a_patch_obs=obs)
+    ops.gemm(a_pl, b_pl, m, n, k, trans=trans, symmetric=sym, out_planes=outp, want_f32=outp == 0, pairs=pairs, bias=bias, relu=bool(outp))
 e1.record()
 torch.cuda.synchronize()
 print(name, "ms", e0.elapsed_time(e1) / iters)

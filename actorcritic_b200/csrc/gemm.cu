@@ -1615,14 +1615,10 @@ void acx_debug_set_fuse_reduce(int mode) { acx::g_fuse_mode = mode; }
 int acx_debug_tc_error(void) {
   int e = acx::tc_error_flag();
   if (!e) e = acx::conv_error_flag();
-  if (!e) e = acx::inv_error_flag();
   return e ? e : acx::inv_resident_error_flag();
 }
 
-int acx_debug_inv_trace(long long* h_out, int count) {
-  const char* e = getenv("ACX_INV_IMPL");
-  return (e && atoi(e) == 1) ? acx::inv_trace_read(h_out, count) : acx::inv_resident_trace_read(h_out, count);
-}
+int acx_debug_inv_trace(long long* h_out, int count) { return acx::inv_resident_trace_read(h_out, count); }
 
 int acx_debug_gemm_trace(long long* h_out4) {
   return cudaMemcpyFromSymbol(h_out4, acx::g_gemm_trace, 12 * sizeof(long long)) == cudaSuccess ? 0 : 1;

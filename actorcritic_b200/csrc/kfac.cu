@@ -1,6 +1,6 @@
 // kfac.cu - the K-FAC side of the ACKTR update that is not a GEMM: homogeneous border of the input
-// factors, the moving average of the factor statistics, pi-adjusted damping from traces, the damped SPD
-// inverses, the <V,U> reduction for the KL clip and the fused clip + momentum + apply steps (K-FAC,
+// factors, the moving average of the factor statistics, pi-adjusted damping from traces, the fp64 chain of
+// damped SPD inverses, the <V,U> reduction for the KL clip and the fused clip + momentum + apply steps (K-FAC,
 // cold momentum-SGD, RMSProp).  Semantics: SURVEY A.5 (tensorflow/kfac 0.1.x as driven by
 // kfac_utils.py:38-53 with the hyper-parameters of a2c_acktr.py:240-251) and nn.py:185-189.
 #include "layers.cuh"
@@ -84,6 +84,10 @@ __global__ void dampings_kernel(const float* const* __restrict__ a_ptrs, const f
 //   D^-1 = inv(M_pp);  R_j = D^-1 M_pj (j != p);  M_ij -= M_ip R_j (i, j != p);
 //   M_ip = -M_ip D^-1 (i != p);  M_pj = R_j;  M_pp = D^-1.
 // After the last block M holds the inverse.  2 n^3 flops; runs only every `invert_every` updates.
+// This chain is the fallback of the fp32 refresh with the tiles resident in shared memory (kfac_inv.cu): it runs when
+// those tiles do not fit the SMs (Atari conv3 > 64, wide fully connected layers).  The same fp64 arithmetic as one
+// persistent kernel with grid barriers between the steps was measured at 1.84 ms per refresh on a B200 at 32 x 20, no
+// faster than this chain, and was dropped (DESIGN.md section 4).
 // ------------------------------------------------------------------------------------------------
 constexpr int IB = 32;  // pivot block
 
@@ -350,368 +354,6 @@ __global__ void inv_finish_kernel(const InvDev* __restrict__ jobs) {
     jb.planes[0][i] = p0;
     jb.planes[1][i] = p1;
     jb.planes[2][i] = p2;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// The same inverse refresh as ONE persistent kernel (the default path).
-//
-// The chain above is 49 dependent pivot steps for the 1569 x 1569 factor of fc4, three launches each: ~150 launches whose
-// dependencies (launch latency + a cold start of every kernel) cost 22 - 37 us per step for ~3 us of arithmetic.  Here one
-// CTA per SM stays resident for the whole refresh and the steps are separated by grid-wide barriers (~1 us) instead of
-// kernel boundaries:
-//   phase D   pi-adjusted dampings (one warp per layer, CTAs 0..5)                                  | barrier
-//   phase P   M = debias * sym(S) + damp * I in fp64 (upper 64-tiles only); CTA j: D_0^-1 of job j  | barrier
-//   step p    panels: every 32 x 32 block b != p of every active job: Rold_b, R_b = D_p^-1 Rold_b; the CTA that owns
-//             block p + 1 of job j (CTA j) also forms the next pivot block as this step's update will leave it and
-//             inverts it - the serial 32-step Gauss-Jordan - WHILE the other CTAs run the update                       | barrier
-//             update: upper 64 x 64 tiles, M_ij -= sigma_i Rold_i^T R_j (+ pivot row / column / block)                   | barrier
-//   phase F   fp32 inverse + its three bf16 operand planes
-// Same arithmetic in the same order as the kernel chain above (bit-identical results; ACX_INV_IMPL=0 selects the chain).
-// Work is assigned statically (item i -> CTA i mod G): no atomics besides the barrier counter.  The kernel needs all its
-// CTAs resident at once: the grid is at most one CTA per SM (256 threads, 34 KB of shared memory), and a CTA that waits
-// at a barrier for longer than ~2 s records an error and leaves instead of hanging the device.
-// ------------------------------------------------------------------------------------------------
-static __device__ int g_inv_error = 0;
-// triage (ACX_INV_TRACE=1): per pivot step, clock64 stamps of thread 0 of the LAST CTA (a generic worker) [0] step start,
-// [1] panels done, [2] barrier 1 passed, [3] update done, [4] barrier 2 passed; of CTA 0 (look-ahead of the largest job):
-// [5] step start, [6] look-ahead panel + pivot inversion done
-static __device__ long long g_inv_trace[128 * 8];
-
-struct InvPersistArgs {
-  const InvDev* jobs;
-  int num_jobs;
-  int steps;                   // ceil(n_max / IB)
-  const Sched* sched;
-  float* damp;                 // [2 * num_layers]
-  const float* const* a_ptrs;
-  const float* const* g_ptrs;
-  const int* a_dims;
-  const int* g_dims;
-  const float* lambdas;
-  int num_layers;
-  unsigned int* bar;           // grid barrier counter, zero at launch
-  int trace;
-};
-
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int* p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-// all CTAs of the grid: everything written before is visible to everyone after.  Returns false after a timeout.
-__device__ __forceinline__ bool grid_barrier(unsigned int* bar, unsigned int& epoch) {
-  ++epoch;
-  const unsigned int target = epoch * gridDim.x;
-  __syncthreads();
-  int ok = 1;
-  if (threadIdx.x == 0) {
-    __threadfence();
-    atomicAdd(bar, 1u);
-    const long long t0 = clock64();
-    while (ld_acquire_u32(bar) < target) {
-      if (clock64() - t0 > 4000000000ll) {   // ~2 s: a CTA of the grid is not running
-        atomicExch(&g_inv_error, 21);
-        ok = 0;
-        break;
-      }
-    }
-    __threadfence();
-  }
-  return __syncthreads_and(ok) != 0;
-}
-
-__device__ __forceinline__ double ldcg_d(const double* p) { return __ldcg(p); }
-
-// one panel item: block `blk` (!= p) of job jb at step p -> Rold_blk, R_blk (global scratch); with `lookahead` also the
-// next pivot block, inverted into scratch_dinv(p + 1).  256 threads; d / t: 32 x 33 shared tiles.
-__device__ __forceinline__ void inv_panel_item(const InvDev& jb, int p, int blk, bool lookahead, double (*d)[IB + 1],
-                                               double (*t)[IB + 1]) {
-  const int n = jb.n;
-  const int p0 = p * IB, b0 = blk * IB;
-  const int tx = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const int nb = min(IB, n - p0);
-  const double* dinv = scratch_dinv(jb, p);
-  __syncthreads();   // the shared tiles may still be read by the previous item
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const int ty = w + 8 * q;
-    d[ty][tx] = ldcg_d(dinv + ty * IB + tx);
-    if ((b0 >> 6) >= (p0 >> 6)) {   // stored as a row of the pivot
-      const int cj = b0 + tx;
-      t[ty][tx] = (ty < nb && cj < n) ? ldcg_d(jb.m + (size_t)(p0 + ty) * n + cj) : 0.0;
-    } else {                        // only its mirror M_bp is stored (b processed, p not): M_pb = -M_bp^T
-      const int gi = b0 + ty;
-      t[tx][ty] = (gi < n && tx < nb) ? -ldcg_d(jb.m + (size_t)gi * n + p0 + tx) : 0.0;
-    }
-  }
-  __syncthreads();
-  const int cj = b0 + tx;
-  double acc[4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const int ty = w + 8 * q;
-    double a = 0.0;
-#pragma unroll 8
-    for (int k = 0; k < IB; ++k) a += d[ty][k] * t[k][tx];
-    acc[q] = a;
-    if (cj < n) {
-      __stcg(scratch_rold(jb) + (size_t)ty * n + cj, t[ty][tx]);
-      __stcg(scratch_r(jb) + (size_t)ty * n + cj, a);
-    }
-  }
-  if (!lookahead) return;
-  // look-ahead: D' = M_qq - Rold_q^T R_q (q = p + 1 is not processed yet: sigma = +1; same k order as the update)
-  __syncthreads();          // everyone is done reading d
-#pragma unroll
-  for (int q = 0; q < 4; ++q) d[w + 8 * q][tx] = acc[q];   // R_q
-  __syncthreads();
-  const int nbq = min(IB, n - b0);
-  double v[4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const int ty = w + 8 * q;
-    double x = (ty < nbq && tx < nbq) ? ldcg_d(jb.m + (size_t)(b0 + ty) * n + b0 + tx) : (ty == tx ? 1.0 : 0.0);
-    if (ty < nbq && tx < nbq) {
-#pragma unroll 8
-      for (int k = 0; k < IB; ++k) x -= t[k][ty] * d[k][tx];
-    }
-    v[q] = x;
-  }
-  __syncthreads();
-#pragma unroll
-  for (int q = 0; q < 4; ++q) d[w + 8 * q][tx] = v[q];
-  invert_block_smem<256>(d);
-  double* out = scratch_dinv(jb, p + 1);
-  for (int e = threadIdx.x; e < IB * IB; e += 256) __stcg(out + e, d[e >> 5][e & 31]);
-}
-
-// one update tile (ti <= tj) of job jb at step p; cs / rs: shared tiles [64][33] / [32][65]
-__device__ __forceinline__ void inv_update_tile(const InvDev& jb, int p, int ti, int tj, double (*cs)[IB + 1], double (*rs)[64 + 1]) {
-  const int n = jb.n;
-  const int p0 = p * IB;
-  const int i0 = ti * 64, j0 = tj * 64;
-  const int nb = min(IB, n - p0);
-  const double* rold = scratch_rold(jb);
-  const double* rb = scratch_r(jb);
-  __syncthreads();   // the shared tiles may still be read by the previous tile
-  {
-    double rc[8], rr[8];
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const int idx = threadIdx.x + 256 * q;
-      const int k = idx / 64, c = idx % 64;
-      const int gi = i0 + c, gj = j0 + c;
-      const double v = (gi < n && k < nb && !(gi >= p0 && gi < p0 + IB)) ? ldcg_d(rold + (size_t)k * n + gi) : 0.0;
-      rc[q] = gi < p0 ? -v : v;
-      rr[q] = (gj < n && k < nb && !(gj >= p0 && gj < p0 + IB)) ? ldcg_d(rb + (size_t)k * n + gj) : 0.0;
-    }
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const int idx = threadIdx.x + 256 * q;
-      cs[idx % 64][idx / 64] = rc[q];
-      rs[idx / 64][idx % 64] = rr[q];
-    }
-  }
-  __syncthreads();
-  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  double acc[4][4];
-#pragma unroll
-  for (int q = 0; q < 4; ++q)
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int gi = i0 + ty + 16 * q, gj = j0 + tx + 16 * r;
-      acc[q][r] = (gi < n && gj < n) ? ldcg_d(jb.m + (size_t)gi * n + gj) : 0.0;
-    }
-#pragma unroll 4
-  for (int k = 0; k < IB; ++k) {
-    double a[4], b[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      a[q] = cs[ty + 16 * q][k];
-      b[q] = rs[k][tx + 16 * q];
-    }
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-#pragma unroll
-      for (int r = 0; r < 4; ++r) acc[q][r] -= a[q] * b[r];
-  }
-  const double* dinv = scratch_dinv(jb, p);
-#pragma unroll
-  for (int q = 0; q < 4; ++q) {
-    const int gi = i0 + ty + 16 * q;
-    if (gi >= n) continue;
-    const bool ip = gi >= p0 && gi < p0 + IB;
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int gj = j0 + tx + 16 * r;
-      if (gj >= n) continue;
-      const bool jp = gj >= p0 && gj < p0 + IB;
-      double* dst = jb.m + (size_t)gi * n + gj;
-      double v;
-      if (ip && jp)
-        v = ldcg_d(dinv + (gi - p0) * IB + (gj - p0));
-      else if (ip)
-        v = ldcg_d(rb + (size_t)(gi - p0) * n + gj);                 // M_pj = R_j
-      else if (jp) {
-        const double x = ldcg_d(rb + (size_t)(gj - p0) * n + gi);    // M_ip = -sigma_i R_i^T
-        v = gi < p0 ? x : -x;
-      } else
-        v = acc[q][r];
-      __stcg(dst, v);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256, 1) inv_persistent_kernel(const InvPersistArgs a) {
-  __shared__ double sh0[64][IB + 1];   // update: sigma Rold^T tile; panels: d (rows 0..31) and t (rows 32..63)
-  __shared__ double sh1[IB][64 + 1];   // update: R tile
-  const int G = gridDim.x, cta = blockIdx.x;
-  unsigned int epoch = 0;
-  // ---- phase D: dampings (dampings_kernel), one warp of CTA l per layer
-  for (int l = cta; l < a.num_layers && threadIdx.x < 32; l += G) {
-    const int lane = threadIdx.x;
-    const float* pa = a.a_ptrs[l];
-    const float* pg = a.g_ptrs[l];
-    const int da = a.a_dims[l], dg = a.g_dims[l];
-    double ta = 0.0, tg = 0.0;
-    for (int i = lane; i < da; i += 32) ta += (double)__ldcg(pa + (size_t)i * da + i);
-    for (int i = lane; i < dg; i += 32) tg += (double)__ldcg(pg + (size_t)i * dg + i);
-    ta = warp_sum_d(ta);
-    tg = warp_sum_d(tg);
-    if (lane == 0) {
-      ta /= (double)da;
-      tg /= (double)dg;
-      const double pi = (ta > 0.0 && tg > 0.0) ? sqrt(ta / tg) : 1.0;
-      const double root = sqrt((double)a.lambdas[l]);
-      a.damp[2 * l] = (float)(pi * root);
-      a.damp[2 * l + 1] = (float)(root / pi);
-    }
-  }
-  if (!grid_barrier(a.bar, epoch)) return;
-  // ---- phase P: fp64 working copies (elements of upper 64-tiles only; the others are never read)
-  const float debias = a.sched->debias;
-  for (int j = 0; j < a.num_jobs; ++j) {
-    const InvDev jb = a.jobs[j];
-    const size_t total = (size_t)jb.n * jb.n;
-    const double dv = (double)__ldcg(a.damp + jb.damp_index);
-    for (size_t i = (size_t)cta * 256 + threadIdx.x; i < total; i += (size_t)G * 256) {
-      const int r = (int)(i / jb.n), c = (int)(i % jb.n);
-      if ((r >> 6) > (c >> 6)) continue;
-      const double v = 0.5 * ((double)__ldcg(jb.s + i) + (double)__ldcg(jb.s + (size_t)c * jb.n + r)) * (double)debias;
-      __stcg(jb.m + i, r == c ? v + dv : v);
-    }
-  }
-  double (*pd)[IB + 1] = sh0;
-  double (*pt)[IB + 1] = sh0 + IB;
-  for (int j0 = cta; j0 < a.num_jobs; j0 += G) {   // D_0^-1 of job j0, straight from S (same values as the working copy)
-    const InvDev jb = a.jobs[j0];
-    __syncthreads();
-    const int n = jb.n, nb = min(IB, n);
-    const double dv = (double)__ldcg(a.damp + jb.damp_index);
-    for (int e = threadIdx.x; e < IB * IB; e += 256) {
-      const int ty = e >> 5, tx = e & 31;
-      double v = ty == tx ? 1.0 : 0.0;
-      if (ty < nb && tx < nb) {
-        v = 0.5 * ((double)__ldcg(jb.s + (size_t)ty * n + tx) + (double)__ldcg(jb.s + (size_t)tx * n + ty)) * (double)debias;
-        if (ty == tx) v += dv;
-      }
-      pd[ty][tx] = v;
-    }
-    invert_block_smem<256>(pd);
-    double* dinv = scratch_dinv(jb, 0);
-    for (int e = threadIdx.x; e < IB * IB; e += 256) __stcg(dinv + e, pd[e >> 5][e & 31]);
-  }
-  if (!grid_barrier(a.bar, epoch)) return;
-  // ---- pivot steps
-  for (int p = 0; p < a.steps; ++p) {
-    int nact = 0;   // jobs are sorted by decreasing n: the active ones are a prefix
-    while (nact < a.num_jobs && a.jobs[nact].n > p * IB) ++nact;
-    if (nact == 0) break;
-    // workers = CTAs that take the generic items; CTAs [0, nact) own the look-ahead of their job (when the grid is too
-    // small to set them aside they also work as generic workers)
-    const bool dedicated = G >= 2 * nact + 8;
-    const int wbase = dedicated ? nact : 0;
-    const int nworkers = G - wbase;
-    const int wid = cta - wbase;
-    const bool tr_w = a.trace && p < 128 && cta == G - 1 && threadIdx.x == 0;
-    const bool tr_0 = a.trace && p < 128 && cta == 0 && threadIdx.x == 0;
-    if (tr_w) g_inv_trace[p * 8 + 0] = clock64();
-    if (tr_0) g_inv_trace[p * 8 + 5] = clock64();
-    // panels
-    for (int j0 = cta; j0 < nact; j0 += G) {
-      const InvDev jb = a.jobs[j0];
-      const int nblk = (jb.n + IB - 1) / IB;
-      if (p + 1 < nblk) inv_panel_item(jb, p, p + 1, true, pd, pt);
-    }
-    if (tr_0) g_inv_trace[p * 8 + 6] = clock64();
-    if (wid >= 0) {
-      int base = 0;
-      for (int j = 0; j < nact; ++j) {
-        const InvDev jb = a.jobs[j];
-        const int nblk = (jb.n + IB - 1) / IB;
-        // generic blocks of this job: all b except p and p + 1
-        const int skip_lo = p, skip_hi = p + 1 < nblk ? p + 1 : p;
-        const int cnt = nblk - (skip_hi - skip_lo + 1);
-        // first item of this job that belongs to this worker
-        int it = wid - (base % nworkers);
-        if (it < 0) it += nworkers;
-        for (; it < cnt; it += nworkers) {
-          int b = it;
-          if (b >= skip_lo) b += skip_hi - skip_lo + 1;
-          inv_panel_item(jb, p, b, false, pd, pt);
-        }
-        base += cnt;
-      }
-    }
-    if (tr_w) g_inv_trace[p * 8 + 1] = clock64();
-    if (!grid_barrier(a.bar, epoch)) return;
-    if (tr_w) g_inv_trace[p * 8 + 2] = clock64();
-    // update
-    if (wid >= 0) {
-      int base = 0;
-      for (int j = 0; j < nact; ++j) {
-        const InvDev jb = a.jobs[j];
-        const int nt = (jb.n + 63) / 64;
-        const int cnt = nt * (nt + 1) / 2;
-        int it = wid - (base % nworkers);
-        if (it < 0) it += nworkers;
-        for (; it < cnt; it += nworkers) {
-          // column-major enumeration of the upper triangle: it = tj (tj + 1) / 2 + ti, ti <= tj
-          int tj = (int)((sqrtf(8.0f * (float)it + 1.0f) - 1.0f) * 0.5f);
-          while (tj * (tj + 1) / 2 > it) --tj;
-          while ((tj + 1) * (tj + 2) / 2 <= it) ++tj;
-          const int ti = it - tj * (tj + 1) / 2;
-          inv_update_tile(jb, p, ti, tj, sh0, sh1);
-        }
-        base += cnt;
-      }
-    }
-    if (tr_w) g_inv_trace[p * 8 + 3] = clock64();
-    if (!grid_barrier(a.bar, epoch)) return;
-    if (tr_w) g_inv_trace[p * 8 + 4] = clock64();
-  }
-  // ---- phase F: fp32 inverse + bf16 planes (inv_finish_kernel)
-  for (int j = 0; j < a.num_jobs; ++j) {
-    const InvDev jb = a.jobs[j];
-    const int n = jb.n;
-    const size_t total = (size_t)n * jb.ld_planes;
-    for (size_t i = (size_t)cta * 256 + threadIdx.x; i < total; i += (size_t)G * 256) {
-      const int r = (int)(i / jb.ld_planes), c = (int)(i % jb.ld_planes);
-      float v = 0.0f;
-      if (c < n) {
-        const int tr = r >> 6, tc = c >> 6;
-        const double up = tr <= tc ? ldcg_d(jb.m + (size_t)r * n + c) : ldcg_d(jb.m + (size_t)c * n + r);
-        v = (float)(tr == tc ? 0.5 * (up + ldcg_d(jb.m + (size_t)c * n + r)) : up);
-        jb.inv[(size_t)r * n + c] = v;
-      }
-      bf16 p0, p1, p2;
-      split3(v, p0, p1, p2);
-      jb.planes[0][i] = p0;
-      jb.planes[1][i] = p1;
-      jb.planes[2][i] = p2;
-    }
   }
 }
 
@@ -1110,65 +752,6 @@ int spd_inverse_batched(const InvJob* h_jobs, const InvJob* d_jobs, int num_jobs
     inv_finish_kernel<<<grid, 256, 0, st>>>(dj);
     ACX_LAUNCH_CHECK();
   }
-  return 0;
-}
-
-int inv_trace_read(long long* h_out, int count) {
-  if (count > 128 * 8) count = 128 * 8;
-  return cudaMemcpyFromSymbol(h_out, g_inv_trace, (size_t)count * sizeof(long long)) == cudaSuccess ? 0 : 1;
-}
-int inv_error_flag() {
-  int v = 0;
-  cudaMemcpyFromSymbol(&v, g_inv_error, sizeof(int));
-  return v;
-}
-
-// the whole refresh (dampings included) as one persistent kernel; `bar`: 4 zero-initialised... bytes of device scratch
-int spd_inverse_persistent(const InvJob* h_jobs, const InvJob* d_jobs, int num_jobs, const Sched* sched, float* d_damp,
-                           const float* const* d_a_ptrs, const float* const* d_g_ptrs, const int* d_a_dims, const int* d_g_dims,
-                           const float* d_lambda, int num_layers, unsigned int* d_bar, cudaStream_t st) {
-  static_assert(sizeof(InvJob) == sizeof(InvDev), "InvJob and InvDev must have the same layout");
-  int nmax = 0;
-  for (int i = 0; i < num_jobs; ++i) nmax = h_jobs[i].n > nmax ? h_jobs[i].n : nmax;
-  ACX_CHECK(nmax > 0, "no inverse jobs");
-  ACX_CHECK(num_layers <= 6 && num_jobs <= 12, "too many jobs");
-  static int grid = 0;
-  if (grid == 0) {
-    int dev = 0, sms = 0, per_sm = 0;
-    ACX_CUDA(cudaGetDevice(&dev));
-    ACX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    ACX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, inv_persistent_kernel, 256, 0));
-    ACX_CHECK(per_sm >= 1 && sms >= 1, "inv_persistent_kernel does not fit an SM");
-    grid = sms;   // one CTA per SM: every CTA of the grid is resident at once (the barriers need that)
-    if (const char* e = getenv("ACX_INV_GRID")) {
-      const int v = atoi(e);
-      if (v >= 1 && v <= sms * per_sm) grid = v;
-    }
-  }
-  ACX_CUDA(cudaMemsetAsync(d_bar, 0, sizeof(unsigned int), st));
-  InvPersistArgs a;
-  a.jobs = reinterpret_cast<const InvDev*>(d_jobs);
-  a.num_jobs = num_jobs;
-  a.steps = ceil_div(nmax, IB);
-  a.sched = sched;
-  a.damp = d_damp;
-  a.a_ptrs = d_a_ptrs;
-  a.g_ptrs = d_g_ptrs;
-  a.a_dims = d_a_dims;
-  a.g_dims = d_g_dims;
-  a.lambdas = d_lambda;
-  a.num_layers = num_layers;
-  a.bar = d_bar;
-  {
-    static int tr = -1;
-    if (tr < 0) {
-      const char* e = getenv("ACX_INV_TRACE");
-      tr = e ? atoi(e) : 0;
-    }
-    a.trace = tr;
-  }
-  inv_persistent_kernel<<<grid, 256, 0, st>>>(a);
-  ACX_LAUNCH_CHECK();
   return 0;
 }
 

@@ -14,8 +14,11 @@
 //   look-ahead  one dedicated CTA per job (it owns no tiles) computes D_{p+1}^-1 = (M_qq - M_pq^T D_p^-1 M_pq)^-1 from the two
 //               blocks published during step p-1 - the serial 32-step inversion - while the owners run step p
 // Work and ownership are static (tile g -> CTA g mod W): no atomics besides the barrier counter; a CTA that waits at a
-// barrier for more than ~2 s records an error and leaves.  The fp64 kernel chain of kfac.cu remains as ACX_INV_IMPL=0 and
-// is used automatically when the tiles do not fit (conv3 widths beyond 64).
+// barrier for more than ~2 s records an error and leaves.  The fp64 kernel chain of kfac.cu is the fallback when the tiles do
+// not fit (conv3 widths beyond 64, wide fully connected layers).
+// The update phase was also built as four 64-thread groups with 8 x 8 register tiles: bit-identical, but measured slower on a
+// B200 at 32 x 20 (0.98 vs 0.85 ms per refresh: late pivot steps have only 2-3 active tiles per CTA, and a 2-warp group
+// cannot hide its own shared-memory latency), so it was removed.
 #include <cstdlib>
 
 #include "layers.cuh"
@@ -62,9 +65,6 @@ struct ResArgs {
   int num_layers;
   unsigned int* bar;
   int trace;
-  int debug;         // triage (ACX_INV_DEBUG): bit 1 = no operand prefetch
-  int groups;        // 4 = the update runs as four 64-thread groups (8 x 8 register tiles), 1 = one tile at a time on 256 threads
-  int group_stage_off;   // floats: staging of groups 1..3 behind the tile slots
 };
 
 __device__ int g_res_error = 0;
@@ -167,9 +167,7 @@ __device__ __forceinline__ float prep_value(const ResJob& jb, int gi, int gj, fl
 }
 
 // blocks (s, s+1) and (s+1, s+1) of the CURRENT matrix, if this tile holds them, for the look-ahead of step s
-__device__ __forceinline__ void publish_pair(const ResJob& jb, int s, int ti, int tj, const float* T, int tid = -1,
-                                             int nthr = RES_THREADS) {
-  if (tid < 0) tid = threadIdx.x;
+__device__ __forceinline__ void publish_pair(const ResJob& jb, int s, int ti, int tj, const float* T) {
   const int n = jb.n;
   const int nblk = (n + RB - 1) / RB;
   const int q = s + 1;
@@ -177,7 +175,7 @@ __device__ __forceinline__ void publish_pair(const ResJob& jb, int s, int ti, in
   if (ti == (s >> 1) && tj == (q >> 1)) {
     const int r0 = (s & 1) * RB, c0 = (q & 1) * RB;
     float* dst = sc_pq(jb, s);
-    for (int e = tid; e < RB * RB; e += nthr) {
+    for (int e = threadIdx.x; e < RB * RB; e += RES_THREADS) {
       const int y = e >> 5, x = e & 31;
       __stcg(dst + e, (q * RB + x < n) ? T[(r0 + y) * TS + c0 + x] : 0.0f);
     }
@@ -185,7 +183,7 @@ __device__ __forceinline__ void publish_pair(const ResJob& jb, int s, int ti, in
   if (ti == (q >> 1) && tj == (q >> 1)) {
     const int r0 = (q & 1) * RB;
     float* dst = sc_qq(jb, s);
-    for (int e = tid; e < RB * RB; e += nthr) {
+    for (int e = threadIdx.x; e < RB * RB; e += RES_THREADS) {
       const int y = e >> 5, x = e & 31;
       const bool in = q * RB + y < n && q * RB + x < n;
       __stcg(dst + e, in ? T[(r0 + y) * TS + r0 + x] : (y == x ? 1.0f : 0.0f));
@@ -357,125 +355,6 @@ __device__ __forceinline__ void update_tile(const ResJob& jb, int p, int ti, int
 #pragma unroll
   for (int q = 0; q < 4; ++q)
     *reinterpret_cast<float4*>(T + (4 * ty + q) * TS + 4 * tx) = make_float4(acc[q][0], acc[q][1], acc[q][2], acc[q][3]);
-}
-
-// ---- the same update with 64 threads per tile (8 x 8 elements each), four tiles of a CTA at a time ----------------
-// With 256 threads on one tile (4 x 4 each) a warp needs 8 shared-memory wavefronts per k for 16 FMAs: the update is bound
-// by shared-memory bandwidth (~2000 cycles per tile).  8 x 8 register tiles need 16 wavefronts for 64 FMAs, so four
-// 64-thread groups working on four tiles keep the FMA pipes busy instead (~1000 cycles per tile).  Same k order per
-// element: bit-identical results.
-constexpr int GROUP_THREADS = 64;
-constexpr int GROUP_STAGE = 3 * RB * OPLD;   // A | B | C pieces of one group
-
-struct OpRegs64 {
-  float4 a[8], b[8];
-};
-__device__ __forceinline__ void group_bar(int g) { asm volatile("bar.sync %0, 64;" ::"r"(g + 1) : "memory"); }
-
-__device__ __forceinline__ void fetch_ops64(const ResJob& jb, int p, int ti, int tj, int t, OpRegs64& o) {
-  const int n = jb.n, p0 = p * RB;
-  const float* rold = sc_rold(jb);
-  const float* rr = sc_r(jb);
-#pragma unroll
-  for (int h = 0; h < 8; ++h) {
-    const int e = t + h * GROUP_THREADS;   // 32 rows x 16 float4
-    const int k = e >> 4, c = (e & 15) * 4;
-    const int gi = ti * TS + c, gj = tj * TS + c;
-    float4 va = make_float4(0.f, 0.f, 0.f, 0.f), vb = va;
-    if (gi < n && !(gi >= p0 && gi < p0 + RB)) {
-      va = __ldcg(reinterpret_cast<const float4*>(rold + (size_t)k * jb.ldp + gi));
-      if (gi < p0) {
-        va.x = -va.x; va.y = -va.y; va.z = -va.z; va.w = -va.w;
-      }
-    }
-    if (gj < n && !(gj >= p0 && gj < p0 + RB)) vb = __ldcg(reinterpret_cast<const float4*>(rr + (size_t)k * jb.ldp + gj));
-    o.a[h] = va;
-    o.b[h] = vb;
-  }
-}
-__device__ __forceinline__ void stage_ops64(const ResJob& jb, int p, int ti, int tj, int t, const OpRegs64& o, float* As,
-                                            float* Bs, float* Cs) {
-#pragma unroll
-  for (int h = 0; h < 8; ++h) {
-    const int e = t + h * GROUP_THREADS;
-    const int k = e >> 4, c = (e & 15) * 4;
-    *reinterpret_cast<float4*>(As + k * OPLD + c) = o.a[h];
-    *reinterpret_cast<float4*>(Bs + k * OPLD + c) = o.b[h];
-  }
-  if (tj == (p >> 1) && ti != tj) {   // off-diagonal tile of the pivot's tile column: R for its row range (rare: not prefetched)
-    const float* rr = sc_r(jb);
-    float4 cr[8];
-#pragma unroll
-    for (int h = 0; h < 8; ++h) {
-      const int e = t + h * GROUP_THREADS;
-      const int k = e >> 4, gi = ti * TS + (e & 15) * 4;
-      cr[h] = gi < jb.n ? __ldcg(reinterpret_cast<const float4*>(rr + (size_t)k * jb.ldp + gi)) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-#pragma unroll
-    for (int h = 0; h < 8; ++h) {
-      const int e = t + h * GROUP_THREADS;
-      *reinterpret_cast<float4*>(Cs + (e >> 4) * OPLD + (e & 15) * 4) = cr[h];
-    }
-  }
-}
-
-// thread t of the group: rows 8 ty .. 8 ty + 7, columns 4 tx .. 4 tx + 3 and 32 + 4 tx .. 32 + 4 tx + 3 (so that a quarter
-// warp reads 128 contiguous bytes of the R piece and of the tile: no bank conflicts)
-__device__ __forceinline__ void update_tile64(const ResJob& jb, int p, int ti, int tj, int t, float* T, const float* As,
-                                              const float* Bs, const float* Cs) {
-  const int n = jb.n, p0 = p * RB, tp = p >> 1;
-  const int ty = t >> 3, tx = t & 7;
-  float acc[8][8];
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    const float4 lo = *reinterpret_cast<const float4*>(T + (8 * ty + q) * TS + 4 * tx);
-    const float4 hi = *reinterpret_cast<const float4*>(T + (8 * ty + q) * TS + 32 + 4 * tx);
-    acc[q][0] = lo.x; acc[q][1] = lo.y; acc[q][2] = lo.z; acc[q][3] = lo.w;
-    acc[q][4] = hi.x; acc[q][5] = hi.y; acc[q][6] = hi.z; acc[q][7] = hi.w;
-  }
-#pragma unroll 4
-  for (int k = 0; k < RB; ++k) {
-    const float4 a0 = *reinterpret_cast<const float4*>(As + k * OPLD + 8 * ty);
-    const float4 a1 = *reinterpret_cast<const float4*>(As + k * OPLD + 8 * ty + 4);
-    const float4 b0 = *reinterpret_cast<const float4*>(Bs + k * OPLD + 4 * tx);
-    const float4 b1 = *reinterpret_cast<const float4*>(Bs + k * OPLD + 32 + 4 * tx);
-    const float a[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-    const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-    for (int q = 0; q < 8; ++q)
-#pragma unroll
-      for (int r = 0; r < 8; ++r) acc[q][r] = fmaf(-a[q], b[r], acc[q][r]);
-  }
-  if (ti == tp || tj == tp) {
-    const float* dinv = sc_dinv(jb, p);
-    const float* Ri = ti == tj ? Bs : Cs;
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const int li = 8 * ty + q, gi = ti * TS + li;
-      const bool ip = gi >= p0 && gi < p0 + RB;
-#pragma unroll
-      for (int r = 0; r < 8; ++r) {
-        const int lj = (r < 4 ? 0 : 28) + 4 * tx + r, gj = tj * TS + lj;
-        const bool jp = gj >= p0 && gj < p0 + RB;
-        if (gi >= n || gj >= n || !(ip || jp)) continue;
-        float v;
-        if (ip && jp)
-          v = __ldcg(dinv + (gi - p0) * RB + (gj - p0));
-        else if (ip)
-          v = Bs[(gi - p0) * OPLD + lj];
-        else {
-          const float x = Ri[(gj - p0) * OPLD + li];
-          v = gi < p0 ? x : -x;
-        }
-        acc[q][r] = v;
-      }
-    }
-  }
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    *reinterpret_cast<float4*>(T + (8 * ty + q) * TS + 4 * tx) = make_float4(acc[q][0], acc[q][1], acc[q][2], acc[q][3]);
-    *reinterpret_cast<float4*>(T + (8 * ty + q) * TS + 32 + 4 * tx) = make_float4(acc[q][4], acc[q][5], acc[q][6], acc[q][7]);
-  }
 }
 
 // fp32 inverse + its bf16 operand planes from a resident tile (and its mirror)
@@ -691,66 +570,30 @@ __global__ void __launch_bounds__(RES_THREADS, 1) inv_resident_kernel(const __gr
     if (!grid_wait(a.bar, epoch)) return;
     if (tr) g_res_trace[p * 8 + 2] = clock64();
     // update (operands of the next tile are fetched while the current one is computed)
-    if (a.groups == 4) {
-      // four 64-thread groups, each on its own tile (8 x 8 register tiles), synchronised by named barriers
-      const int g = threadIdx.x >> 6, t = threadIdx.x & 63;
-      float* gA = (g == 0 ? stage : smem + a.group_stage_off + (g - 1) * GROUP_STAGE);
-      float* gB = gA + RB * OPLD;
-      float* gC = gB + RB * OPLD;
-      // the g-th, (g+4)-th ... active slot of this CTA
-      auto nth_active = [&](int from, int skip) {
-        for (; from < a.slots; ++from) {
-          if (s_job[from] < 0 || s_jobs[s_job[from]].n <= p0) continue;
-          if (skip == 0) return from;
-          --skip;
-        }
-        return a.slots;
-      };
-      int s = nth_active(0, g);
-      OpRegs64 regs;
-      if (s < a.slots) fetch_ops64(s_jobs[s_job[s]], p, s_ti[s], s_tj[s], t, regs);
-      while (s < a.slots) {
-        const ResJob& jb = s_jobs[s_job[s]];
-        const int ti = s_ti[s], tj = s_tj[s];
-        float* T = tiles + (size_t)s * TILE_FLOATS;
-        group_bar(g);                    // the group's previous tile is done with its staging buffers
-        stage_ops64(jb, p, ti, tj, t, regs, gA, gB, gC);
-        group_bar(g);
-        const int sn = nth_active(s + 1, 3);
-        if (sn < a.slots) fetch_ops64(s_jobs[s_job[sn]], p, s_ti[sn], s_tj[sn], t, regs);
-        update_tile64(jb, p, ti, tj, t, T, gA, gB, gC);
-        group_bar(g);
-        publish_pair(jb, p + 1, ti, tj, T, t, GROUP_THREADS);    // for the look-ahead of step p + 1
-        s = sn;
-      }
-    } else {
-      int s = 0;
-      auto next_active = [&](int from) {
-        while (from < a.slots && (s_job[from] < 0 || s_jobs[s_job[from]].n <= p0)) ++from;
-        return from;
-      };
-      s = next_active(0);
-      const int first = s;
-      OpRegs regs;
-      if (s < a.slots) fetch_ops(s_jobs[s_job[s]], p, s_ti[s], s_tj[s], regs);
-      while (s < a.slots) {
-        const ResJob& jb = s_jobs[s_job[s]];
-        const int ti = s_ti[s], tj = s_tj[s];
-        float* T = tiles + (size_t)s * TILE_FLOATS;
-        __syncthreads();                 // the previous tile is done with the staging buffers
-        stage_ops(regs, As, Bs, Cs, tj == (p >> 1) && ti != tj);
-        __syncthreads();
-        if (tr2 && s == first) g_res_trace[p * 8 + 5] = clock64();
-        const int sn = next_active(s + 1);
-        if (sn < a.slots && !(a.debug & 2)) fetch_ops(s_jobs[s_job[sn]], p, s_ti[sn], s_tj[sn], regs);
-        update_tile(jb, p, ti, tj, T, As, Bs, Cs);
-        if (tr2 && s == first) g_res_trace[p * 8 + 6] = clock64();
-        __syncthreads();
-        if (sn < a.slots && (a.debug & 2)) fetch_ops(s_jobs[s_job[sn]], p, s_ti[sn], s_tj[sn], regs);
-        publish_pair(jb, p + 1, ti, tj, T);    // for the look-ahead of step p + 1
-        if (tr2 && s == first) g_res_trace[p * 8 + 7] = clock64();
-        s = sn;
-      }
+    auto next_active = [&](int from) {
+      while (from < a.slots && (s_job[from] < 0 || s_jobs[s_job[from]].n <= p0)) ++from;
+      return from;
+    };
+    int s = next_active(0);
+    const int first = s;
+    OpRegs regs;
+    if (s < a.slots) fetch_ops(s_jobs[s_job[s]], p, s_ti[s], s_tj[s], regs);
+    while (s < a.slots) {
+      const ResJob& jb = s_jobs[s_job[s]];
+      const int ti = s_ti[s], tj = s_tj[s];
+      float* T = tiles + (size_t)s * TILE_FLOATS;
+      __syncthreads();                 // the previous tile is done with the staging buffers
+      stage_ops(regs, As, Bs, Cs, tj == (p >> 1) && ti != tj);
+      __syncthreads();
+      if (tr2 && s == first) g_res_trace[p * 8 + 5] = clock64();
+      const int sn = next_active(s + 1);
+      if (sn < a.slots) fetch_ops(s_jobs[s_job[sn]], p, s_ti[sn], s_tj[sn], regs);
+      update_tile(jb, p, ti, tj, T, As, Bs, Cs);
+      if (tr2 && s == first) g_res_trace[p * 8 + 6] = clock64();
+      __syncthreads();
+      publish_pair(jb, p + 1, ti, tj, T);    // for the look-ahead of step p + 1
+      if (tr2 && s == first) g_res_trace[p * 8 + 7] = clock64();
+      s = sn;
     }
     if (tr) g_res_trace[p * 8 + 3] = clock64();
     grid_arrive(a.bar, epoch);
@@ -790,11 +633,7 @@ int spd_inverse_resident(const InvJob* h_jobs, int num_jobs, const Sched* sched,
     ACX_CUDA(cudaGetDevice(&dev));
     ACX_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   }
-  int grid = sms;
-  if (const char* e = getenv("ACX_INV_GRID")) {
-    const int v = atoi(e);
-    if (v >= 1 && v <= sms) grid = v;
-  }
+  const int grid = sms;
   if (grid < num_jobs + 8) return -1;
   ResArgs a;
   int nmax = 0, total = 0;
@@ -818,7 +657,7 @@ int spd_inverse_resident(const InvJob* h_jobs, int num_jobs, const Sched* sched,
   const int owners = grid - num_jobs;
   int slots = ceil_div(total, owners);
   if (slots < 2) slots = 2;   // the look-ahead CTAs use the tile area for five 32 x 33 blocks
-  size_t smem = ((size_t)STAGE_FLOATS + (size_t)slots * TILE_FLOATS) * sizeof(float);
+  const size_t smem = ((size_t)STAGE_FLOATS + (size_t)slots * TILE_FLOATS) * sizeof(float);
   static int dyn_limit = -1;
   if (dyn_limit < 0) {
     cudaFuncAttributes fa;
@@ -827,20 +666,6 @@ int spd_inverse_resident(const InvJob* h_jobs, int num_jobs, const Sched* sched,
     ACX_CUDA(cudaFuncSetAttribute(inv_resident_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit));
   }
   if (slots > 16 || smem > (size_t)dyn_limit) return -1;
-  // ACX_INV_GROUPS=4 (opt-in): the update phase as four 64-thread groups with 8 x 8 register tiles, when their staging fits
-  // next to the tiles.  Bit-identical, but measured SLOWER on B200 at 32 x 20 (0.98 vs 0.85 ms per refresh): late pivot steps
-  // have only 2-3 active tiles per CTA, and a 2-warp group cannot hide its own shared-memory latency.
-  static int want_groups = -1;
-  if (want_groups < 0) {
-    const char* e = getenv("ACX_INV_GROUPS");
-    want_groups = e ? atoi(e) : 1;
-  }
-  a.groups = 1;
-  a.group_stage_off = STAGE_FLOATS + slots * TILE_FLOATS;
-  if (want_groups == 4 && smem + (size_t)3 * GROUP_STAGE * sizeof(float) <= (size_t)dyn_limit) {
-    a.groups = 4;
-    smem += (size_t)3 * GROUP_STAGE * sizeof(float);
-  }
   a.num_jobs = num_jobs;
   a.steps = ceil_div(nmax, RB);
   a.slots = slots;
@@ -861,12 +686,6 @@ int spd_inverse_resident(const InvJob* h_jobs, int num_jobs, const Sched* sched,
       tr = e ? atoi(e) : 0;
     }
     a.trace = tr;
-    static int dbg = -1;
-    if (dbg < 0) {
-      const char* e = getenv("ACX_INV_DEBUG");
-      dbg = e ? atoi(e) : 0;
-    }
-    a.debug = dbg;
   }
   ACX_CUDA(cudaMemsetAsync(d_bar, 0, sizeof(unsigned int), st));
   inv_resident_kernel<<<grid, RES_THREADS, smem, st>>>(a);

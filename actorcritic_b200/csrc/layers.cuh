@@ -98,17 +98,12 @@ int compute_dampings(const float* const* d_a_ptrs, const float* const* d_g_ptrs,
                      const float* d_lambda, int num_layers, float* d_damp, cudaStream_t st);
 int spd_inverse_batched(const InvJob* h_jobs, const InvJob* d_jobs, int num_jobs, const Sched* sched, const float* d_damp,
                         cudaStream_t st, cudaStream_t side = nullptr);
-int spd_inverse_persistent(const InvJob* h_jobs, const InvJob* d_jobs, int num_jobs, const Sched* sched, float* d_damp,
-                           const float* const* d_a_ptrs, const float* const* d_g_ptrs, const int* d_a_dims, const int* d_g_dims,
-                           const float* d_lambda, int num_layers, unsigned int* d_bar, cudaStream_t st);
 // kfac_inv.cu: fp32 refresh with the factor tiles resident in shared memory; -1 = does not fit (use the chain above)
 int spd_inverse_resident(const InvJob* h_jobs, int num_jobs, const Sched* sched, float* d_damp, const float* const* d_a_ptrs,
                          const float* const* d_g_ptrs, const int* d_a_dims, const int* d_g_dims, const float* d_lambda,
                          int num_layers, unsigned int* d_bar, cudaStream_t st);
 int inv_resident_error_flag();
 int inv_resident_trace_read(long long* h_out, int count);
-int inv_error_flag();
-int inv_trace_read(long long* h_out, int count);
 int sched_step(Sched* s, float lr_start, float lr_end, double decay_steps, float* out_lr, int gs_inc, int ncov_inc,
                float ema_decay, int zero_debias, cudaStream_t st);
 int sched_begin(Sched* s, float lr_start, float lr_end, double decay_steps, float* out_lr, cudaStream_t st);

@@ -796,25 +796,9 @@ static int issue_phase2(acx_learner* l, const Plan& p, cudaStream_t st) {
   }
   mark(l, 6, st);
   if (p.invert) ACX_TRY(join_lane(l, sched_ln, st));   // the refresh reads the zero-debias factor of the new covariance count
-  if (p.invert) {
-    // ACX_INV_IMPL: 2 (default) = fp32, all factor tiles resident in shared memory, one persistent kernel (kfac_inv.cu);
-    // 1 = the fp64 Gauss-Jordan as one persistent kernel; 0 = the round-1 fp64 chain of ~150 launches (also the fallback when
-    // the tiles do not fit the SMs' shared memory)
-    static int inv_impl = -1;
-    if (inv_impl < 0) {
-      const char* e = getenv("ACX_INV_IMPL");
-      inv_impl = e ? atoi(e) : 2;
-    }
-    // (the serial pivot-block inversions of the chain run on a side lane next to the trailing updates, joined inside, step by step)
-    const cudaStream_t side = lane_of(l, 1, st).st;
-    if (inv_impl == 2)
-      ACX_TRY(l->invert(st, side));
-    else if (inv_impl == 1)
-      ACX_TRY(spd_inverse_persistent(l->h_jobs, l->d_jobs, 12, l->sched, l->damp, l->d_a_ptrs, l->d_g_ptrs, l->d_a_dims,
-                                     l->d_g_dims, l->lambdas, 6, l->inv_bar, st));
-    else
-      ACX_TRY(l->invert_chain(st, side));
-  }
+  // (when the refresh falls back to the fp64 chain, its serial pivot-block inversions run on a side lane next to the
+  // trailing updates, joined inside, step by step)
+  if (p.invert) ACX_TRY(l->invert(st, lane_of(l, 1, st).st));
   mark(l, 7, st);
   if (p.kfac_apply) {
     ACX_TRY(precondition(l, st));

@@ -276,10 +276,7 @@ int KfacBlocks::split_inverses(cudaStream_t st) {
 
 int KfacBlocks::invert(cudaStream_t st, cudaStream_t side) {
   const int r = spd_inverse_resident(h_jobs, 2 * nb, sched, damp, d_a_ptrs, d_g_ptrs, d_a_dims, d_g_dims, lambdas, nb, inv_bar, st);
-  return r < 0 ? invert_chain(st, side) : r;
-}
-
-int KfacBlocks::invert_chain(cudaStream_t st, cudaStream_t side) {
+  if (r >= 0) return r;
   ACX_TRY(compute_dampings(d_a_ptrs, d_g_ptrs, d_a_dims, d_g_dims, lambdas, nb, damp, st));
   return spd_inverse_batched(h_jobs, d_jobs, 2 * nb, sched, damp, st, side);
 }

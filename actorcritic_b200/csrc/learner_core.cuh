@@ -117,10 +117,9 @@ struct KfacBlocks {
   int get_params(float* h_params, cudaStream_t st);
   // the bf16 planes of the stored inverses (derived state, after the inverses were written from outside)
   int split_inverses(cudaStream_t st);
-  // inverse refresh: factor tiles resident in shared memory (kfac_inv.cu), else `invert_chain`
+  // inverse refresh: factor tiles resident in shared memory (kfac_inv.cu); when they do not fit, dampings and then the
+  // fp64 chain (kfac.cu), with its serial pivot-block inversions on `side` when given
   int invert(cudaStream_t st, cudaStream_t side = nullptr);
-  // dampings, then the fp64 chain (the serial pivot-block inversions on `side` when given)
-  int invert_chain(cudaStream_t st, cudaStream_t side = nullptr);
 };
 
 // what one update's optimizer step does, decided on the host from the schedule counters (kfac_utils.py:38-53)

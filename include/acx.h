@@ -160,9 +160,10 @@ int acx_debug_tc_error(void);
 /* triage: with ACX_GEMM_TRACE=1 in the environment, CTA 0 of the last acx_gemm launch records cycle counts of its MMA warp:
  * [0] total, [1] waiting for operands, [2] waiting for a drained accumulator, [3] k-blocks processed. */
 int acx_debug_gemm_trace(long long* h_out4);
-/* triage: with ACX_INV_TRACE=1 the persistent inverse-refresh kernel records, per pivot step (8 slots each), clock64 stamps
- * of a worker CTA ([0] step start [1] panels done [2] barrier passed [3] update done [4] barrier passed) and of CTA 0
- * ([5] step start [6] look-ahead pivot inversion done); copies `count` (<= 1024) values. */
+/* triage: with ACX_INV_TRACE=1 the resident inverse-refresh kernel records, per pivot step (8 slots each), clock64 stamps
+ * of the last owner CTA ([0] step start [1] panels done [2] barrier passed [3] update done [4] barrier passed) and of
+ * look-ahead CTA 0 ([5] step start [6] pivot inversion done [7] barrier passed); a refresh that falls back to the fp64
+ * chain records nothing.  Copies `count` (<= 1024) values. */
 int acx_debug_inv_trace(long long* h_out, int count);
 /* debug hook: override the UMMA shared-memory descriptor strides (bytes) used for MN-major operands;
  * 0 restores the built-in values. */

@@ -9,6 +9,7 @@ from oracle import kfac as K
 from oracle import learner as OL
 from oracle import network as onet
 
+from actorcritic_b200 import _lib
 from actorcritic_b200 import engine as eng
 
 
@@ -151,7 +152,9 @@ def run_schedule(cfg, num_updates, seed=0, obs_kind="uniform", collect=None, res
         gs_before = e.global_step
         assert gs_before == o.global_step
         params_before = oracle_flat_params(o)
+        launches_before = _lib.launch_count()
         scal = e.update(batch, fl if cfg.acktr else None, fe if cfg.acktr else None)
+        launches = _lib.launch_count() - launches_before
         # the oracle differentiates its ReLUs at the engine's masks (the forward activations of this update are still in
         # the arena), and the units where that differs from its own branch must be within rounding of zero
         masks = engine_relu_masks(e)
@@ -159,7 +162,7 @@ def run_schedule(cfg, num_updates, seed=0, obs_kind="uniform", collect=None, res
         for name, (count, frac, worst) in mask_disagreement(masks, info["fwd"]).items():
             assert worst <= 1e-4 and frac <= 1e-3, ("ReLU branch disagreement", u, name, count, frac, worst)
         torch.cuda.synchronize()
-        rec = dict(update=u, gs_before=gs_before, gs_after=e.global_step, oracle_gs_after=o.global_step,
+        rec = dict(update=u, gs_before=gs_before, gs_after=e.global_step, oracle_gs_after=o.global_step, launches=launches,
                    params_rel=rel_err(e.get_params_flat(), oracle_flat_params(o)),
                    step_rel=rel_err(e.get_params_flat().astype(np.float64) - params_before,
                                     oracle_flat_params(o) - params_before),

@@ -310,15 +310,31 @@ def test_full_update_with_inverse_refresh_headline_size(kind):
     assert 0.0 < records[-1]["clip_coeff"][0] <= 1.0
 
 
-def test_full_update_with_inverse_refresh_conv3_64():
-    """The class default conv3 = 64 (envs/atari/model.py:45): the 3137 x 3137 input factor of fc4 that north_star names
-    is accumulated, inverted and used by the fc4 preconditioning GEMMs."""
+def _wide_refresh_launches(c3):
+    """A refreshing update at 8 envs x 5 steps against the oracle; returns the kernel launches the refresh update adds to
+    the covariance-only update before it.  The resident refresh is one launch, the fp64 chain about three per 32-row
+    pivot step of the largest factor."""
     eng = _engine_mod()
-    cfg = eng.EngineConfig(num_envs=8, num_steps=5, conv3_filters=64, num_cold_updates=0, invert_every=1)
+    cfg = eng.EngineConfig(num_envs=8, num_steps=5, conv3_filters=c3, num_cold_updates=0, invert_every=1)
     records = _refreshing_update(cfg, "sparse")
     assert records[-1]["inv_A"]["fc4"] <= TOL_DEFAULT
     _check_schedule(records, TOL_DEFAULT)
     assert records[-1]["step_rel"] <= TOL_DEFAULT, records[-1]["step_rel"]
+    return records[1]["launches"] - records[0]["launches"]
+
+
+def test_full_update_with_inverse_refresh_conv3_64():
+    """The class default conv3 = 64 (envs/atari/model.py:45): the 3137 x 3137 input factor of fc4 that north_star names
+    is accumulated, inverted by the resident kernel and used by the fc4 preconditioning GEMMs."""
+    added = _wide_refresh_launches(64)
+    assert added < 100, added
+
+
+def test_full_update_with_inverse_refresh_conv3_96_fp64_chain():
+    """conv3 = 96: the 4705 x 4705 input factor of fc4 is 2775 upper 64-tiles, more than the SMs' shared memory holds,
+    so the refresh falls back to the fp64 kernel chain (148 pivot steps for fc4)."""
+    added = _wide_refresh_launches(96)
+    assert added > 300, added
 
 
 @pytest.mark.parametrize("tag", ["reference", "short", "odd"])

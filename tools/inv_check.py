@@ -1,6 +1,8 @@
-"""python tools/inv_check.py [c3]: runs 4 refreshing updates (invert_every = 1) and prints a digest of the inverses plus the
-inverse-stage time; run once with ACX_INV_IMPL=1 (persistent kernel) and once with ACX_INV_IMPL=0 (kernel chain): the
-digests must be identical (same arithmetic in the same order)."""
+"""python tools/inv_check.py [c3]: runs 4 refreshing updates (invert_every = 1) and prints a digest of the inverses (equal
+digests across two builds mean bit-identical inverses), their error against numpy fp64, the inverse-stage time and which
+refresh path ran, read from the launch count: the resident fp32 kernel is one launch, its fallback for factors whose tiles do
+not fit the SMs (conv3 > 64) is the fp64 chain of about three launches per 32-row pivot step.  With ACX_INV_TRACE=1|2 it
+also prints the per-step clock64 breakdown of the resident kernel."""
 import hashlib
 import os
 import sys
@@ -27,7 +29,7 @@ for u in range(4):
     e.update(b, fl, fe, fetch=False)
 torch.cuda.synchronize()
 inv = e.buffer("inverses").cpu().numpy()
-print("impl", os.environ.get("ACX_INV_IMPL", "1"), "c3", c3, "tc_error", _lib.load().acx_debug_tc_error(),
+print("c3", c3, "tc_error", _lib.load().acx_debug_tc_error(),
       "finite", bool(np.isfinite(inv).all()), "digest", hashlib.sha1(inv.tobytes()).hexdigest()[:16],
       "params", hashlib.sha1(e.get_params_flat().tobytes()).hexdigest()[:16])
 # accuracy of every stored inverse against numpy fp64 on the engine's own running sums and dampings
@@ -56,12 +58,17 @@ for li, layer in enumerate(eng.LAYERS):
 print("inverse rel err vs fp64:", {k: "%.1e" % v for k, v in worst.items()})
 e.set_profiling(True)
 ts = []
+launches0 = _lib.launch_count()
 for u in range(6):
     e.update(b, fl, fe, fetch=False)
     torch.cuda.synchronize()
     ts.append(e.stage_ms()["inverse"])
 e.set_profiling(False)
+launches = (_lib.launch_count() - launches0) / 6
+n_fc4 = 49 * c3 + 1
+path = "fp64 chain" if launches > 3 * (n_fc4 // 32) else "resident fp32"
 print("inverse stage ms per refresh (serial, eager):", ["%.3f" % t for t in ts])
+print("launches per refreshing update %.0f: %s refresh" % (launches, path))
 # graph-replayed whole update with refresh
 ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 with torch.cuda.stream(e.stream):

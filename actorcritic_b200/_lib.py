@@ -82,6 +82,12 @@ class MLPConfig(ctypes.Structure):
                 ("use_graphs", ctypes.c_int), ("seed", ctypes.c_uint64)]
 
 
+class CNNConfig(ctypes.Structure):
+    _fields_ = [("mlp", MLPConfig), ("obs_hw", ctypes.c_int), ("obs_channels", ctypes.c_int), ("obs_u8", ctypes.c_int),
+                ("num_conv", ctypes.c_int), ("filters", ctypes.c_int * 3), ("kernel", ctypes.c_int * 3),
+                ("stride", ctypes.c_int * 3)]
+
+
 # every symbol include/acx.h declares: name -> (restype, argtypes)
 _P = ctypes.c_void_p
 SIGNATURES = {
@@ -162,6 +168,9 @@ SIGNATURES = {
                                          ctypes.POINTER(ctypes.c_int)]),
     "acx_mlp_global_step": (ctypes.c_int64, [_P]),
     "acx_mlp_act": (ctypes.c_int, [_P, _P, ctypes.c_int, _P, ctypes.c_int, _P, _P, _P, _P]),
+    "acx_cnn_arena_bytes": (ctypes.c_size_t, [ctypes.POINTER(CNNConfig)]),
+    "acx_cnn_create": (_P, [ctypes.POINTER(CNNConfig), _P, ctypes.c_size_t]),
+    "acx_cnn_act": (ctypes.c_int, [_P, _P, ctypes.c_int, _P, ctypes.c_int, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -107,10 +107,39 @@ __global__ void __launch_bounds__(256) im2col_bf16_kernel(const Planes pin, cons
   }
 }
 
+// observation im2col for any NHWC geometry: obs [rows / (hw_out^2), hw_in, hw_in, c] (uint8 or fp32) -> patch planes
+// [rows, ld] in the order (ky, kx, c), columns k*k*c .. ld-1 zero.  uint8 observations are written as their raw byte
+// values on one plane (exact in bf16; the caller folds the 1/255 into its GEMM alpha and factor scales), fp32 observations
+// as the hi / mid (/ lo) split over the output's planes.  One thread per output element (grid-stride).
+template <typename T>
+__global__ void __launch_bounds__(256) im2col_obs_kernel(const T* __restrict__ obs, const Planes out, long long rows, int hw_in,
+                                                         int c, int k, int s, int hw_out) {
+  pdl_enter();
+  const int kc = k * c, kkc = k * kc, per = hw_out * hw_out;
+  const long long total = rows * out.ld;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long row = i / out.ld;
+    const int col = (int)(i - row * out.ld);
+    float v = 0.0f;
+    if (col < kkc) {
+      const long long n = row / per;
+      const int loc = (int)(row - n * per), oy = loc / hw_out, ox = loc - oy * hw_out;
+      const int ky = col / kc, rem = col - ky * kc, kx = rem / c, ci = rem - kx * c;
+      v = (float)__ldg(obs + ((size_t)(n * hw_in + oy * s + ky) * hw_in + ox * s + kx) * c + ci);
+    }
+    bf16 hi, mid, lo;
+    split3(v, hi, mid, lo);
+    out.p[0][i] = hi;
+    if (out.n > 1) out.p[1][i] = mid;
+    if (out.n > 2) out.p[2][i] = lo;
+  }
+}
+
 // col2im (adjoint of im2col) as a gather + ReLU mask + bf16 split:
 //   dX[n,y,x,c] = sum_{ky,kx : (y-ky)%s==0, (x-kx)%s==0, in range} dP[(n,oy,ox), (ky,kx,c)]
 //   dPre[n,y,x,c] = dX * 1[act(n % mask_n, y, x, c) > 0]       (true rows and Fisher rows share the mask)
-// One CTA per (sample, input row y); a thread owns (x, 4 channels), so the only integer division is per CTA.
+// blockIdx.x = (sample, input row y); a thread owns (x, 4 channels), so the only integer division is per CTA.  A row of more
+// than 256 such threads is spread over gridDim.y CTAs; every element is summed in the same order either way.
 __global__ void __launch_bounds__(256) col2im_mask_split_kernel(const float* __restrict__ dp, const bf16* __restrict__ act_hi,
                                                                 const Planes out, int n_begin, int mask_n, int hw_in, int c, int k,
                                                                 int s, int hw_out) {
@@ -118,7 +147,8 @@ __global__ void __launch_bounds__(256) col2im_mask_split_kernel(const float* __r
   // the global sample number
   const int cv = c >> 2;
   const int n = blockIdx.x / hw_in, y = blockIdx.x - n * hw_in;
-  const int x = threadIdx.x / cv, c4 = (threadIdx.x - x * cv) << 2;
+  const int t = blockIdx.y * blockDim.x + threadIdx.x;
+  const int x = t / cv, c4 = (t - x * cv) << 2;
   if (x >= hw_in) return;
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
   const int kkc = k * k * c;
@@ -746,10 +776,25 @@ int im2col_bf16(const Planes& in, const Planes& out, int rows_total, int hw_in, 
 }
 int col2im_mask_split(const float* dp, const bf16* act_hi, const Planes& out, int n_begin, int n_total, int mask_n, int hw_in, int c,
                       int k, int s, int hw_out, cudaStream_t st) {
-  const int threads = (hw_in * (c / 4) + 31) / 32 * 32;
-  ACX_CHECK(threads <= 256 && (c & 3) == 0, "col2im: row does not fit one CTA");
-  col2im_mask_split_kernel<<<n_total * hw_in, threads, 0, st>>>(dp, act_hi, out, n_begin, mask_n, hw_in, c, k, s, hw_out);
+  ACX_CHECK((c & 3) == 0, "col2im: channels must be a multiple of 4");
+  const int row_threads = hw_in * (c / 4);
+  const int threads = row_threads <= 256 ? (row_threads + 31) / 32 * 32 : 256;
+  const dim3 grid(n_total * hw_in, ceil_div(row_threads, threads));
+  col2im_mask_split_kernel<<<grid, threads, 0, st>>>(dp, act_hi, out, n_begin, mask_n, hw_in, c, k, s, hw_out);
   ACX_LAUNCH_CHECK();
+  return 0;
+}
+int im2col_obs(const void* obs, int obs_u8, const Planes& out, long long rows, int hw_in, int c, int k, int s, int hw_out,
+               cudaStream_t st) {
+  ACX_CHECK(out.ld >= k * k * c && (out.ld & 7) == 0, "im2col_obs: ld must be a multiple of 8 covering k*k*c");
+  long long blocks = (rows * out.ld + 255) / 256;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  if (obs_u8)
+    ACX_PDL_LAUNCH(im2col_obs_kernel<uint8_t>, (unsigned)blocks, 256, 0, st, static_cast<const uint8_t*>(obs), out, rows, hw_in, c,
+                   k, s, hw_out);
+  else
+    ACX_PDL_LAUNCH(im2col_obs_kernel<float>, (unsigned)blocks, 256, 0, st, static_cast<const float*>(obs), out, rows, hw_in, c, k,
+                   s, hw_out);
   return 0;
 }
 int heads_fwd(const Planes& act4, const float* vpol, const float* vval, int rows, int num_actions, float* logits, float* values,

@@ -30,6 +30,9 @@ int im2col_conv1(const uint8_t* obs, bf16* out, int rows_total, cudaStream_t st)
 int im2col_bf16(const Planes& in, const Planes& out, int rows_total, int hw_in, int c, int k, int s, int hw_out, cudaStream_t st);
 int col2im_mask_split(const float* dp, const bf16* act_hi, const Planes& out, int n_begin, int n_total, int mask_n, int hw_in, int c,
                       int k, int s, int hw_out, cudaStream_t st);
+// im2col of uint8 (obs_u8) or fp32 NHWC observations of any geometry -> bf16 patch planes [rows, out.ld] (see layers.cu)
+int im2col_obs(const void* obs, int obs_u8, const Planes& out, long long rows, int hw_in, int c, int k, int s, int hw_out,
+               cudaStream_t st);
 int heads_fwd(const Planes& act4, const float* vpol, const float* vval, int rows, int num_actions, float* logits, float* values,
               cudaStream_t st);
 int loss_grad(const float* logits, const float* values, const uint8_t* actions, const float* targets, const int32_t* fl,

@@ -854,3 +854,78 @@ class MLPEngine(_ArenaEngine):
         with self.on_stream():
             _lib.check(self.lib.acx_mlp_update(self._h, fl, fe, self._stream()))
         return self._fetched(fetch)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# convolutional models on square images (CNNModel, include/acx.h `acx_cnn_*`: the fully connected learner with a conv trunk)
+# ---------------------------------------------------------------------------------------------------------------------
+def cnn_layers(num_conv, num_hidden):
+    """Block names in the order of the flat parameter vector: conv1 .. convK, fc(K+1) .. fc(K+L), the heads."""
+    return (tuple("conv%d" % (i + 1) for i in range(num_conv)) + tuple("fc%d" % (num_conv + i + 1) for i in range(num_hidden))
+            + ("fc_policy", "fc_baseline"))
+
+
+def cnn_conv_geometry(obs_hw, obs_channels, conv_layers):
+    """[(hw_in, c_in, filters, kernel, stride, hw_out)] per conv layer (VALID)."""
+    out, hw, c = [], int(obs_hw), int(obs_channels)
+    for f, k, s in conv_layers:
+        o = (hw - int(k)) // int(s) + 1
+        out.append((hw, c, int(f), int(k), int(s), o))
+        hw, c = o, int(f)
+    return out
+
+
+def cnn_param_shapes(obs_hw, obs_channels, conv_layers, hidden_sizes, num_actions):
+    """nn.conv2d_params (HWIO [k, k, c_in, filters]) for the conv layers, nn.fully_connected_params ([in, out]) after them."""
+    geo = cnn_conv_geometry(obs_hw, obs_channels, conv_layers)
+    names = cnn_layers(len(geo), len(hidden_sizes))
+    shapes = {}
+    for name, (_, c, f, k, _, _) in zip(names, geo):
+        shapes[name + "/weights"], shapes[name + "/bias"] = (k, k, c, f), (f,)
+    hw, c = geo[-1][5], geo[-1][2]
+    ins = [hw * hw * c] + [int(h) for h in hidden_sizes]
+    outs = [int(h) for h in hidden_sizes] + [int(num_actions), 1]
+    ins.append(ins[-1])
+    for name, k, c in zip(names[len(geo):], ins, outs):
+        shapes[name + "/weights"], shapes[name + "/bias"] = (k, c), (c,)
+    return shapes
+
+
+@dataclasses.dataclass
+class CNNEngineConfig(MLPEngineConfig):
+    obs_hw: int = 84
+    obs_channels: int = 4
+    obs_u8: bool = True
+    conv_layers: tuple = ((32, 8, 4), (64, 4, 2), (64, 3, 1))   # (filters, kernel, stride) per layer, VALID
+    hidden_sizes: tuple = (512,)
+    obs_dim: int = None                                          # derived: obs_hw * obs_hw * obs_channels
+
+    def to_c(self):
+        if not 1 <= len(self.conv_layers) <= 3:
+            raise ValueError("1 to 3 conv layers")
+        c = _lib.CNNConfig()
+        c.mlp = MLPEngineConfig.to_c(dataclasses.replace(self, obs_dim=self.obs_hw * self.obs_hw * self.obs_channels))
+        c.obs_hw, c.obs_channels, c.obs_u8, c.num_conv = self.obs_hw, self.obs_channels, int(bool(self.obs_u8)), len(self.conv_layers)
+        for i, (f, k, s) in enumerate(self.conv_layers):
+            c.filters[i], c.kernel[i], c.stride[i] = int(f), int(k), int(s)
+        return c
+
+
+class CNNEngine(MLPEngine):
+    """Learner of a convolutional actor-critic model on square images [rows, H, H, C] (uint8 or float32 as configured):
+    acx_cnn_create / acx_cnn_act, and every other call of the fully connected learner (acx_mlp_*) on the same handle."""
+
+    _CNN_CALLS = ("arena_bytes", "create", "act")
+
+    def __init__(self, config, device=None):
+        self._OBS_DTYPE = torch.uint8 if config.obs_u8 else torch.float32
+        self._open(config, device, (config.obs_hw, config.obs_hw, config.obs_channels))
+        self.layers = cnn_layers(len(config.conv_layers), len(config.hidden_sizes))
+        self._shapes = cnn_param_shapes(config.obs_hw, config.obs_channels, config.conv_layers, config.hidden_sizes,
+                                        config.num_actions)
+
+    def _fn(self, name):
+        return getattr(self.lib, ("acx_cnn_" if name in self._CNN_CALLS else "acx_mlp_") + name)
+
+    def _layer_cols(self, layer):
+        return self._shapes[layer + "/bias"][0]

@@ -10,6 +10,9 @@ train step runs in libacx's fully connected learner (acx_mlp_*), created on the 
 [environments, steps] batch shape is known; `A2CObjective(model).optimize_shared(...)` with nn.ClipGlobalNormOptimizer
 (RMSProp) or kfac.KfacOptimizer / kfac_utils.ColdStartPeriodicInvUpdateKfacOpt drives it through `Session.run` as for
 AtariModel.
+
+CNNModel (cnn.py) is this model with a convolutional trunk in front: it overrides the hooks below (observation checks,
+layers and their initial values, K-FAC registration, engine config and class).
 """
 import numpy as np
 import torch
@@ -26,31 +29,23 @@ MAX_OBS_DIM = 2048
 
 
 class MLPModel(ActorCriticModel):
+    _ENGINE = eng.MLPEngine
+
     def __init__(self, observation_space, action_space, hidden_sizes=(64, 64), random_seed=None, name=None):
         super().__init__(observation_space, action_space)
-        if not spaces.is_box(observation_space) or np.dtype(observation_space.low.dtype) != np.float32:
-            raise TypeError("MLPModel needs a float32 Box observation space, got %r" % (observation_space,))
+        self._check_observation_space(observation_space)
         if not spaces.is_discrete(action_space):
             raise TypeError("Unsupported space")
-        self.obs_shape = tuple(int(d) for d in observation_space.shape)
-        self.obs_dim = int(np.prod(self.obs_shape))
-        if not 1 <= self.obs_dim <= MAX_OBS_DIM:
-            raise ValueError("observations must have 1 to %d features, got %d" % (MAX_OBS_DIM, self.obs_dim))
         self.num_actions = int(action_space.n)
         if not 1 <= self.num_actions <= 31:
-            raise ValueError("MLPModel supports 1 to 31 actions, got %d" % self.num_actions)
+            raise ValueError("%s supports 1 to 31 actions, got %d" % (type(self).__name__, self.num_actions))
         self.hidden_sizes = tuple(int(h) for h in hidden_sizes)
         if not 1 <= len(self.hidden_sizes) <= 4 or any(h < 8 or h > 1024 or h % 8 for h in self.hidden_sizes):
             raise ValueError("hidden_sizes: 1 to 4 widths, each a multiple of 8 in [8, 1024], got %s" % (hidden_sizes,))
+        self._check_trunk()
         self.random_seed = random_seed
-        self.layers = eng.mlp_layers(len(self.hidden_sizes))
-        shapes = eng.mlp_param_shapes(self.obs_dim, self.hidden_sizes, self.num_actions)
-        rng = np.random.default_rng(random_seed)
-        gains = {"fc_policy": 0.01, "fc_baseline": 1.0}
-        self._params = {}
-        for layer in self.layers:
-            w, b = nn.fully_connected_params(*shapes[layer + "/weights"], rng=rng, gain=gains.get(layer, 2.0 ** 0.5))
-            self._params[layer + "/weights"], self._params[layer + "/bias"] = w, b
+        self.layers = self._layer_names()
+        self._params = self._initial_params(np.random.default_rng(random_seed))
         self._policy = SoftmaxPolicy(self, self.num_actions)
         self._baseline = StateValueFunction(self)
         self._bootstrap_values = Fetch("bootstrap_values", self, "bootstrap_values")
@@ -61,6 +56,36 @@ class MLPModel(ActorCriticModel):
         # the two heads are registered with the SAME inputs tensor (as envs/atari/model.py:243,246) -> one shared factor
         self._layer_tokens["fc_baseline"] = (self._layer_tokens["fc_policy"][0], self._layer_tokens["fc_baseline"][1])
         self.engine_options = {}     # extra MLPEngineConfig fields (seed, use_graphs ...)
+
+    # ------------------------------------------------------------------ what a subclass with another trunk overrides
+    def _check_observation_space(self, observation_space):
+        if not spaces.is_box(observation_space) or np.dtype(observation_space.low.dtype) != np.float32:
+            raise TypeError("MLPModel needs a float32 Box observation space, got %r" % (observation_space,))
+        self.obs_shape = tuple(int(d) for d in observation_space.shape)
+        self.obs_dim = int(np.prod(self.obs_shape))
+        if not 1 <= self.obs_dim <= MAX_OBS_DIM:
+            raise ValueError("observations must have 1 to %d features, got %d" % (MAX_OBS_DIM, self.obs_dim))
+        self._engine_obs_shape = (self.obs_dim,)     # one observation as the engine's "observations" buffer holds it
+        self._obs_dtype = np.float32
+
+    def _check_trunk(self):
+        pass
+
+    def _layer_names(self):
+        return eng.mlp_layers(len(self.hidden_sizes))
+
+    def _initial_params(self, rng):
+        """Orthogonal weights, gains sqrt(2) (trunk), 0.01 (policy), 1.0 (value); zero biases."""
+        shapes = eng.mlp_param_shapes(self.obs_dim, self.hidden_sizes, self.num_actions)
+        gains = {"fc_policy": 0.01, "fc_baseline": 1.0}
+        params = {}
+        for layer in self.layers:
+            w, b = nn.fully_connected_params(*shapes[layer + "/weights"], rng=rng, gain=gains.get(layer, 2.0 ** 0.5))
+            params[layer + "/weights"], params[layer + "/bias"] = w, b
+        return params
+
+    def _engine_config(self, **kw):
+        return eng.MLPEngineConfig(obs_dim=self.obs_dim, hidden_sizes=self.hidden_sizes, **kw)
 
     # ------------------------------------------------------------------ K-FAC registration
     def register_layers(self, layer_collection):
@@ -92,12 +117,13 @@ class MLPModel(ActorCriticModel):
     def _build_engine(self, session, num_envs, num_steps, objective):
         if session.group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()
                                          and torch.distributed.get_world_size() > 1):
-            raise NotImplementedError("MLPModel trains on one GPU: data-parallel learners are not implemented for it")
-        kw = dict(num_envs=num_envs, num_steps=num_steps, obs_dim=self.obs_dim, hidden_sizes=self.hidden_sizes,
-                  num_actions=self.num_actions)
+            raise NotImplementedError("%s trains on one GPU: data-parallel learners are not implemented for it"
+                                      % type(self).__name__)
+        kw = dict(num_envs=num_envs, num_steps=num_steps, num_actions=self.num_actions)
         if objective is not None:
             if getattr(objective, "_separate", None) is not None:
-                raise NotImplementedError("optimize_separate is not implemented for MLPModel: use optimize_shared")
+                raise NotImplementedError("optimize_separate is not implemented for %s: use optimize_shared"
+                                          % type(self).__name__)
             kw.update(gamma=objective.discount_factor, entropy_beta=objective.entropy_regularization_strength,
                       value_loss_weight=objective._baseline_loss_weight)
             kw.update(objective._optimizer.engine_overrides())
@@ -107,11 +133,11 @@ class MLPModel(ActorCriticModel):
             base = self.random_seed if self.random_seed is not None else int.from_bytes(__import__("os").urandom(4), "little")
             kw["seed"] = (int(base) * 1000003) & 0x7FFFFFFFFFFFFFFF
         kw.update(self.engine_options)
-        cfg = eng.MLPEngineConfig(**kw)
+        cfg = self._engine_config(**kw)
         old = self._engine
         if old is not None:
             self._params = old.get_params()
-        e = eng.MLPEngine(cfg, session.device)
+        e = self._ENGINE(cfg, session.device)
         e.set_params(self._params)
         if old is not None and old.config.acktr == cfg.acktr:
             e.load_state_dict(old.state_dict())      # the learner state does not depend on the batch shape
@@ -147,9 +173,9 @@ class MLPModel(ActorCriticModel):
             if not isinstance(v, torch.Tensor):
                 v = np.asarray(v, dtype=ph.dtype if ph.dtype != np.bool_ else np.bool_)
             if name == "observations":
-                v = v.reshape(e, t, self.obs_dim)
+                v = v.reshape((e, t) + self._engine_obs_shape)
             elif name == "bootstrap_observations":
-                v = v.reshape(e, self.obs_dim)
+                v = v.reshape((e,) + self._engine_obs_shape)
             out.append(v)
         return out
 
@@ -158,9 +184,9 @@ class MLPModel(ActorCriticModel):
         if obs is None:
             raise ValueError("observations_placeholder must be fed")
         if not isinstance(obs, torch.Tensor):
-            obs = torch.from_numpy(np.ascontiguousarray(np.asarray(obs, np.float32)))
+            obs = torch.from_numpy(np.ascontiguousarray(np.asarray(obs, self._obs_dtype)))
         lead = tuple(obs.shape[:obs.dim() - len(self.obs_shape)])
-        flat = obs.reshape(-1, self.obs_dim)
+        flat = obs.reshape((-1,) + self._engine_obs_shape)
         e = self._engine
         if e is None:
             e = self._build_engine(session, flat.shape[0], 1, None)

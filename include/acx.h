@@ -410,6 +410,31 @@ int64_t acx_mlp_global_step(const acx_mlp_t* l);
 int acx_mlp_act(acx_mlp_t* l, const float* d_obs, int rows, const float* d_uniform, int greedy, int32_t* d_actions,
                 float* d_logits, float* d_values, void* stream);
 
+/* ---- convolutional learner (one process per GPU) ---------------------------------------------- */
+/* The fully connected learner above with a trunk of 1..3 conv layers in front of its fully connected layers, for square
+ * NHWC image observations [H, H, C]: conv1 .. convK (VALID, stride s, ReLU; HWIO weights, nn.py:55-110), the (h, w, c) flatten
+ * of nn.flatten, then fc(K+1) .. fc(K+L) and the heads as acx_mlp_*.  One K-FAC conv block per conv layer
+ * (register_conv2d: factors over every output location, damping lambda / T and the preconditioned block / T with T = oh * ow
+ * true locations, as the Atari learner).  uint8 observations are scaled by 1/255 (envs/atari/model.py:93), fp32 ones are used
+ * as given.  The handle is an acx_mlp_t: every acx_mlp_* call other than acx_mlp_act accepts it; acting goes through
+ * acx_cnn_act.  Its buffers are those of acx_mlp_buffer ("observations": uint8 or f32 [N+E, H, H, C]) and per conv layer
+ * "act_hi/conv<i>" [(N+E) * oh * ow, filters] (the ReLU masks). */
+typedef struct {
+  acx_mlp_config_t mlp;        /* num_hidden / hidden[]: the fully connected layers after the trunk; obs_dim is derived */
+  int obs_hw, obs_channels;    /* H in [4, 128], C in [1, 16] */
+  int obs_u8;                  /* 1: uint8 observations, 0: fp32 */
+  int num_conv;                /* 1..3, and num_conv + mlp.num_hidden <= 4 */
+  int filters[3];              /* multiples of 8 in [8, 128] */
+  int kernel[3];               /* in [1, 8]; kernel^2 * input channels + 1 <= 3137 */
+  int stride[3];               /* in [1, min(kernel, 4)]; every output at least 1 x 1, flattened output + 1 <= 3137 */
+} acx_cnn_config_t;
+
+size_t acx_cnn_arena_bytes(const acx_cnn_config_t* cfg);
+acx_mlp_t* acx_cnn_create(const acx_cnn_config_t* cfg, void* d_arena, size_t arena_bytes);
+/* acx_mlp_act for this learner: d_obs uint8 or f32 (as configured) [rows, H, H, C] */
+int acx_cnn_act(acx_mlp_t* l, const void* d_obs, int rows, const float* d_uniform, int greedy, int32_t* d_actions,
+                float* d_logits, float* d_values, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

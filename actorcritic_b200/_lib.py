@@ -99,6 +99,10 @@ SIGNATURES = {
     "acx_preprocess_reset_u8": (ctypes.c_int, [_P, _P, ctypes.c_size_t, ctypes.c_int, _P]),
     "acx_frame_max_u8": (ctypes.c_int, [_P, _P, _P, ctypes.c_size_t, _P]),
     "acx_framestack_push_u8": (ctypes.c_int, [_P, _P, _P, _P, ctypes.c_int, _P]),
+    "acx_preprocess_stack_sq_u8": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
+                                                  ctypes.c_int, _P]),
+    "acx_preprocess_reset_sq_u8": (ctypes.c_int, [_P, _P, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_int, _P]),
+    "acx_framestack_push_sq_u8": (ctypes.c_int, [_P, _P, _P, _P, ctypes.c_int, ctypes.c_int, ctypes.c_int, _P]),
     "acx_returns_adv": (ctypes.c_int, [_P, _P, _P, _P, ctypes.c_float, ctypes.c_int, ctypes.c_int, _P, _P, _P]),
     "acx_gemm": (ctypes.c_int, [ctypes.POINTER(Gemm), ctypes.c_int, _P]),
     "acx_gemm_workspace_bytes": (ctypes.c_size_t, [ctypes.POINTER(Gemm)]),

@@ -2,10 +2,13 @@
 (observations, actions, rewards, terminals, next_observations, infos) in batch-major [environment][step] order
 (agents.py:26-45,157-228) - for any `MultiEnv`.  When the environment is device resident
 (envs.atari.device_env.DeviceAtariMultiEnv) the rollout stays on the GPU: K-PRE writes each step's frame stacks
-straight into a [E,T,84,84,4] rollout buffer and the tuple holds torch tensors instead of nested lists (the
-replacement for the reference's Python list shuffling, SURVEY 8(a) a4)."""
+straight into a [E,T,*observation_shape] rollout buffer (sized from the environment's observation space: [E,T,84,84,4]
+for AtariModel, [E,T,S,S,k] for a CNNModel on other frames) and the tuple holds torch tensors instead of nested lists
+(the replacement for the reference's Python list shuffling, SURVEY 8(a) a4).  The acting engine is the model's own
+(`_build_engine`), so any model with an engine (AtariModel, CNNModel) rolls out this way."""
 from abc import ABCMeta, abstractmethod
 
+import numpy as np
 import torch
 
 
@@ -57,7 +60,7 @@ class MultiEnvAgent(Agent):
         if engine is None:
             engine = self._model._build_engine(session, env.num_envs, t_count, None)
         if self._observations is None:
-            self._observations = env.reset()                                       # uint8 [E,84,84,4] on the device
+            self._observations = env.reset()                                       # uint8 [E,S,S,k] on the device
         # A device environment whose rollouts of this length always touch the same buffers (rollout_repeats) is replayed as
         # ONE CUDA graph: T x (K-PRE, acting forward, sample, bookkeeping copies) = ~14 T launches become one.  The first
         # rollout runs eagerly (one-time host work of the library), the second is captured, later ones are replayed.
@@ -69,10 +72,13 @@ class MultiEnvAgent(Agent):
     def _rollout_buffers(self, engine):
         env, t_count = self._env, self._num_steps
         e_count, dev = env.num_envs, env.device
+        space = env.observation_space
+        obs_shape = tuple(int(d) for d in space.shape)
+        obs_dtype = torch.from_numpy(np.zeros(0, space.low.dtype)).dtype
         if getattr(self, "_step_actions", None) is None or self._step_actions.shape != (t_count, e_count):
             self._step_actions = torch.empty((t_count, e_count), dtype=torch.int32, device=dev)
-            self._obs_buf = torch.empty((e_count, t_count, 84, 84, 4), dtype=torch.uint8, device=dev)
-            self._next_obs_buf = torch.empty((e_count, 84, 84, 4), dtype=torch.uint8, device=dev)
+            self._obs_buf = torch.empty((e_count, t_count) + obs_shape, dtype=obs_dtype, device=dev)
+            self._next_obs_buf = torch.empty((e_count,) + obs_shape, dtype=obs_dtype, device=dev)
             self._act_buf = torch.empty((e_count, t_count), dtype=torch.uint8, device=dev)
             self._rew_buf = torch.empty((e_count, t_count), dtype=torch.float32, device=dev)
             self._term_buf = torch.empty((e_count, t_count), dtype=torch.uint8, device=dev)

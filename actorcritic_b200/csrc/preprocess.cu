@@ -18,6 +18,19 @@
 // 16-byte loads (a 480-byte row = 30 uint4), takes the max, converts to gray, and leaves the gray band
 // in shared memory as bytes.  Phase 2: a thread owns an output column and 10 source rows: horizontal taps into
 // registers, vertical taps of its 4 output rows, round + stack push with coalesced 32-bit stores.
+//
+// The end of the file holds the same work at any square output size S in [4, 128] and stack depth k in [1, 16]
+// (preprocess_sq_kernel, framestack_sq_kernel; acx_*_sq_u8) for observations other than 84x84x4: tap tables of any
+// length (CSR arrays, built once per size and device), a band of output rows per CTA whose raw rows are read once, the
+// horizontal pass in shared memory, stacks [E,S,S,k] written with coalesced stores over the k bytes of each pixel.  At S
+// = 5 and 10, where both scales are integers, cv2 averages blocks in integers instead (resizeAreaFast_); the kernel does
+// the same.  84x84x4 keeps running through the K-PRE kernels above.
+#include <algorithm>
+#include <cfloat>
+#include <map>
+#include <mutex>
+#include <vector>
+
 #include "tc.cuh"
 
 namespace acx {
@@ -486,6 +499,281 @@ __global__ void __launch_bounds__(256) framestack_kernel(const uint8_t* __restri
   }
 }
 
+// ---- K-PRE at any square size S in [4, 128] and stack depth k in [1, 16] ----------------------------------------------
+// The same per-environment work as K-PRE (max, gray, INTER_AREA to S x S, stack push / zero / reset) with variable-length
+// tap tables: the tap counts reach 16 (x) and 20 (y) at S = 11, so K-PRE's fixed 3-tap tables and its 2.5 row pattern do
+// not carry over.  Stacks are uint8 [E, S, S, k], the k frames of a pixel contiguous.
+constexpr int SQ_MIN_SIZE = 4, SQ_MAX_SIZE = 128, SQ_MAX_FRAMES = 16;
+constexpr int SQ_THREADS = 256;
+constexpr int SQ_BAND_SRC = 32;   // a band of output rows spans about this many source rows (K-PRE: 30)
+
+// OpenCV's computeResizeAreaTab (resize.cpp) for one axis, cn = 1, packed CSR-style: the taps of output d are
+// [off[d], off[d + 1]), in table order (build_axis above without the 3-tap bound)
+static void area_axis(int ssize, int dsize, std::vector<int>& off, std::vector<int>& src, std::vector<float>& w) {
+  const double scale = (double)ssize / dsize;
+  off.assign(1, 0);
+  src.clear();
+  w.clear();
+  for (int d = 0; d < dsize; ++d) {
+    const double fsx1 = d * scale, fsx2 = fsx1 + scale;
+    const double cell = scale < (ssize - fsx1) ? scale : (ssize - fsx1);
+    int sx1 = (int)ceil(fsx1), sx2 = (int)floor(fsx2);
+    if (sx2 > ssize - 1) sx2 = ssize - 1;
+    if (sx1 > sx2) sx1 = sx2;
+    if (sx1 - fsx1 > 1e-3) {
+      src.push_back(sx1 - 1);
+      w.push_back((float)((sx1 - fsx1) / cell));
+    }
+    for (int sx = sx1; sx < sx2; ++sx) {
+      src.push_back(sx);
+      w.push_back((float)(1.0 / cell));
+    }
+    if (fsx2 - sx2 > 1e-3) {
+      double a = fsx2 - sx2;
+      if (a > 1.0) a = 1.0;
+      if (a > cell) a = cell;
+      src.push_back(sx2);
+      w.push_back((float)(a / cell));
+    }
+    off.push_back((int)src.size());
+  }
+}
+
+// the device tables of one output size (one allocation: xoff, xsrc, yoff, ysrc as int32, then xw, yw as fp32)
+struct SqTables {
+  const int* xoff;
+  const int* xsrc;
+  const int* yoff;
+  const int* ysrc;
+  const float* xw;
+  const float* yw;
+  float scale;        // 0, or 1 / block area at the sizes where cv2 takes its integer-scale path (see sq_tables)
+  int band_rows;      // output rows per CTA
+  int num_bands;
+  int max_src_rows;   // the most source rows one band spans
+};
+
+// shared memory of one CTA: gray rows [R][160] u8 | horizontal results [R][S] f32 | old stack bytes of the band
+// [rows][S][k] | the band's new plane [rows][S] | its reset plane [rows][S]
+static size_t sq_smem_bytes(const SqTables& t, int size, int frames) {
+  return (size_t)t.max_src_rows * RAW_W + (size_t)t.max_src_rows * size * 4 + (size_t)t.band_rows * size * (frames + 2);
+}
+
+// max + gray + INTER_AREA of one band of one frame (pair) into `plane` [rows][S]; every thread of the CTA calls it
+//   phase 1: 48 raw bytes (16 pixels) of each frame per thread with 16-byte loads -> byte-wise max -> 16 gray bytes in
+//            shared memory (each raw row is read once per CTA)
+//   phase 2: the horizontal taps of every (source row, output column) into shared fp32: buf = 0, buf = buf + src * w
+//   phase 3: the vertical taps of every output pixel of the band: first term assigned, the rest added; round half to
+//            even, saturate
+// Every multiply and add is a separate fp32 rounding (__fmul_rn / __fadd_rn are never contracted into an FMA), in
+// OpenCV's order, which is what makes the result bit-exact.
+__device__ __forceinline__ void sq_band_plane(const uint8_t* fa, const uint8_t* fb, bool single, int R, int y0, int d0,
+                                              int rows, int size, const SqTables& t, uint8_t* s_gray, float* s_h,
+                                              uint8_t* plane) {
+  const int tid = threadIdx.x;
+  const uint4* pa = reinterpret_cast<const uint4*>(fa + (size_t)y0 * RAW_ROW_BYTES);
+  const uint4* pb = reinterpret_cast<const uint4*>(fb + (size_t)y0 * RAW_ROW_BYTES);
+  for (int g = tid; g < R * (RAW_ROW_BYTES / 48); g += SQ_THREADS) {
+    const uint4 a0 = __ldg(pa + 3 * g), a1 = __ldg(pa + 3 * g + 1), a2 = __ldg(pa + 3 * g + 2);
+    uint4 b0 = a0, b1 = a1, b2 = a2;
+    if (!single) b0 = __ldg(pb + 3 * g), b1 = __ldg(pb + 3 * g + 1), b2 = __ldg(pb + 3 * g + 2);
+    *reinterpret_cast<uint4*>(s_gray + 16 * g) = gray_group(a0, a1, a2, b0, b1, b2, single);
+  }
+  __syncthreads();
+  for (int i = tid; i < R * size; i += SQ_THREADS) {
+    const int r = i / size, dx = i - r * size;
+    const uint8_t* row = s_gray + r * RAW_W;
+    const int t0 = __ldg(t.xoff + dx), t1 = __ldg(t.xoff + dx + 1);
+    float acc = __fmul_rn((float)row[__ldg(t.xsrc + t0)], __ldg(t.xw + t0));
+    for (int k = t0 + 1; k < t1; ++k) acc = __fadd_rn(acc, __fmul_rn((float)row[__ldg(t.xsrc + k)], __ldg(t.xw + k)));
+    s_h[i] = acc;
+  }
+  __syncthreads();
+  for (int i = tid; i < rows * size; i += SQ_THREADS) {
+    const int dl = i / size, dx = i - dl * size;
+    const int t0 = __ldg(t.yoff + d0 + dl), t1 = __ldg(t.yoff + d0 + dl + 1);
+    float sum = __fmul_rn(__ldg(t.yw + t0), s_h[(__ldg(t.ysrc + t0) - y0) * size + dx]);
+    for (int k = t0 + 1; k < t1; ++k) sum = __fadd_rn(sum, __fmul_rn(__ldg(t.yw + k), s_h[(__ldg(t.ysrc + k) - y0) * size + dx]));
+    if (t.scale != 0.0f) sum = __fmul_rn(sum, t.scale);   // integer-scale path: the exact block sum times 1 / area
+    int v = __float2int_rn(sum);  // cvRound
+    plane[i] = (uint8_t)(v < 0 ? 0 : (v > 255 ? 255 : v));
+  }
+}
+
+// One CTA per (environment, band of t.band_rows output rows), 256 threads.  The old stack bytes of the band are fetched
+// into shared memory first (cp.async, so the fetch overlaps the frame work; every byte of the band is read before any is
+// written, which makes the in-place update safe), then the frame pipeline runs - twice for an environment whose previous
+// step was terminal: first on the reset frame, whose plane only seeds the stack (k copies), then on the step frames.  The
+// new band [rows][S][k] is contiguous in the output and is written with coalesced 32-bit stores where it is aligned.
+template <bool RESET>
+__global__ void __launch_bounds__(SQ_THREADS, 4) preprocess_sq_kernel(const uint8_t* __restrict__ raw_a,
+                                                                   const uint8_t* __restrict__ raw_b,
+                                                                   const uint8_t* __restrict__ terminal,
+                                                                   const uint8_t* __restrict__ reset_mask,
+                                                                   const uint8_t* __restrict__ reset_raw,
+                                                                   const uint8_t* stack_in, uint8_t* stack_out,
+                                                                   size_t out_env_stride, int size, int frames,
+                                                                   SqTables t) {
+  extern __shared__ __align__(16) uint8_t sq_smem[];
+  const int env = blockIdx.x / t.num_bands, band = blockIdx.x - env * t.num_bands;
+  const int tid = threadIdx.x;
+  const int d0 = band * t.band_rows;
+  const int rows = min(size - d0, t.band_rows);
+  const int y0 = __ldg(t.ysrc + __ldg(t.yoff + d0));
+  const int R = __ldg(t.ysrc + __ldg(t.yoff + d0 + rows) - 1) + 1 - y0;
+  uint8_t* s_gray = sq_smem;
+  float* s_h = reinterpret_cast<float*>(sq_smem + t.max_src_rows * RAW_W);
+  uint8_t* s_old = sq_smem + t.max_src_rows * RAW_W + t.max_src_rows * size * 4;
+  uint8_t* s_plane = s_old + t.band_rows * size * frames;
+  uint8_t* s_rplane = s_plane + t.band_rows * size;
+
+  const bool do_reset = (!RESET) && (reset_mask != nullptr) && reset_mask[env] != 0;
+  const bool term = (!RESET) && (terminal != nullptr) && terminal[env] != 0;
+  const int band_bytes = rows * size * frames;
+  const size_t stack_bytes = (size_t)size * size * frames;
+  if (!RESET && !do_reset && !term && frames > 1) {
+    const uint8_t* sin = stack_in + (size_t)env * stack_bytes + (size_t)d0 * size * frames;
+    if ((((uintptr_t)sin | (uintptr_t)band_bytes) & 3) == 0) {
+      for (int i = 4 * tid; i < band_bytes; i += 4 * SQ_THREADS)
+        asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(s_old + i)), "l"(sin + i) : "memory");
+    } else {
+      for (int i = tid; i < band_bytes; i += SQ_THREADS) s_old[i] = sin[i];
+    }
+  }
+  const size_t frame_off = (size_t)env * RAW_FRAME_BYTES;
+  if (do_reset) {
+    sq_band_plane(reset_raw + frame_off, reset_raw + frame_off, true, R, y0, d0, rows, size, t, s_gray, s_h, s_rplane);
+    __syncthreads();   // the step pass overwrites s_gray and s_h
+  }
+  sq_band_plane(raw_a + frame_off, raw_b + frame_off, RESET, R, y0, d0, rows, size, t, s_gray, s_h, s_plane);
+  asm volatile("cp.async.wait_all;" ::: "memory");
+  __syncthreads();
+
+  // byte j of the band = frame c of pixel p: roll by -1 along the frames, zero on terminal, the new frame last
+  auto byte_at = [&](int j) -> uint32_t {
+    const int p = j / frames, c = j - p * frames;
+    if (RESET || c == frames - 1) return s_plane[p];
+    if (term) return 0u;
+    return do_reset ? s_rplane[p] : s_old[j + 1];
+  };
+  uint8_t* sout = stack_out + (size_t)env * out_env_stride + (size_t)d0 * size * frames;
+  int j0 = 0;
+  if (((uintptr_t)sout & 3) == 0) {
+    const int words = band_bytes >> 2;
+    for (int w = tid; w < words; w += SQ_THREADS)
+      reinterpret_cast<uint32_t*>(sout)[w] =
+          byte_at(4 * w) | (byte_at(4 * w + 1) << 8) | (byte_at(4 * w + 2) << 16) | (byte_at(4 * w + 3) << 24);
+    j0 = words << 2;
+  }
+  for (int j = j0 + tid; j < band_bytes; j += SQ_THREADS) sout[j] = (uint8_t)byte_at(j);
+}
+
+// FrameStackWrapper.step / reset on already preprocessed frames uint8 [E, S, S] for stacks uint8 [E, S, S, k]: one thread
+// per pixel, frames in ascending order (frame c + 1 is read before frame c is written, so in place is safe)
+__global__ void __launch_bounds__(256) framestack_sq_kernel(const uint8_t* __restrict__ frames, const uint8_t* __restrict__ mode,
+                                                            const uint8_t* stack_in, uint8_t* stack_out, int num_envs,
+                                                            int size, int k) {
+  const int per = size * size;
+  const size_t total = (size_t)num_envs * per;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+    const int env = (int)(i / per);
+    const uint8_t q = frames[i];
+    const int m = mode ? mode[env] : 0;
+    const uint8_t* in = stack_in + i * k;
+    uint8_t* out = stack_out + i * k;
+    for (int c = 0; c < k - 1; ++c) out[c] = m == 2 ? q : (m == 1 ? 0 : in[c + 1]);
+    out[k - 1] = q;
+  }
+}
+
+// The tap tables of one output size, built on the host once per (device, size) and kept for the life of the process.
+// The first call for a size uploads them (a synchronous copy): make it outside stream capture, as for K-PRE's tables.
+static int sq_tables(int size, SqTables* out) {
+  static std::mutex mu;
+  static std::map<std::pair<int, int>, SqTables> cache;
+  static std::map<int, size_t> smem_configured;   // per device: the dynamic shared memory both kernels are allowed
+  int dev = 0;
+  ACX_CUDA(cudaGetDevice(&dev));
+  std::lock_guard<std::mutex> lock(mu);
+  auto it = cache.find({dev, size});
+  if (it == cache.end()) {
+    std::vector<int> xoff, xsrc, yoff, ysrc;
+    std::vector<float> xw, yw;
+    area_axis(RAW_W, size, xoff, xsrc, xw);
+    area_axis(RAW_H, size, yoff, ysrc, yw);
+    // cv2.resize takes resizeAreaFast_ instead when both scales are integers to DBL_EPSILON (sizes 5 and 10 here):
+    // round(float(integer block sum) * (1.f / area)).  With unit weights the two passes add the block's bytes exactly in
+    // fp32 (at most 255 * 1344 < 2^24), and one multiply by 1 / area follows.
+    const double fx = 1.0 / ((double)size / RAW_W), fy = 1.0 / ((double)size / RAW_H);
+    const int ix = (int)lrint(fx), iy = (int)lrint(fy);
+    const bool fast = fabs(fx - ix) < DBL_EPSILON && fabs(fy - iy) < DBL_EPSILON;
+    if (fast) {
+      std::fill(xw.begin(), xw.end(), 1.0f);
+      std::fill(yw.begin(), yw.end(), 1.0f);
+    }
+    std::vector<int> ints;
+    ints.insert(ints.end(), xoff.begin(), xoff.end());
+    ints.insert(ints.end(), xsrc.begin(), xsrc.end());
+    ints.insert(ints.end(), yoff.begin(), yoff.end());
+    ints.insert(ints.end(), ysrc.begin(), ysrc.end());
+    std::vector<float> floats(xw);
+    floats.insert(floats.end(), yw.begin(), yw.end());
+    void* d = nullptr;
+    const size_t ibytes = ints.size() * sizeof(int), fbytes = floats.size() * sizeof(float);
+    ACX_CUDA(cudaMalloc(&d, ibytes + fbytes));
+    ACX_CUDA(cudaMemcpy(d, ints.data(), ibytes, cudaMemcpyHostToDevice));
+    ACX_CUDA(cudaMemcpy((char*)d + ibytes, floats.data(), fbytes, cudaMemcpyHostToDevice));
+    SqTables t;
+    const int* di = static_cast<const int*>(d);
+    t.xoff = di;
+    t.xsrc = t.xoff + xoff.size();
+    t.yoff = t.xsrc + xsrc.size();
+    t.ysrc = t.yoff + yoff.size();
+    t.xw = reinterpret_cast<const float*>((const char*)d + ibytes);
+    t.yw = t.xw + xw.size();
+    t.scale = fast ? 1.0f / (float)(ix * iy) : 0.0f;
+    int band_rows = SQ_BAND_SRC * size / RAW_H;
+    t.band_rows = band_rows < 1 ? 1 : band_rows;
+    t.num_bands = (size + t.band_rows - 1) / t.band_rows;
+    t.max_src_rows = 0;
+    for (int b = 0; b < t.num_bands; ++b) {
+      const int d0 = b * t.band_rows, d1 = std::min(size, d0 + t.band_rows);
+      t.max_src_rows = std::max(t.max_src_rows, ysrc[yoff[d1] - 1] + 1 - ysrc[yoff[d0]]);
+    }
+    it = cache.emplace(std::make_pair(dev, size), t).first;
+  }
+  // the attribute is raised once to the largest stack depth of each size met so far, outside any capture
+  const size_t need = sq_smem_bytes(it->second, size, SQ_MAX_FRAMES);
+  if (need > smem_configured[dev]) {
+    ACX_CUDA(cudaFuncSetAttribute(preprocess_sq_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+    ACX_CUDA(cudaFuncSetAttribute(preprocess_sq_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
+    smem_configured[dev] = need;
+  }
+  *out = it->second;
+  return 0;
+}
+
+static int check_sq_shape(int size, int frames) {
+  ACX_CHECK(size >= SQ_MIN_SIZE && size <= SQ_MAX_SIZE, "size must be in [4, 128], got " + std::to_string(size));
+  ACX_CHECK(frames >= 1 && frames <= SQ_MAX_FRAMES, "num_frames must be in [1, 16], got " + std::to_string(frames));
+  return 0;
+}
+
+template <bool RESET>
+static int launch_kpre_sq(const uint8_t* raw_a, const uint8_t* raw_b, const uint8_t* terminal, const uint8_t* reset_mask,
+                          const uint8_t* reset_raw, const uint8_t* stack_in, uint8_t* stack_out, size_t out_env_stride,
+                          int num_envs, int size, int frames, cudaStream_t st) {
+  SqTables t;
+  int r = sq_tables(size, &t);
+  if (r) return r;
+  const size_t grid = (size_t)num_envs * t.num_bands;
+  ACX_CHECK(grid < (1u << 31), "too many environments");
+  preprocess_sq_kernel<RESET><<<(unsigned)grid, SQ_THREADS, sq_smem_bytes(t, size, frames), st>>>(
+      raw_a, raw_b, terminal, reset_mask, reset_raw, stack_in, stack_out, out_env_stride, size, frames, t);
+  ACX_LAUNCH_CHECK();
+  return 0;
+}
+
 }  // namespace acx
 
 extern "C" {
@@ -547,5 +835,59 @@ int acx_preprocess_reset_u8(const uint8_t* d_raw, uint8_t* d_stack_out, size_t o
   if (r) return r;
   return launch_kpre<true>(d_raw, d_raw, nullptr, nullptr, nullptr, d_stack_out, d_stack_out, out_env_stride, num_envs,
                            reinterpret_cast<cudaStream_t>(stream));
+}
+}
+
+extern "C" {
+
+int acx_preprocess_stack_sq_u8(const uint8_t* d_raw_a, const uint8_t* d_raw_b, const uint8_t* d_terminal,
+                               const uint8_t* d_reset_mask, const uint8_t* d_reset_raw, const uint8_t* d_stack_in,
+                               uint8_t* d_stack_out, size_t out_env_stride, int num_envs, int size, int num_frames,
+                               void* stream) {
+  using namespace acx;
+  int r = check_sq_shape(size, num_frames);
+  if (r) return r;
+  ACX_CHECK(num_envs >= 0, "num_envs < 0");
+  if (num_envs == 0) return 0;
+  const size_t stack_bytes = (size_t)size * size * num_frames;
+  ACX_CHECK(d_raw_a && d_raw_b && d_stack_in && d_stack_out, "null pointer");
+  ACX_CHECK(out_env_stride >= stack_bytes, "out_env_stride below size * size * num_frames");
+  ACX_CHECK(d_stack_in != d_stack_out || out_env_stride == stack_bytes, "in place needs out_env_stride == size * size * num_frames");
+  ACX_CHECK(d_reset_mask == nullptr || d_reset_raw != nullptr, "reset_mask without reset_raw");
+  ACX_CHECK(((uintptr_t)d_raw_a % 16) == 0 && ((uintptr_t)d_raw_b % 16) == 0 &&
+                (d_reset_raw == nullptr || ((uintptr_t)d_reset_raw % 16) == 0),
+            "misaligned raw frames");
+  return launch_kpre_sq<false>(d_raw_a, d_raw_b, d_terminal, d_reset_mask, d_reset_raw, d_stack_in, d_stack_out,
+                               out_env_stride, num_envs, size, num_frames, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int acx_preprocess_reset_sq_u8(const uint8_t* d_raw, uint8_t* d_stack_out, size_t out_env_stride, int num_envs, int size,
+                               int num_frames, void* stream) {
+  using namespace acx;
+  int r = check_sq_shape(size, num_frames);
+  if (r) return r;
+  ACX_CHECK(num_envs >= 0, "num_envs < 0");
+  if (num_envs == 0) return 0;
+  ACX_CHECK(d_raw && d_stack_out, "null pointer");
+  ACX_CHECK(out_env_stride >= (size_t)size * size * num_frames, "out_env_stride below size * size * num_frames");
+  ACX_CHECK(((uintptr_t)d_raw % 16) == 0, "misaligned raw frames");
+  return launch_kpre_sq<true>(d_raw, d_raw, nullptr, nullptr, nullptr, nullptr, d_stack_out, out_env_stride, num_envs, size,
+                              num_frames, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int acx_framestack_push_sq_u8(const uint8_t* d_frames, const uint8_t* d_mode, const uint8_t* d_stack_in, uint8_t* d_stack_out,
+                              int num_envs, int size, int num_frames, void* stream) {
+  using namespace acx;
+  int r = check_sq_shape(size, num_frames);
+  if (r) return r;
+  ACX_CHECK(num_envs >= 0, "num_envs < 0");
+  if (num_envs == 0) return 0;
+  ACX_CHECK(d_frames && d_stack_in && d_stack_out, "null pointer");
+  size_t blocks = ((size_t)num_envs * size * size + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  framestack_sq_kernel<<<(unsigned)blocks, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      d_frames, d_mode, d_stack_in, d_stack_out, num_envs, size, num_frames);
+  ACX_LAUNCH_CHECK();
+  return 0;
 }
 }

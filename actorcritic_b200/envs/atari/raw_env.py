@@ -7,6 +7,8 @@ max of the last two frames, wrappers.py:52-67), `AtariPreprocessFrameWrapper` (c
 the learner process.  Here the environments only run the emulator part of that chain (action repeat, reward sum, early
 exit on terminal, auto-reset): each step leaves the last two raw frames of every environment in PINNED host buffers, one
 asynchronous copy moves them to the GPU, and one K-PRE launch does max + gray + resize + stack push for all of them.
+Observations are uint8 [E, S, S, k]: `size` S in [4, 128] (84 by default) and `num_stacked_frames` k in [1, 16] (4 by
+default); 84 x 84 x 4 runs K-PRE, any other pair its S x S form.
 Observations stay on the device (`device_resident`), so `MultiEnvAgent.interact` feeds them to acting and to the train
 step without another copy.
 
@@ -28,7 +30,7 @@ import numpy as np
 import torch
 
 from ... import spaces
-from .wrappers import BatchedAtariPreprocessor
+from .wrappers import BatchedAtariPreprocessor, check_frame_shape
 
 RAW_SHAPE = (210, 160, 3)
 
@@ -36,7 +38,9 @@ RAW_SHAPE = (210, 160, 3)
 class RawFrameMultiEnv:
     device_resident = True
 
-    def __init__(self, envs, frameskip=4, device=None, num_threads=None, clip_rewards=False, step_hook=None):
+    def __init__(self, envs, frameskip=4, device=None, num_threads=None, clip_rewards=False, step_hook=None, size=84,
+                 num_stacked_frames=4):
+        size, num_stacked_frames = check_frame_shape(size, num_stacked_frames)
         if len(envs) == 0:
             raise ValueError("at least one environment is required")
         if not torch.cuda.is_available():
@@ -51,7 +55,7 @@ class RawFrameMultiEnv:
         self.clip_rewards = bool(clip_rewards)
         self.step_hook = step_hook
         self.device = torch.device("cuda") if device is None else torch.device(device)
-        self.observation_space = spaces.Box(low=0, high=255, shape=(84, 84, 4), dtype=np.uint8)
+        self.observation_space = spaces.Box(low=0, high=255, shape=(size, size, num_stacked_frames), dtype=np.uint8)
         self.action_space = self._envs[0].action_space
         self._executor = concurrent.futures.ThreadPoolExecutor(num_threads or min(32, self.num_envs))
         e = self.num_envs
@@ -68,7 +72,7 @@ class RawFrameMultiEnv:
         self._d_rewards = torch.empty(e, dtype=torch.float32, device=self.device)
         self._terminated = [False] * e                  # _AutoResetWrapper._terminated (multi_env.py:124,131)
         self._staged = torch.cuda.Event()
-        self.pre = BatchedAtariPreprocessor(e, self.device)
+        self.pre = BatchedAtariPreprocessor(e, self.device, num_stacked_frames=num_stacked_frames, size=size)
         self.last_infos = [{} for _ in range(e)]
         self._closed = False
 
@@ -112,7 +116,7 @@ class RawFrameMultiEnv:
 
     # ------------------------------------------------------------------ MultiEnv surface
     def reset(self):
-        """MultiEnv.reset (multi_env.py:49-57): uint8 [E,84,84,4] on the device, 4 copies of the first frame."""
+        """MultiEnv.reset (multi_env.py:49-57): uint8 [E,S,S,k] on the device, k copies of the first frame."""
         self._wait_staging_free()
         list(self._executor.map(self._reset_one, range(self.num_envs)))
         self._d_frames[0].copy_(self._h_frames[0], non_blocking=True)
@@ -120,7 +124,7 @@ class RawFrameMultiEnv:
         return self.pre.reset(self._d_frames[0])
 
     def step_device(self, actions):
-        """actions: int tensor [E] (device or host) or a list.  Returns device tensors (observations uint8 [E,84,84,4],
+        """actions: int tensor [E] (device or host) or a list.  Returns device tensors (observations uint8 [E,S,S,k],
         rewards float32 [E], terminals uint8 [E]); `last_infos` holds the environments' info dicts."""
         if isinstance(actions, torch.Tensor):
             actions = actions.cpu().tolist()            # the emulators need the actions on the host: one small sync

@@ -77,6 +77,64 @@ def framestack_push(frames, stack_in, mode=None, out=None):
     return out
 
 
+def preprocess_stack_sq(raw_a, raw_b, stack_in, terminal=None, reset_mask=None, reset_raw=None, out=None,
+                        out_env_stride=None):
+    """K-PRE at any square size and stack depth (acx_preprocess_stack_sq_u8): the size S and depth k are read from
+    stack_in uint8 [E,S,S,k]; raw_*: uint8 [E,210,160,3].  `out` may be a slice of a batch-major rollout buffer
+    [E,T,S,S,k]; out_env_stride is then its env stride in bytes."""
+    _need_cuda(raw_a, raw_b, stack_in)
+    e = raw_a.shape[0]
+    assert raw_a.dtype == torch.uint8 and tuple(raw_a.shape[1:]) == (210, 160, 3) and raw_a.is_contiguous()
+    assert raw_b.shape == raw_a.shape and raw_b.is_contiguous()
+    assert stack_in.dtype == torch.uint8 and stack_in.dim() == 4 and stack_in.shape[0] == e and stack_in.is_contiguous()
+    size, k = stack_in.shape[1], stack_in.shape[3]
+    assert stack_in.shape[2] == size
+    if out is None:
+        out = torch.empty_like(stack_in)
+        out_env_stride = size * size * k
+    elif out_env_stride is None:
+        out_env_stride = out.stride(0)
+    for t in (terminal, reset_mask):
+        assert t is None or (t.dtype == torch.uint8 and t.is_contiguous())
+    assert reset_raw is None or (reset_raw.shape == raw_a.shape and reset_raw.is_contiguous())
+    _lib.check(_lib.load().acx_preprocess_stack_sq_u8(_ptr(raw_a), _ptr(raw_b), _ptr(terminal), _ptr(reset_mask),
+                                                      _ptr(reset_raw), _ptr(stack_in), _ptr(out),
+                                                      ctypes.c_size_t(out_env_stride), e, size, k, _stream()))
+    return out
+
+
+def preprocess_reset_sq(raw, size, num_frames, out=None, out_env_stride=None):
+    """acx_preprocess_reset_sq_u8: stacks uint8 [E,size,size,num_frames] = num_frames copies of preprocess(raw)."""
+    _need_cuda(raw)
+    e = raw.shape[0]
+    assert raw.dtype == torch.uint8 and tuple(raw.shape[1:]) == (210, 160, 3) and raw.is_contiguous()
+    if out is None:
+        out = torch.empty((e, size, size, num_frames), dtype=torch.uint8, device=raw.device)
+        out_env_stride = size * size * num_frames
+    elif out_env_stride is None:
+        out_env_stride = out.stride(0)
+    _lib.check(_lib.load().acx_preprocess_reset_sq_u8(_ptr(raw), _ptr(out), ctypes.c_size_t(out_env_stride), e, size,
+                                                      num_frames, _stream()))
+    return out
+
+
+def framestack_push_sq(frames, stack_in, mode=None, out=None):
+    """acx_framestack_push_sq_u8: frames uint8 [E,S,S(,1)], stacks uint8 [E,S,S,k]; mode uint8 [E]: 0 push, 1 push after a
+    terminal step, 2 reset (k copies)."""
+    _need_cuda(frames, stack_in)
+    assert stack_in.dtype == torch.uint8 and stack_in.dim() == 4 and stack_in.is_contiguous()
+    e, size, k = stack_in.shape[0], stack_in.shape[1], stack_in.shape[3]
+    assert stack_in.shape[2] == size
+    assert frames.dtype == torch.uint8 and frames.is_contiguous() and frames.numel() == e * size * size
+    assert mode is None or (mode.dtype == torch.uint8 and mode.is_contiguous() and mode.numel() == e)
+    if out is None:
+        out = torch.empty_like(stack_in)
+    assert out.shape == stack_in.shape and out.is_contiguous()
+    _lib.check(_lib.load().acx_framestack_push_sq_u8(_ptr(frames), _ptr(mode), _ptr(stack_in), _ptr(out), e, size, k,
+                                                     _stream()))
+    return out
+
+
 def returns_adv(rewards, terminals, values, bootstrap_values, gamma):
     """K-RET.  rewards f32 [E,T], terminals uint8/bool [E,T], values f32 [E,T], bootstrap f32 [E]."""
     _need_cuda(rewards, terminals, values, bootstrap_values)

@@ -67,6 +67,23 @@ int acx_frame_max_u8(const uint8_t* d_a, const uint8_t* d_b, uint8_t* d_out, siz
 int acx_framestack_push_u8(const uint8_t* d_frames, const uint8_t* d_mode, const uint8_t* d_stack_in, uint8_t* d_stack_out,
                            int num_envs, void* stream);
 
+/* K-PRE at any square output size and stack depth: the three calls above for stacks uint8 [E,size,size,num_frames]
+ * (the num_frames frames of a pixel contiguous), size in [4, 128], num_frames in [1, 16]; anything else returns an
+ * error.  The resize is cv2 INTER_AREA 210x160 -> size x size with OpenCV's tap tables (built once per size and
+ * device; the first call for a size uploads them synchronously, so make it outside stream capture).
+ * acx_preprocess_stack_sq_u8  as acx_preprocess_stack_u8; out_env_stride >= size*size*num_frames bytes, in place
+ *                             allowed when it equals size*size*num_frames.
+ * acx_preprocess_reset_sq_u8  stack = num_frames copies of preprocess(raw).
+ * acx_framestack_push_sq_u8   as acx_framestack_push_u8 on frames uint8 [E,size,size]; mode 2 = num_frames copies. */
+int acx_preprocess_stack_sq_u8(const uint8_t* d_raw_a, const uint8_t* d_raw_b, const uint8_t* d_terminal,
+                               const uint8_t* d_reset_mask, const uint8_t* d_reset_raw,
+                               const uint8_t* d_stack_in, uint8_t* d_stack_out, size_t out_env_stride,
+                               int num_envs, int size, int num_frames, void* stream);
+int acx_preprocess_reset_sq_u8(const uint8_t* d_raw, uint8_t* d_stack_out, size_t out_env_stride,
+                               int num_envs, int size, int num_frames, void* stream);
+int acx_framestack_push_sq_u8(const uint8_t* d_frames, const uint8_t* d_mode, const uint8_t* d_stack_in,
+                              uint8_t* d_stack_out, int num_envs, int size, int num_frames, void* stream);
+
 /* ---- K-RET: n-step returns and advantages --------------------------------------------------- */
 /* Replaces objectives._discount/_discount_bootstrap + targets/advantage (objectives.py:123-130,
  * 178-214).  rewards f32 [E,T], terminals u8 [E,T], values f32 [E,T], bootstrap f32 [E]

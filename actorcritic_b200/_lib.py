@@ -122,6 +122,8 @@ SIGNATURES = {
                                               ctypes.c_int, ctypes.POINTER(_P), ctypes.c_int, _P]),
     "acx_debug_gemm_trace": (ctypes.c_int, [ctypes.POINTER(ctypes.c_longlong)]),
     "acx_debug_inv_trace": (ctypes.c_int, [ctypes.POINTER(ctypes.c_longlong), ctypes.c_int]),
+    "acx_debug_kfac_invert": (ctypes.c_int, [ctypes.c_int, _P, _P, _P, ctypes.c_int, ctypes.c_float, ctypes.c_float, _P,
+                                             ctypes.c_int, ctypes.c_int, _P, _P, _P, ctypes.POINTER(ctypes.c_int)]),
     "acx_debug_conv_trace": (ctypes.c_int, [ctypes.POINTER(ctypes.c_longlong)]),
     "acx_learner_arena_bytes": (ctypes.c_size_t, [ctypes.POINTER(LearnerConfig)]),
     "acx_learner_create": (_P, [ctypes.POINTER(LearnerConfig), _P, ctypes.c_size_t]),

@@ -370,4 +370,111 @@ int GraphCache::end_capture(Entry& ge, cudaStream_t st, int issue_result, uint64
   return 0;
 }
 
+// ------------------------------------------------------------------------------------------------
+// test hook: one inverse refresh of a block set built as the learners build it (include/acx.h)
+// ------------------------------------------------------------------------------------------------
+namespace {
+
+struct DebugRefresh {
+  KfacBlocks kb;
+  void* arena = nullptr;
+  cudaStream_t st = nullptr, side = nullptr;
+  ~DebugRefresh() {
+    if (st) cudaStreamSynchronize(st);
+    if (side) cudaStreamSynchronize(side);
+    if (arena) cudaFree(arena);
+    if (st) cudaStreamDestroy(st);
+    if (side) cudaStreamDestroy(side);
+  }
+};
+
+int debug_kfac_invert(int num_blocks, const int* h_k, const int* h_c, const int* h_tnorm, int shared_heads, float damping,
+                      float debias, const float* h_sums, int path, int side_stream, float* h_inv, uint16_t* h_planes,
+                      float* h_damp, int* h_path_ran) {
+  ACX_CHECK(num_blocks >= 1 && num_blocks <= kMaxBlocks && h_k && h_c && h_tnorm && h_sums && h_inv && h_planes && h_damp &&
+                h_path_ran, "bad argument");
+  ACX_CHECK(path >= 0 && path <= 2, "path must be 0, 1 or 2");
+  ACX_CHECK(!shared_heads || (num_blocks >= 2 && h_k[num_blocks - 1] == h_k[num_blocks - 2]),
+            "shared heads need two blocks with the same input dimension");
+  const int nfac = shared_heads ? num_blocks - 1 : num_blocks;
+  ACX_CHECK(nfac <= kMaxBlocks - 1, "at most 5 input factors");
+  DebugRefresh d;
+  KfacBlocks& kb = d.kb;
+  for (int i = 0; i < num_blocks; ++i) {
+    ACX_CHECK(h_k[i] >= 0 && h_c[i] >= 1 && h_tnorm[i] >= 1, "bad block dimensions");
+    kb.blk[i].name = "b" + std::to_string(i);
+    kb.blk[i].K = h_k[i];
+    kb.blk[i].C = h_c[i];
+    kb.blk[i].Tnorm = h_tnorm[i];
+    kb.blk[i].afac = i < nfac ? i : nfac - 1;
+  }
+  kb.set_blocks(num_blocks);
+  Arena sizing;
+  kb.take_state(sizing);
+  kb.take_tables(sizing);
+  const size_t bytes = align_up(sizing.used, 256);
+  ACX_CUDA(cudaMalloc(&d.arena, bytes));
+  Arena ar;
+  ar.base = reinterpret_cast<uint8_t*>(d.arena);
+  kb.take_state(ar);
+  kb.take_tables(ar);
+  ACX_TRY(kb.upload(d.arena, bytes, false, 0.0f, damping));
+  ACX_CUDA(cudaStreamCreateWithFlags(&d.st, cudaStreamNonBlocking));
+  if (side_stream) ACX_CUDA(cudaStreamCreateWithFlags(&d.side, cudaStreamNonBlocking));
+  size_t off = 0;
+  for (int f = 0; f < nfac; ++f) {
+    const size_t n2 = (size_t)kb.adim[f] * kb.adim[f];
+    ACX_CUDA(cudaMemcpy(kb.sums + kb.aoff[f], h_sums + off, n2 * sizeof(float), cudaMemcpyHostToDevice));
+    off += n2;
+  }
+  for (int i = 0; i < num_blocks; ++i) {
+    const size_t n2 = (size_t)kb.blk[i].C * kb.blk[i].C;
+    ACX_CUDA(cudaMemcpy(kb.sums + kb.goff[i], h_sums + off, n2 * sizeof(float), cudaMemcpyHostToDevice));
+    off += n2;
+  }
+  const Sched s = {0ull, 0ull, 0.0f, debias};
+  ACX_CUDA(cudaMemcpy(kb.sched, &s, sizeof(s), cudaMemcpyHostToDevice));
+  ACX_CUDA(cudaDeviceSynchronize());   // the set-up above ran on the legacy stream, the refresh runs on a non-blocking one
+  const uint64_t launches = g_launch_count;
+  if (path == 0) {
+    ACX_TRY(kb.invert(d.st, d.side));
+    *h_path_ran = g_launch_count - launches == 1 ? 0 : 1;   // the resident refresh is one launch, the chain several
+  } else if (path == 1) {
+    const int r = spd_inverse_resident(kb.h_jobs, 2 * num_blocks, kb.sched, kb.damp, kb.d_a_ptrs, kb.d_g_ptrs, kb.d_a_dims,
+                                       kb.d_g_dims, kb.lambdas, num_blocks, kb.inv_bar, d.st);
+    if (r < 0) return -1;
+    ACX_TRY(r);
+    *h_path_ran = 0;
+  } else {
+    ACX_TRY(compute_dampings(kb.d_a_ptrs, kb.d_g_ptrs, kb.d_a_dims, kb.d_g_dims, kb.lambdas, num_blocks, kb.damp, d.st));
+    ACX_TRY(spd_inverse_batched(kb.h_jobs, kb.d_jobs, 2 * num_blocks, kb.sched, kb.damp, d.st, d.side));
+    *h_path_ran = 1;
+  }
+  ACX_CUDA(cudaStreamSynchronize(d.st));
+  size_t io = 0, po = 0;
+  for (int j = 0; j < 2 * num_blocks; ++j) {
+    const int i = j % num_blocks;
+    const int n = j < num_blocks ? kb.blk[i].K + 1 : kb.blk[i].C;
+    const float* inv = kb.inv + (j < num_blocks ? kb.ainv_off[i] : kb.ginv_off[i]);
+    const Planes& pl = j < num_blocks ? kb.ainv_pl[i] : kb.ginv_pl[i];
+    ACX_CUDA(cudaMemcpy(h_inv + io, inv, (size_t)n * n * sizeof(float), cudaMemcpyDeviceToHost));
+    io += (size_t)n * n;
+    for (int q = 0; q < 3; ++q) {
+      ACX_CUDA(cudaMemcpy(h_planes + po, pl.p[q], (size_t)n * pl.ld * sizeof(bf16), cudaMemcpyDeviceToHost));
+      po += (size_t)n * pl.ld;
+    }
+  }
+  ACX_CUDA(cudaMemcpy(h_damp, kb.damp, 2 * num_blocks * sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+}  // namespace
+
 }  // namespace acx
+
+extern "C" int acx_debug_kfac_invert(int num_blocks, const int* h_k, const int* h_c, const int* h_tnorm, int shared_heads,
+                                     float damping, float debias, const float* h_sums, int path, int side_stream, float* h_inv,
+                                     uint16_t* h_planes, float* h_damp, int* h_path_ran) {
+  return acx::debug_kfac_invert(num_blocks, h_k, h_c, h_tnorm, shared_heads, damping, debias, h_sums, path, side_stream, h_inv,
+                                h_planes, h_damp, h_path_ran);
+}

@@ -398,3 +398,44 @@ def clip_momentum_step(params, accum, grads, lr, momentum=0.9, clip_norm=3.4e38)
                                                   float(lr), float(momentum), float(clip_norm), _ptr(scratch),
                                                   ctypes.c_void_p(scratch.data_ptr() + 296 * 4), _stream()))
     return scratch[296]
+
+
+def kfac_invert(a_sums, g_sums, tnorm=None, shared_heads=False, damping=0.01, debias=1.0, path=0, side_stream=False):
+    """acx_debug_kfac_invert: one K-FAC inverse refresh of the blocks the learners would build, on host fp32 running sums.
+    a_sums: one [d, d] input factor per block (one fewer with shared_heads: the last two blocks share the last one);
+    g_sums: one [C, C] output factor per block; tnorm: T~ per block (default 1).  path 0 = the learners' refresh,
+    1 = the resident kernel only, 2 = the fp64 chain only.  Returns None when path 1 does not fit, else a dict with
+    inv_a / inv_g (fp32 [n, n] per block), planes_a / planes_g (uint16 bf16 bits [3, n, pad8(n)] per block),
+    damp (fp32 [num_blocks, 2]: damp_A, damp_G) and path (0 = resident kernel ran, 1 = fp64 chain)."""
+    import numpy as np
+    a_sums = [np.ascontiguousarray(a, dtype=np.float32) for a in a_sums]
+    g_sums = [np.ascontiguousarray(g, dtype=np.float32) for g in g_sums]
+    nb = len(g_sums)
+    assert len(a_sums) == (nb - 1 if shared_heads else nb)
+    dims_a = [a_sums[min(i, len(a_sums) - 1)].shape[0] for i in range(nb)]
+    dims_g = [g.shape[0] for g in g_sums]
+    tnorm = [1] * nb if tnorm is None else list(tnorm)
+    sums = np.concatenate([s.ravel() for s in a_sums + g_sums])
+    dims = dims_a + dims_g
+    inv = np.empty(sum(n * n for n in dims), np.float32)
+    planes = np.empty(sum(3 * n * pad8(n) for n in dims), np.uint16)
+    damp = np.empty(2 * nb, np.float32)
+    ran = ctypes.c_int(-1)
+
+    def ints(v):
+        return (ctypes.c_int * nb)(*[int(x) for x in v])
+    st = _lib.load().acx_debug_kfac_invert(nb, ints([d - 1 for d in dims_a]), ints(dims_g), ints(tnorm), int(bool(shared_heads)),
+                                           float(damping), float(debias), sums.ctypes.data, int(path), int(bool(side_stream)),
+                                           inv.ctypes.data, planes.ctypes.data, damp.ctypes.data, ctypes.byref(ran))
+    if st == -1 and path == 1:
+        return None
+    _lib.check(st)
+    out = dict(inv_a=[], inv_g=[], planes_a=[], planes_g=[], damp=damp.reshape(nb, 2), path=ran.value)
+    io = po = 0
+    for j, n in enumerate(dims):
+        kind = "a" if j < nb else "g"
+        out["inv_" + kind].append(inv[io:io + n * n].reshape(n, n))
+        out["planes_" + kind].append(planes[po:po + 3 * n * pad8(n)].reshape(3, n, pad8(n)))
+        io += n * n
+        po += 3 * n * pad8(n)
+    return out

@@ -182,6 +182,22 @@ int acx_debug_gemm_trace(long long* h_out4);
  * look-ahead CTA 0 ([5] step start [6] pivot inversion done [7] barrier passed); a refresh that falls back to the fp64
  * chain records nothing.  Copies `count` (<= 1024) values. */
 int acx_debug_inv_trace(long long* h_out, int count);
+/* test hook: one K-FAC inverse refresh, as the learners run it, on caller-given running sums.  Builds num_blocks K-FAC blocks
+ * (input factor K[i] + 1, output factor C[i], T~ tnorm[i]; shared_heads != 0: the last two blocks read one input factor, as
+ * the policy and value heads do; at most 5 input factors), lays out and zeroes their state in a device arena of its own,
+ * copies the sums in, sets the zero-debias factor and runs
+ *   path 0  the learners' refresh: the resident fp32 kernel, or the fp64 chain when its tiles do not fit;
+ *   path 1  the resident kernel only; returns -1 (and writes nothing) when the tiles do not fit;
+ *   path 2  the dampings and the fp64 chain only.
+ * side_stream != 0: the chain inverts its pivot blocks on a second stream, as the Atari learner does.
+ * h_sums: the input factors [d, d] in factor order, then the output factors [C, C] in block order, packed.  Outputs, packed
+ * in job order (the input-factor inverse of each block, then the output-factor inverse of each block): h_inv fp32 [n, n];
+ * h_planes the bf16 bits of the three operand planes of each inverse [3][n][ld], ld = n rounded up to 8; h_damp the
+ * dampings [2 * num_blocks] (A, G per block); *h_path_ran 0 = resident kernel, 1 = fp64 chain.  Synchronous; frees
+ * everything it allocated before it returns. */
+int acx_debug_kfac_invert(int num_blocks, const int* h_k, const int* h_c, const int* h_tnorm, int shared_heads, float damping,
+                          float debias, const float* h_sums, int path, int side_stream, float* h_inv, uint16_t* h_planes,
+                          float* h_damp, int* h_path_ran);
 /* debug hook: override the UMMA shared-memory descriptor strides (bytes) used for MN-major operands;
  * 0 restores the built-in values. */
 void acx_debug_set_mn_desc(uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t kstep_bytes);

@@ -8,11 +8,11 @@ out.  The optimizer side is oracle.mlp.MLPOracle with the true VALID location co
 (damping / T, preconditioned block / T; oracle.kfac TRUE_LOCATIONS at the Nature geometry).  Parameters: conv kernels HWIO
 in and [k*k*c_in, filters] (the [K+1, C] block layout) inside the learner; forward / backward accept either.
 """
-import math
 
 import numpy as np
 import torch
 
+from . import kfac as K
 from . import mlp as OM
 from . import network as net
 
@@ -145,13 +145,10 @@ class CNNOracle(OM.MLPOracle):
     def update_inverses(self):
         """pi-damped inverses with damping lambda / T (oracle.kfac.KfacState.dampings)."""
         for l in self.layers:
-            a = self.sum_a[OM.factor_of(l)] * self._debias()
-            g = self.sum_g[l] * self._debias()
-            tr_a, tr_g = float(torch.trace(a)) / a.shape[0], float(torch.trace(g)) / g.shape[0]
-            pi = math.sqrt(tr_a / tr_g) if tr_a > 0 and tr_g > 0 else 1.0
-            root = math.sqrt(self.cfg.damping / self.locations[l])
-            self.inv_a[l] = torch.linalg.inv(a + pi * root * torch.eye(a.shape[0], dtype=self.dtype))
-            self.inv_g[l] = torch.linalg.inv(g + root / pi * torch.eye(g.shape[0], dtype=self.dtype))
+            sa, sg, debias = self.sum_a[OM.factor_of(l)], self.sum_g[l], self._debias()
+            damp_a, damp_g = K.pi_dampings(sa * debias, sg * debias, self.cfg.damping / self.locations[l])
+            self.inv_a[l] = K.damped_inverse(sa, debias, damp_a)
+            self.inv_g[l] = K.damped_inverse(sg, debias, damp_g)
 
     def precondition(self, grads):
         """U = A^-1 V G^-1 / T with the stored inverses."""

@@ -12,6 +12,7 @@ Unpinned choices (SURVEY A.7 U1-U6) are explicit parameters of KfacConfig.
 import dataclasses
 import math
 
+import numpy as np
 import torch
 
 from . import network as net
@@ -101,6 +102,86 @@ def batch_factors(fwd, fisher_pre_grads):
     return a, g
 
 
+def pi_dampings(a, g, lam):
+    """pi-adjusted damping of one block (SURVEY A.5 'Damping') from its input and output factors:
+    pi = sqrt((tr A / dim A) / (tr G / dim G)) (1 when either trace is not positive), returns (pi sqrt(lam), sqrt(lam) / pi).
+    A common scale of A and G (the zero-debias factor) cancels in pi."""
+    tr_a = torch.trace(a) / a.shape[0]
+    tr_g = torch.trace(g) / g.shape[0]
+    pi = math.sqrt(float(tr_a) / float(tr_g)) if float(tr_a) > 0 and float(tr_g) > 0 else 1.0
+    root = math.sqrt(lam)
+    return pi * root, root / pi
+
+
+def damped_inverse(s, debias, damp):
+    """(debias * sym(S) + damp * I)^-1 of a running sum S, sym(S) = (S + S^T) / 2 (the kernels symmetrise the sums they
+    load; a symmetric S is used exactly as it is)."""
+    s = torch.as_tensor(s)
+    m = 0.5 * (s + s.T) * debias
+    return torch.linalg.inv(m + damp * torch.eye(s.shape[0], dtype=s.dtype))
+
+
+# ------------------------------------------------------------------------------------------------ test factors
+# Seeded fp32 running sums for the inverse-refresh tests (tests/test_gpu_kfac_inverse.py), as float64 tensors whose values are
+# exactly representable in fp32.
+def gram_factor(n, rows, seed, homogeneous=True, scale_octaves=14):
+    """S = X^T X / rows, X [rows, n] of small integers times per-column powers of two in [2^-scale_octaves, 1] (the last
+    column all ones with `homogeneous`, as the border of an input factor).  rows a power of two: every entry of S is then
+    computed exactly and is exactly representable in fp32, so S is exactly PSD with rank min(rows, n), and the extreme
+    eigenvalues come from the smaller Gram matrix.  Returns (S, lam_min, lam_max), lam_min = 0 when rows < n."""
+    assert rows & (rows - 1) == 0 and rows <= 4096
+    rng = np.random.default_rng(seed)
+    x = rng.integers(-7, 8, (rows, n)).astype(np.float64) * np.exp2(-rng.integers(0, scale_octaves + 1, n))
+    if homogeneous:
+        x[:, -1] = 1.0
+    x = torch.from_numpy(x)
+    s = x.T @ x / rows
+    small = s if rows >= n else x @ x.T / rows
+    lam = torch.linalg.eigvalsh(small)
+    assert torch.equal(s, s.float().double())
+    return s, (float(lam[0]) if rows >= n else 0.0), float(lam[-1])
+
+
+def spectrum_factor(eigenvalues, seed):
+    """Q diag(eigenvalues) Q^T with a seeded random orthogonal Q, rounded to fp32 (so its spectrum is the prescribed one
+    up to fp32 rounding, relative to the largest eigenvalue)."""
+    lam = torch.as_tensor(np.asarray(eigenvalues, np.float64))
+    n = lam.shape[0]
+    q, r = torch.linalg.qr(torch.from_numpy(np.random.default_rng(seed).standard_normal((n, n))))
+    q = q * torch.sign(torch.diagonal(r))
+    s = (q * lam) @ q.T
+    return (0.5 * (s + s.T)).float().double()
+
+
+def zero_factor(n):
+    """An all-zero running sum: its trace is 0, so pi falls back to 1 for its block."""
+    return torch.zeros((n, n), dtype=torch.float64)
+
+
+def with_antisymmetric_ulp(s):
+    """S plus a one-ulp antisymmetric part: above the diagonal every other entry of S moves one fp32 ulp up, its mirror one
+    ulp down - what the kernels must symmetrise away (sym of the result equals sym of S up to half an ulp)."""
+    s32 = s.float().numpy().copy()
+    iu = np.triu_indices(s32.shape[0], 1)
+    i, j = iu[0][::2], iu[1][::2]
+    s32[i, j] = np.nextafter(s32[i, j], np.float32(np.inf))
+    s32[j, i] = np.nextafter(s32[j, i], np.float32(-np.inf))
+    return torch.from_numpy(s32).double()
+
+
+def damping_for_kappa(a, g, kappa, debias=1.0, tnorm=1, lam_min=None, lam_max=None):
+    """The `damping` hyper-parameter at which the damped input factor debias * sym(A) + damp_A I of a block reaches the
+    condition number `kappa`, with damp_A from the fp64 pi formula (lam = damping / tnorm).  lam_min / lam_max: the extreme
+    eigenvalues of sym(A) when known (else computed)."""
+    if lam_min is None or lam_max is None:
+        lam = torch.linalg.eigvalsh(0.5 * (a + a.T))
+        lam_min, lam_max = float(lam[0]), float(lam[-1])
+    damp_a = debias * (lam_max - kappa * lam_min) / (kappa - 1.0)
+    assert damp_a > 0, "kappa %g is beyond the factor's own condition number" % kappa
+    pi = pi_dampings(a, g, 1.0)[0]   # damp_A = pi sqrt(lam)
+    return (damp_a / pi) ** 2 * tnorm
+
+
 class KfacState:
     """Running covariance sums, debias counter, stored inverses, velocities (SURVEY A.5)."""
 
@@ -145,24 +226,13 @@ class KfacState:
 
     def dampings(self, layer):
         """pi-adjusted damping of one block: (damp_A, damp_G)."""
-        a = self.cov_a(A_FACTOR_OF[layer])
-        g = self.cov_g(layer)
-        lam = self.cfg.damping / self.cfg.locations(layer)
-        tr_a = torch.trace(a) / a.shape[0]
-        tr_g = torch.trace(g) / g.shape[0]
-        pi = math.sqrt(float(tr_a) / float(tr_g)) if float(tr_a) > 0 and float(tr_g) > 0 else 1.0
-        root = math.sqrt(lam)
-        return pi * root, root / pi
+        return pi_dampings(self.cov_a(A_FACTOR_OF[layer]), self.cov_g(layer), self.cfg.damping / self.cfg.locations(layer))
 
     def update_inverses(self):
         for layer in net.LAYERS:
             damp_a, damp_g = self.dampings(layer)
-            a = self.cov_a(A_FACTOR_OF[layer])
-            g = self.cov_g(layer)
-            eye_a = torch.eye(a.shape[0], dtype=self.dtype)
-            eye_g = torch.eye(g.shape[0], dtype=self.dtype)
-            self.inv_a[layer] = torch.linalg.inv(a + damp_a * eye_a)
-            self.inv_g[layer] = torch.linalg.inv(g + damp_g * eye_g)
+            self.inv_a[layer] = damped_inverse(self.sum_a[A_FACTOR_OF[layer]], self._debias(), damp_a)
+            self.inv_g[layer] = damped_inverse(self.sum_g[layer], self._debias(), damp_g)
 
     def precondition(self, grads):
         """U_l = A^-1 V_l G^-1 / T~_l with the STORED inverses."""

@@ -134,13 +134,10 @@ class MLPOracle:
     def update_inverses(self):
         """pi-damped inverses (damping / T~ with T~ = 1 for fully connected blocks)."""
         for l in self.layers:
-            a = self.sum_a[factor_of(l)] * self._debias()
-            g = self.sum_g[l] * self._debias()
-            tr_a, tr_g = float(torch.trace(a)) / a.shape[0], float(torch.trace(g)) / g.shape[0]
-            pi = math.sqrt(tr_a / tr_g) if tr_a > 0 and tr_g > 0 else 1.0
-            root = math.sqrt(self.cfg.damping)
-            self.inv_a[l] = torch.linalg.inv(a + pi * root * torch.eye(a.shape[0], dtype=self.dtype))
-            self.inv_g[l] = torch.linalg.inv(g + root / pi * torch.eye(g.shape[0], dtype=self.dtype))
+            sa, sg, debias = self.sum_a[factor_of(l)], self.sum_g[l], self._debias()
+            damp_a, damp_g = K.pi_dampings(sa * debias, sg * debias, self.cfg.damping)
+            self.inv_a[l] = K.damped_inverse(sa, debias, damp_a)
+            self.inv_g[l] = K.damped_inverse(sg, debias, damp_g)
 
     def precondition(self, grads):
         return {l: self.inv_a[l] @ grads[l] @ self.inv_g[l] for l in self.layers}

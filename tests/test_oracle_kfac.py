@@ -306,3 +306,79 @@ def test_one_relu_unit_within_rounding_of_zero_moves_a_conv_gradient_by_1e_4():
     assert worst < 1e-5                                            # the disagreeing units ARE within rounding of zero
     assert max(sync.values()) < 5e-6, sync                         # arithmetic error once the branches agree
     assert own["conv1"] > 20 * sync["conv1"] and own["conv1"] > 1e-5, (flips, own, sync)
+
+
+# ------------------------------------------------------------------------------------------------ inverse-refresh reference
+def test_kfac_state_inverses_are_the_shared_reference():
+    """KfacState.dampings / update_inverses go through pi_dampings / damped_inverse, and give exactly what the inline formulas
+    gave before: pi from the traces of the debiased factors, (S debias + damp I)^-1 of the (symmetric) running sums."""
+    o, _ = _state_after_updates(2)
+    st_ = o.kfac
+    debias = st_._debias()
+    assert debias != 1.0
+    st_.update_inverses()
+    for layer in onet.LAYERS:
+        a, g = st_.cov_a(K.A_FACTOR_OF[layer]), st_.cov_g(layer)
+        lam = st_.cfg.damping / st_.cfg.locations(layer)
+        tr_a, tr_g = float(torch.trace(a)) / a.shape[0], float(torch.trace(g)) / g.shape[0]
+        pi = math.sqrt(tr_a / tr_g)
+        assert st_.dampings(layer) == (pi * math.sqrt(lam), math.sqrt(lam) / pi)
+        want_a = torch.linalg.inv(a + pi * math.sqrt(lam) * torch.eye(a.shape[0], dtype=torch.float64))
+        want_g = torch.linalg.inv(g + math.sqrt(lam) / pi * torch.eye(g.shape[0], dtype=torch.float64))
+        assert torch.equal(st_.inv_a[layer], want_a) and torch.equal(st_.inv_g[layer], want_g)
+
+
+def test_pi_dampings_edge_cases():
+    a, g = torch.eye(3, dtype=torch.float64) * 4.0, torch.eye(2, dtype=torch.float64)
+    assert K.pi_dampings(a, g, 0.01) == pytest.approx((0.2, 0.05), rel=1e-15)
+    assert K.pi_dampings(a * 7.0, g * 7.0, 0.01) == K.pi_dampings(a, g, 0.01)     # a common scale cancels
+    assert K.pi_dampings(a, K.zero_factor(2), 0.01) == (0.1, 0.1)                  # zero trace: pi = 1
+    assert K.pi_dampings(K.zero_factor(3), g, 0.25) == (0.5, 0.5)
+
+
+def test_damped_inverse_symmetrises():
+    s, _, _ = K.gram_factor(40, 16, 3)
+    a = K.with_antisymmetric_ulp(s)
+    assert not torch.equal(a, a.T) and torch.equal(a.float().double(), a)
+    assert float((a - s).abs().max()) <= float(s.abs().max()) * 2.0 ** -23
+    assert float((0.5 * (a + a.T) - s).abs().max()) <= float(s.abs().max()) * 2.0 ** -24
+    inv = K.damped_inverse(a, 2.0, 0.5)
+    m = 2.0 * 0.5 * (a + a.T) + 0.5 * torch.eye(40, dtype=torch.float64)
+    assert torch.equal(inv, inv.T) or float((inv - inv.T).abs().max()) < 1e-14
+    assert float((inv @ m - torch.eye(40, dtype=torch.float64)).abs().max()) < 1e-12
+
+
+@pytest.mark.parametrize("n, rows", [(1, 64), (33, 64), (513, 64), (65, 128)])
+def test_gram_factor_is_exact_with_the_stated_spectrum(n, rows):
+    s, lo, hi = K.gram_factor(n, rows, n)
+    assert torch.equal(s, s.T) and torch.equal(s, s.float().double())
+    assert float(s[-1, -1]) == 1.0                                              # homogeneous corner
+    lam = torch.linalg.eigvalsh(s)
+    assert abs(float(lam[-1]) - hi) <= 1e-12 * hi
+    assert abs(float(lam[0]) - lo) <= 1e-12 * hi
+    assert int((lam > 1e-10 * hi).sum()) == min(n, rows)
+
+
+def test_spectrum_factor_has_the_prescribed_spectrum():
+    want = np.geomspace(1.0, 1e-3, 50)
+    s = K.spectrum_factor(want, 4)
+    assert torch.equal(s, s.T) and torch.equal(s, s.float().double())
+    got = torch.linalg.eigvalsh(s).numpy()[::-1]
+    assert np.abs(got - want).max() <= 1e-6
+
+
+@pytest.mark.parametrize("kappa", [1e1, 1e4, 1e7])
+@pytest.mark.parametrize("n, rows", [(513, 64), (513, 2048), (1569, 64), (1569, 2048)])
+@pytest.mark.parametrize("debias", [1.0, 1.0 / (1.0 - 0.99 ** 3)])
+def test_damping_for_kappa_reaches_the_target(kappa, n, rows, debias):
+    """The damping the conditioning tests use puts the damped input factor at the target condition number, through the fp64
+    pi formula and the fp32 lambda the learners store (damping / T~ in fp32)."""
+    s, lo, hi = K.gram_factor(n, rows, 11)
+    g = K.spectrum_factor([1.0, 0.5, 0.25, 0.125], 1)
+    damping = K.damping_for_kappa(s, g, kappa, debias, tnorm=4, lam_min=lo, lam_max=hi)
+    lam = float(np.float32(np.float32(damping) / np.float32(4)))
+    d = float(np.float32(K.pi_dampings(s, g, lam)[0]))
+    assert abs((debias * hi + d) / (debias * lo + d) / kappa - 1) < 1e-5
+    if n == 513:   # the spectrum the shortcut used, against the full eigendecomposition
+        lam_m = torch.linalg.eigvalsh(debias * s + d * torch.eye(n, dtype=torch.float64))
+        assert abs(float(lam_m[-1] / lam_m[0]) / kappa - 1) < 1e-4
